@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: pMHC graphs/s of the ImmunoStruct hot path on B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): HybridModelv2 inference (eval, no_grad) over synthetic pMHC
 graphs of the named shape (200 residues, directed 10-NN contacts, 283x21 sequence one-hots), batch
@@ -77,7 +77,33 @@ def parse():
                     help="bracket the timed inference region with cudaProfilerStart/Stop (ncu --profile-from-start off)")
     ap.add_argument("--no-train", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed inference step returned (probabilities and the model's recon, mu, "
+                         "logvar, logits) as DIR/<name>.npy, float32, rank 0; inputs are seeded, so two builds can be "
+                         "compared output for output")
     return ap.parse_args()
+
+
+DUMP_LIMIT = 64 * 10 ** 6           # bytes of all dumped arrays together
+
+
+def dump_outputs(path, tensors):
+    """Write each tensor as <path>/<name>.npy (float32).  If they exceed DUMP_LIMIT together, the largest is cut to
+    a fixed, seeded sample of its rows (the same rows in every run with the same arguments)."""
+    import numpy as np
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in tensors.items()}
+    big = max(arrays, key=lambda k: arrays[k].nbytes)
+    rest = sum(a.nbytes for k, a in arrays.items() if k != big)
+    a = arrays[big]
+    rows = (DUMP_LIMIT - rest - 4096 * len(arrays)) // max(1, a[0].nbytes)
+    if rows < 0:
+        raise ValueError(f"--dump-outputs: the arrays other than {big} alone exceed {DUMP_LIMIT} bytes")
+    if rows < a.shape[0]:
+        idx = np.sort(np.random.default_rng(0).choice(a.shape[0], rows, replace=False))
+        arrays[big] = a[idx]
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
 
 
 def measured_peaks():
@@ -291,11 +317,12 @@ def main():
     broadcast_parameters(model)
     pool = make_pool(B, POOL, seed=1 + 1000 * rank, device=dev)
     keys = ("x", "src", "dst", "edge_attr", "node_counts", "edge_counts")
+    last = {}                                      # model outputs of the latest inference step (for --dump-outputs)
 
     def infer_step(arr, dense):
         gb = GraphBatch.from_arrays(*(arr[k] for k in keys), max_nodes=N_NODES)
-        out = model(gb, dense["seq"], dense["prop"])[3]
-        return torch.sigmoid(out).squeeze()
+        last["outputs"] = model(gb, dense["seq"], dense["prop"])
+        return torch.sigmoid(last["outputs"][3]).squeeze()
 
     # ---- device-resident inference throughput (the headline `value`) ---------------------------
     model.eval()
@@ -335,6 +362,9 @@ def main():
             torch.cuda.profiler.stop()
         ms = min(infer_windows)
     value = world * B * K / (ms / 1e3)
+    if args.dump_outputs and rank == 0:
+        recon, mu, logvar, logits = last["outputs"]
+        dump_outputs(args.dump_outputs, {"probs": probs, "recon": recon, "mu": mu, "logvar": logvar, "logits": logits})
 
     # ---- BASELINE configs[1], literally: a scan of 27 000 graphs = 52 full batches of 512 + one of 376 (the last,
     # partial batch of the reference's no-drop_last loader, procedures/infer.py:14-31); per rank at N > 1 ------------
@@ -443,7 +473,7 @@ def main():
     train = None
     if not args.no_train:
         losses = I.Losses(VAE_IN, [0.81, 0.19], sequence=True)
-        kt = max(5, min(K, 20))
+        kt = K
         wt = max(W, 5)                 # the training path touches far more kernels / allocator blocks than inference
 
         def run_training(tmodel, opt, reducer, tpool, batch, steps, warm):
@@ -492,7 +522,7 @@ def main():
             tm = I.model_map["HybridModelv2"](vae_input_dim=VAE_IN, device=dev).to(dev)
             tm.load_state_dict(state0)
             t_adam = run_training(tm, torch.optim.Adam(tm.parameters(), lr=1e-3), GradientAllReducer(tm.parameters()), pool, B,
-                                  max(5, kt // 2), wt)
+                                  kt, wt)
             train["torch_adam"] = {k: t_adam[k] for k in ("value", "unit", "ms_per_step", "final_loss")}
             del tm
         # BASELINE configs[3]: FIXED global batch of 4 096 graphs (strong scaling): 4096 / N graphs per GPU
@@ -537,7 +567,7 @@ def main():
             copt.step()
             return loss
 
-        kc = max(5, min(K, 20))
+        kc = K
         for i in range(max(W, 5)):
             cmp_step(i)
         cwin = []

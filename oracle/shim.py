@@ -7,9 +7,8 @@ neither ``dgl`` nor ``torch_geometric``.  TEST INFRASTRUCTURE ONLY (see referenc
 ``import models`` / ``import utils`` resolve to the reference's own packages.  The stand-ins'
 arithmetic (EGNNConv, batch, pooling) is the restatement in ``oracle/reference_ops.py``; everything
 else the imported classes execute is the reference's literal code.  Used by
-``tests/golden/make_golden.py`` to generate the committed vectors and by
-``tests/test_oracle.py::test_restatement_matches_reference_code`` (skipped where
-``/root/reference`` does not exist, e.g. on the GPU box).
+``tests/golden/make_golden.py`` / ``make_golden_r2.py`` to generate the committed vectors, which the tests
+read instead of the reference tree.
 """
 from __future__ import annotations
 

@@ -1,6 +1,5 @@
-"""The oracle against (1) the committed golden vectors produced by the unmodified reference code,
-(2) hand-derived known answers for the un-vendored DGL/PyG operators, (3) the live reference
-when /root/reference exists (build container only)."""
+"""The oracle against (1) the committed golden vectors produced by the unmodified reference code, at the small
+test widths and at the production width, (2) hand-derived known answers for the un-vendored DGL/PyG operators."""
 import math
 
 import pytest
@@ -8,7 +7,6 @@ import torch
 
 from conftest import assert_grads_close, load_golden, oracle_graph, rel_err
 from oracle import reference_ops as R
-from oracle import shim
 
 TOL = 1e-5
 
@@ -151,23 +149,26 @@ def test_batch_and_csr_known_answer():
     assert c["csc_pos"].tolist() == [2, 0, 1, 4, 3]
 
 
-@pytest.mark.skipif(not shim.reference_available(), reason="/root/reference not on this box")
-def test_restatement_matches_reference_code_live():
-    """Default-size HybridModelv2 (vae_input_dim 5943) straight from the reference's class."""
-    from immunostruct_b200.synthetic import synthetic_graph_arrays, synthetic_dense, split_graphs
-    model_map, Losses, _ = shim.load_reference()
-    torch.manual_seed(1)
-    model = model_map["HybridModelv2"](vae_input_dim=5943, device="cpu").eval()
-    arr = synthetic_graph_arrays(2, 40, 6, seed=11, n_pad=3)
-    dense = synthetic_dense(2, seed=11)
-    g = R.dgl_batch(split_graphs(arr))
-    torch.manual_seed(5)
-    ref = model(shim.graph_from_dict(g), dense["seq"], dense["prop"])
-    torch.manual_seed(5)
-    eps = torch.randn(2, 32)
-    got = R.hybrid_forward(dict(model.state_dict()), g, dense["seq"], dense["prop"], eps)
-    for a, b in zip(got, ref):
-        assert rel_err(a, b.detach()) < TOL
+def test_restatement_matches_reference_code_production_width():
+    """HybridModelv2 at the production width (vae_input_dim 5943, vae_hidden_dim 512) against the outputs of the
+    reference's own class stored in r2_big_hybrid_v2.npz (tests/golden/make_golden_r2.py); the weights are regenerated
+    from the same name-keyed seed."""
+    import immunostruct_b200 as I
+    from golden_util import sample_big, seeded_state_dict
+    gd = load_golden("r2_big_hybrid_v2")
+    n_layers = int(gd["meta"]["gcn_layers"])
+    model = I.model_map["HybridModelv2"](vae_input_dim=5943, device="cpu", gcn_layers=n_layers - 1)
+    p = seeded_state_dict(model, int(gd["meta"]["seed"]))
+    d, o = gd["dense"], gd["out"]
+    seq = torch.nn.functional.one_hot(d["seq_tokens"].long(), 21).float()
+    recon, mu, logvar, out = R.hybrid_forward(p, oracle_graph(gd["graph"]), seq, d["prop"], d["eps"], n_layers=n_layers)
+    assert rel_err(out, o["logits"]) < TOL and rel_err(out, o["logits64"]) < TOL
+    assert rel_err(mu, o["mu"]) < TOL and rel_err(logvar, o["logvar"]) < TOL
+    r = sample_big(recon)
+    assert rel_err(r[1:], o["recon_sample"][1:]) < TOL
+    assert abs(float(r[0]) - float(o["recon_sample"][0])) < TOL * float(o["recon_sample"][0])
+    loss = R.bce_loss(recon, seq, mu, logvar, out, d["target"], float(gd["meta"]["pos_weight"]))
+    assert rel_err(loss, o["loss"]) < TOL and rel_err(loss, o["loss64"]) < TOL
 
 
 def test_pooled_only_attention_backward_closed_form():

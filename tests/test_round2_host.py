@@ -51,27 +51,41 @@ def test_segment_pool_modes_and_tie_gradient(cpu_backend):
 
 # ---- contrastive module ----------------------------------------------------------------------------
 def test_contrastive_module_matches_reference_module_including_bn_buffers(cpu_backend):
-    from oracle import shim
-    if not shim.reference_available():
-        pytest.skip("reference tree not present")
-    torch.manual_seed(5)
-    ref = shim.load_reference()[2](embedding_dim=104)
+    """The reference's PairedContrastiveLoss as stored in comparative_v2.npz (tests/golden/make_golden.py): its initial
+    state_dict, the embeddings it was called on and the loss it returned.  Over two further steps on seeded inputs the
+    BatchNorm buffers are held to a default torch.nn.BatchNorm1d (the reference's projector module, run in fp64 on the
+    cancer, then the wild-type projection, as the reference's forward calls it), losses and gradients to fp64 autograd of the restatement
+    (oracle/reference_ops.py paired_contrastive, itself checked against the same stored loss in tests/test_oracle.py)."""
+    gd = load_golden("comparative_v2")
+    state = gd["projector"]
     mine = I.PairedContrastiveLoss(embedding_dim=104)
-    mine.load_state_dict(ref.state_dict())
+    mine.load_state_dict(state)
+    assert rel_err(mine(gd["out"]["emb_c"], gd["out"]["emb_w"], gd["dense"]["target"]), gd["out"]["loss_contrastive"]) < 1e-5
+
+    mine = I.PairedContrastiveLoss(embedding_dim=104)
+    mine.load_state_dict(state)
+    bn = torch.nn.Sequential(torch.nn.Linear(104, 128, bias=False), torch.nn.BatchNorm1d(128)).double()
+    bn.load_state_dict({k[len("projector."):]: v for k, v in state.items() if k.startswith(("projector.0.", "projector.1."))})
+    p64 = {k: v.double().requires_grad_(True) for k, v in state.items() if k.endswith(("weight", "bias"))}
+    torch.manual_seed(5)
     ec, ew = torch.randn(12, 104) * 2, torch.randn(12, 104) * 2
     t = (torch.arange(12) % 3 == 0).float()
-    e1, e2 = ec.clone().requires_grad_(True), ew.clone().requires_grad_(True)
+    e1, e2 = ec.double().requires_grad_(True), ew.double().requires_grad_(True)
     f1, f2 = ec.clone().requires_grad_(True), ew.clone().requires_grad_(True)
+    l_ref = R.paired_contrastive(p64, e1, e2, t)
     for step in range(2):                                   # two steps: running statistics accumulate
-        l_ref = ref(e1, e2, t)
         l_mine = mine(f1, f2, t)
+        bn(ec.double()), bn(ew.double())
         assert rel_err(l_mine, l_ref) < 1e-5
     l_ref.backward(); l_mine.backward()
     assert rel_err(f1.grad, e1.grad) < 1e-4 and rel_err(f2.grad, e2.grad) < 1e-4
-    for (k, a), (_, b) in zip(mine.state_dict().items(), ref.state_dict().items()):
-        assert torch.allclose(a.float(), b.float(), rtol=1e-5, atol=1e-6), k
-    for (k, p), (_, q) in zip(mine.named_parameters(), ref.named_parameters()):
-        assert rel_err(p.grad, q.grad) < 1e-4, k
+    ref_state = {"projector." + k: v for k, v in bn.state_dict().items()}
+    for k, a in mine.state_dict().items():
+        b = ref_state.get(k, state[k])
+        assert torch.allclose(a.double(), b.double(), rtol=1e-5, atol=1e-6), k
+    assert int(mine.projector[1].num_batches_tracked) == 4
+    for k, p in mine.named_parameters():
+        assert rel_err(p.grad, p64[k].grad) < 1e-4, k
     # gated-off batches leave the BatchNorm buffers alone, like the reference (which returns before the projector)
     before = copy.deepcopy(mine.state_dict())
     assert float(mine(f1, f2, torch.ones(12))) == 0.0
