@@ -48,7 +48,8 @@ def exported_symbols():
             "is_fusion_attn_bwd", "is_loss_fwd", "is_loss_bwd", "is_umma_selftest", "is_umma_timing", "is_egnn_edge_fwd_tc", "is_attn_pool_infer", "is_egnn_node_post_pre_tc", "is_egnn_edge_bwd_tc", "is_egnn_edge_bwd_ws", "is_egnn_set_bwd_ws_warps", "is_linear_tc", "is_linear_tc_split_k", "is_attn_pool_infer_tc", "is_vae_mid_infer", "is_head_infer", "is_unpack_nodes", "is_unpack_edges", "is_onehot_tokens", "is_egnn_node_post_bwd_tc", "is_egnn_node_pre_bwd_tc", "is_attn_pool_bwd_tc",
             "is_segment_pool_fwd", "is_segment_pool_bwd", "is_contrastive_scratch_floats", "is_contrastive_fwd",
             "is_contrastive_bwd", "is_fused_adam", "is_rotate_coords", "is_mask_single_residue", "is_mask_rows", "is_gemm_tma_split_k",
-            "is_split_planes", "is_gemm_planes_tma", "is_egnn_set_ws_buffers", "is_egnn_set_ws_variant", "is_reduce_partials3", "is_fused_adam_capturable"]
+            "is_split_planes", "is_gemm_planes_tma", "is_egnn_set_ws_buffers", "is_egnn_set_ws_variant", "is_reduce_partials3", "is_fused_adam_capturable",
+            "is_egnn_edge_attr_grad"]
 
 
 def _check(rc: int, name: str):
@@ -322,6 +323,14 @@ def egnn_node_pre_bwd_tc(gz1, gQ, gD, gxd, gx_out, gh_direct, g, h, W1, gh, gx, 
           _t(gx_out, f32, "gx_out"), _t(gh_direct, f32, "gh_direct"), _t(g.outptr, i32, "outptr"),
           _t(g.csc_pos, i32, "csc_pos"), hp, ldh, _i32(h.shape[1]), _t(W1, f32, "W1"), _t(gh, f32, "gh"),
           _t(gx, f32, "gx"), _t(partials, f32, "partials"), _i64(h.shape[0]), _stream())
+
+
+def egnn_edge_attr_grad(gz1, g, W1, F, g_attr, accumulate):
+    """g_attr [E] (original edge order) (+)= gz1 [E, 64] (CSR order) . W1[:, 2F+1]: one layer's gradient of the scalar edge
+    features (csrc/egnn_edge_attr.cu)."""
+    f32 = torch.float32
+    _call("is_egnn_edge_attr_grad", _t(gz1, f32, "gz1"), _t(g.csr_eid, torch.int32, "csr_eid"), _t(W1, f32, "W1"), _i32(F),
+          _t(g_attr, f32, "g_attr"), _i64(gz1.shape[0]), _i32(1 if accumulate else 0), _stream())
 
 
 def reduce_partials(partials, out):

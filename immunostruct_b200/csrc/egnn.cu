@@ -233,7 +233,7 @@ node_post_fwd_kernel(const float* __restrict__ h, int64_t ldh, int F, const floa
 __global__ void __launch_bounds__(IS_THREADS)
 node_post_bwd_kernel(const float* __restrict__ gh_out, const float* __restrict__ h, int64_t ldh, int F,
                      const float* __restrict__ hn, const float* __restrict__ W5, const float* __restrict__ b5,
-                     const float* __restrict__ W6, float* __restrict__ gh_direct /* [M,64] or null */,
+                     const float* __restrict__ W6, float* __restrict__ gh_direct /* [M,F] or null */,
                      float* __restrict__ ghn, float* __restrict__ partials, int64_t M) {
     extern __shared__ __align__(16) float smem[];
     const int K = F + 64, lda = K + 4;
@@ -298,13 +298,13 @@ node_post_bwd_kernel(const float* __restrict__ gh_out, const float* __restrict__
             int64_t m = m0 + ty + 16 * i;
             if (m < M) *reinterpret_cast<float4*>(ghn + m * 64 + 4 * tx) = make_float4(acc[i][0], acc[i][1], acc[i][2], acc[i][3]);
         }
-        if (gh_direct) {                                  // only for F == 64 layers
+        if (gh_direct) {                                  // [M, F]: columns F .. 63 of the product are zero (zero-padded W5h)
             zero_acc(acc);
             gemm_128x64(acc, G, IS_LD, WB + 4096, 64, ty, tx);
 #pragma unroll
             for (int i = 0; i < 8; ++i) {
                 int64_t m = m0 + ty + 16 * i;
-                if (m < M) *reinterpret_cast<float4*>(gh_direct + m * 64 + 4 * tx) = make_float4(acc[i][0], acc[i][1], acc[i][2], acc[i][3]);
+                if (m < M && 4 * tx < F) *reinterpret_cast<float4*>(gh_direct + m * F + 4 * tx) = make_float4(acc[i][0], acc[i][1], acc[i][2], acc[i][3]);
             }
         }
     }
@@ -592,10 +592,10 @@ edge_bwd_kernel(EdgeCommon p, const float* __restrict__ ghn, const float* __rest
 __global__ void __launch_bounds__(IS_THREADS)
 node_pre_bwd_kernel(const float* __restrict__ gz1, const float* __restrict__ gQ, const float* __restrict__ gD,
                     const float* __restrict__ gxd, const float* __restrict__ gx_out /* or null */,
-                    const float* __restrict__ gh_direct /* [M,64] or null */,
+                    const float* __restrict__ gh_direct /* [M,F] or null */,
                     const int* __restrict__ outptr, const int* __restrict__ csc_pos,
                     const float* __restrict__ h, int64_t ldh, int F, const float* __restrict__ W1,
-                    float* __restrict__ gh /* [M,64] or null */, float* __restrict__ gx /* [M,3] or null */,
+                    float* __restrict__ gh /* [M,F] or null */, float* __restrict__ gx /* [M,3] or null */,
                     float* __restrict__ partials, int64_t M) {
     extern __shared__ __align__(16) float smem[];
     const int lda = F + 4;
@@ -680,13 +680,14 @@ node_pre_bwd_kernel(const float* __restrict__ gz1, const float* __restrict__ gQ,
 #pragma unroll
             for (int i = 0; i < 8; ++i) {
                 int64_t m = m0 + ty + 16 * i;
-                if (m < M) {
+                if (m < M && 4 * tx < F) {                 // [M, F] rows (F = 20: Ws / Wd zero-padded beyond column F)
+                    const size_t off = (size_t)m * F + 4 * tx;
                     float4 o = make_float4(acc[i][0], acc[i][1], acc[i][2], acc[i][3]);
                     if (gh_direct) {
-                        const float4 g = __ldg(reinterpret_cast<const float4*>(gh_direct + m * 64) + tx);
+                        const float4 g = __ldg(reinterpret_cast<const float4*>(gh_direct + off));
                         o.x += g.x; o.y += g.y; o.z += g.z; o.w += g.w;
                     }
-                    *reinterpret_cast<float4*>(gh + m * 64 + 4 * tx) = o;
+                    *reinterpret_cast<float4*>(gh + off) = o;
                 }
             }
         }
@@ -830,7 +831,7 @@ int is_egnn_node_post_bwd(const float* gh_out, const float* h, int64_t ldh, int 
                           const float* W5, const float* b5, const float* W6,
                           float* gh_direct, float* ghn, float* partials, int64_t n_nodes, void* stream) {
     if (!(F == 20 || F == 64) || n_nodes <= 0) return IS_ERR_ARG;
-    if (gh_direct && F != 64) return IS_ERR_ARG;
+    if ((reinterpret_cast<uintptr_t>(gh_direct) & 15) != 0) return IS_ERR_ARG;          // 128-bit stores
     int K = F + 64;
     size_t smem = sizeof(float) * (IS_TM * (K + 4) + 2 * IS_TM * IS_LD + IS_TM * 64);
     int rc = set_smem(node_post_bwd_kernel, smem);
@@ -873,7 +874,7 @@ int is_egnn_node_pre_bwd(const float* gz1, const float* gQ, const float* gD, con
                          const int* outptr, const int* csc_pos, const float* h, int64_t ldh, int F,
                          const float* W1, float* gh, float* gx, float* partials, int64_t n_nodes, void* stream) {
     if (!(F == 20 || F == 64) || n_nodes <= 0) return IS_ERR_ARG;
-    if (gh && F != 64) return IS_ERR_ARG;
+    if (((reinterpret_cast<uintptr_t>(gh) | reinterpret_cast<uintptr_t>(gh_direct)) & 15) != 0) return IS_ERR_ARG;   // 128-bit accesses
     size_t smem = sizeof(float) * (2 * IS_TM * IS_LD + IS_TM * (F + 4) + 2 * 4096);
     int rc = set_smem(node_pre_bwd_kernel, smem);
     if (rc) return rc;

@@ -79,6 +79,23 @@ __device__ __forceinline__ void store2(uint8_t* __restrict__ tile, const float (
 }
 __device__ __forceinline__ uint8_t* chunk_at(uint8_t* tile, int row, int chunk) { return tile + (row >> 3) * SBO + (row & 7) * 16 + chunk * LBO; }
 
+// The 16 columns c0 .. c0 + 15 of one row of an [M, F] fp32 matrix, F = 20 (the layer-0 input features): 80-byte rows are
+// only 16-byte aligned, so 128-bit accesses, and only the columns below F (c0 = 16 holds 16 .. 19).
+__device__ __forceinline__ void load_row16_narrow(float (&v)[CW], const float* __restrict__ row, int c0, int F) {
+#pragma unroll
+    for (int j = 0; j < CW / 4; ++j)
+        if (c0 + 4 * j < F) {
+            const float4 a = __ldg(reinterpret_cast<const float4*>(row + c0 + 4 * j));
+            v[4 * j] = a.x; v[4 * j + 1] = a.y; v[4 * j + 2] = a.z; v[4 * j + 3] = a.w;
+        }
+}
+__device__ __forceinline__ void store_row16_narrow(float* __restrict__ row, const float (&v)[CW], int c0, int F) {
+#pragma unroll
+    for (int j = 0; j < CW / 4; ++j)
+        if (c0 + 4 * j < F)
+            *reinterpret_cast<float4*>(row + c0 + 4 * j) = make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
+}
+
 // sum over the warp's 32 rows of 16 per-lane column values; afterwards lane L holds the total of column (L >> 1) & 15
 __device__ __forceinline__ float colsum16(const float (&v)[16], int lane) {
     float w8[8], w4[4], w2[2];
@@ -116,7 +133,7 @@ __device__ __forceinline__ void silu_both_acc(float z, float& y, float& dy) {
 __global__ void __launch_bounds__(nb::NT, 1)
 node_post_bwd_tc_kernel(const float* __restrict__ gh_out, const float* __restrict__ h, int64_t ldh, int F,
                         const float* __restrict__ hn, const float* __restrict__ W5, const float* __restrict__ b5,
-                        const float* __restrict__ W6, float* __restrict__ gh_direct /* [M,64] or null */,
+                        const float* __restrict__ W6, float* __restrict__ gh_direct /* [M,F] or null */,
                         float* __restrict__ ghn, float* __restrict__ partials, int64_t M) {
     using namespace nb;
     extern __shared__ __align__(128) uint8_t smem_raw[];
@@ -259,13 +276,16 @@ node_post_bwd_tc_kernel(const float* __restrict__ gh_out, const float* __restric
                 }
             }
             if (gh_direct) {
+                // (F = 20: W5h was staged zero-padded beyond column F, so columns F .. 63 of the product are zero)
                 tmem_ld<CW>(t_lane + 192, z);
-                if (m < M) {
+                if (m < M && F == 64) {
 #pragma unroll
                     for (int g = 0; g < CW / 8; ++g) {
                         const float o[8] = {z[8 * g], z[8 * g + 1], z[8 * g + 2], z[8 * g + 3], z[8 * g + 4], z[8 * g + 5], z[8 * g + 6], z[8 * g + 7]};
                         stg256(gh_direct + m * 64 + CW * cq + 8 * g, o);
                     }
+                } else if (m < M) {
+                    store_row16_narrow(gh_direct + m * F, z, CW * cq, F);
                 }
             }
         }
@@ -348,10 +368,10 @@ node_post_bwd_tc_kernel(const float* __restrict__ gh_out, const float* __restric
 __global__ void __launch_bounds__(nb::NT, 1)
 node_pre_bwd_tc_kernel(const float* __restrict__ gz1, const float* __restrict__ gQ, const float* __restrict__ gD,
                        const float* __restrict__ gxd, const float* __restrict__ gx_out /* or null */,
-                       const float* __restrict__ gh_direct /* [M,64] or null */,
+                       const float* __restrict__ gh_direct /* [M,F] or null */,
                        const int* __restrict__ outptr, const int* __restrict__ csc_pos,
                        const float* __restrict__ h, int64_t ldh, int F, const float* __restrict__ W1,
-                       float* __restrict__ gh /* [M,64] or null */, float* __restrict__ gx /* [M,3] or null */,
+                       float* __restrict__ gh /* [M,F] or null */, float* __restrict__ gx /* [M,3] or null */,
                        float* __restrict__ partials, int64_t M) {
     using namespace nb;
     extern __shared__ __align__(128) uint8_t smem_raw[];
@@ -510,15 +530,19 @@ node_pre_bwd_tc_kernel(const float* __restrict__ gz1, const float* __restrict__ 
 #pragma unroll
             for (int i = 0; i < CW; ++i) g[i] = 0.0f;
             if (gh_direct && m < M) {                        // in flight under the MMAs
-                ldg256(gh_direct + m * 64 + CW * cq, *reinterpret_cast<float(*)[8]>(g));
-                ldg256(gh_direct + m * 64 + CW * cq + 8, *reinterpret_cast<float(*)[8]>(g + 8));
+                if (F == 64) {
+                    ldg256(gh_direct + m * 64 + CW * cq, *reinterpret_cast<float(*)[8]>(g));
+                    ldg256(gh_direct + m * 64 + CW * cq + 8, *reinterpret_cast<float(*)[8]>(g + 8));
+                } else {
+                    load_row16_narrow(g, gh_direct + m * F, CW * cq, F);
+                }
             }
             mbar_wait(&mbar, phase);
             phase ^= 1;
             fence_after_sync();
             float z[CW];
             tmem_ld<CW>(t_lane, z);
-            if (m < M) {
+            if (m < M && F == 64) {
 #pragma unroll
                 for (int gg = 0; gg < CW / 8; ++gg) {
                     float o[8];
@@ -526,6 +550,10 @@ node_pre_bwd_tc_kernel(const float* __restrict__ gz1, const float* __restrict__ 
                     for (int i = 0; i < 8; ++i) o[i] = z[8 * gg + i] + g[8 * gg + i];
                     stg256(gh + m * 64 + CW * cq + 8 * gg, o);
                 }
+            } else if (m < M) {                              // F = 20: Ws / Wd staged zero-padded beyond column F
+#pragma unroll
+                for (int i = 0; i < CW; ++i) z[i] += g[i];
+                store_row16_narrow(gh + m * F, z, CW * cq, F);
             }
             fence_before_sync();
         }
@@ -585,8 +613,8 @@ int is_egnn_node_post_bwd_tc(const float* gh_out, const float* h, int64_t ldh, i
                              const float* W5, const float* b5, const float* W6,
                              float* gh_direct, float* ghn, float* partials, int64_t n_nodes, void* stream) {
     if (!(F == 20 || F == 64) || n_nodes <= 0) return IS_ERR_ARG;
-    if (gh_direct && F != 64) return IS_ERR_ARG;
-    if (((reinterpret_cast<uintptr_t>(ghn) | reinterpret_cast<uintptr_t>(gh_direct)) & 31) != 0) return IS_ERR_ARG;   // 256-bit stores
+    if ((reinterpret_cast<uintptr_t>(ghn) & 31) != 0) return IS_ERR_ARG;                                // 256-bit stores
+    if ((reinterpret_cast<uintptr_t>(gh_direct) & (F == 64 ? 31 : 15)) != 0) return IS_ERR_ARG;         // 256- / 128-bit stores
     const size_t smem = 9 * (size_t)nb::T_BYTES + 9 * (size_t)nb::W_BYTES + sizeof(float) * (64 + 16 * 16);
     cudaError_t e = cudaFuncSetAttribute(node_post_bwd_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
@@ -603,8 +631,8 @@ int is_egnn_node_pre_bwd_tc(const float* gz1, const float* gQ, const float* gD, 
                             const float* gh_direct, const int* outptr, const int* csc_pos, const float* h, int64_t ldh, int F,
                             const float* W1, float* gh, float* gx, float* partials, int64_t n_nodes, void* stream) {
     if (!(F == 20 || F == 64) || n_nodes <= 0) return IS_ERR_ARG;
-    if (gh && F != 64) return IS_ERR_ARG;
-    if (((reinterpret_cast<uintptr_t>(gh) | reinterpret_cast<uintptr_t>(gh_direct)) & 31) != 0) return IS_ERR_ARG;   // 256-bit accesses
+    if (((reinterpret_cast<uintptr_t>(gh) | reinterpret_cast<uintptr_t>(gh_direct)) & (F == 64 ? 31 : 15)) != 0)
+        return IS_ERR_ARG;                                                                  // 256- / 128-bit accesses
     const size_t smem = 9 * (size_t)nb::T_BYTES + 6 * (size_t)nb::W_BYTES + (size_t)IS_TM * 64 * sizeof(float);
     cudaError_t e = cudaFuncSetAttribute(node_pre_bwd_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;

@@ -122,23 +122,25 @@ class _EGNNLayer(torch.autograd.Function):
     def backward(ctx, gh_out, gx_out):
         h, x, edge_attr, PQ, hn, *params = ctx.saved_tensors
         has_coord = ctx.update_coords and gx_out is not None
+        g_attr = _new(edge_attr, *edge_attr.shape) if ctx.needs_input_grad[4] else None
         gh, gx, grads = _egnn_layer_backward(ctx.graph, h, x, edge_attr, PQ, hn, params, gh_out,
                                              gx_out if has_coord else None, ctx.needs_input_grad[2],
-                                             ctx.needs_input_grad[3])
-        return (None, None, gh, gx, None, *grads)
+                                             ctx.needs_input_grad[3], g_attr)
+        return (None, None, gh, gx, g_attr, *grads)
 
 
-def _egnn_layer_backward(g, h, x, edge_attr, PQ, hn, params, gh_out, gx_out, need_gh, need_gx):
+def _egnn_layer_backward(g, h, x, edge_attr, PQ, hn, params, gh_out, gx_out, need_gh, need_gx, g_attr=None,
+                         attr_accumulate=False):
     """Backward of one EGNN layer from its saved inputs: node_post_bwd -> edge_bwd -> node_pre_bwd ->
     deterministic reduction of the per-CTA partials.  ``gx_out`` None = the layer's coordinate output
-    received no gradient (coord_mlp then gets NO gradient: None, as in the reference).
+    received no gradient (coord_mlp then gets NO gradient: None, as in the reference).  ``gh`` is [N, F] (F = 20 for
+    the input layer).  ``g_attr`` (or None): buffer of the edge-feature gradient [E] or [E, 1], written (or, with
+    ``attr_accumulate``, added to) from the layer's edge pre-activation gradient.
     Returns (gh or None, gx or None, 11 parameter gradients)."""
     W1, b1, W2, b2, W3, b3, w4, W5, b5, W6, b6 = params
     n, f = h.shape
     e = g.n_edges
     k = f + H
-    if need_gh and f != H:
-        raise NotImplementedError("gradient w.r.t. the 20-wide input features is not needed by any model")
     if gh_out is None:
         gh_out = torch.zeros(n, H, dtype=torch.float32, device=h.device)
     gh_out = gh_out.contiguous()
@@ -148,7 +150,7 @@ def _egnn_layer_backward(g, h, x, edge_attr, PQ, hn, params, gh_out, gx_out, nee
     grid_n, grid_e = _C.egnn_node_grid(n), _C.egnn_edge_bwd_grid(n)
     # node_post backward
     ghn = _new(h, n, H)
-    gh_direct = _new(h, n, H) if need_gh else None
+    gh_direct = _new(h, n, f) if need_gh else None
     p_post = _new(h, grid_n, H * k + H + H * H + H)
     tc = _PRECISIONS[_precision] is not None          # tensor-core (bf16x3) backward kernels in every mode but "fp32"
     (_C.egnn_node_post_bwd_tc if tc else _C.egnn_node_post_bwd)(gh_out, h, hn, W5, b5, W6, gh_direct, ghn, p_post)
@@ -158,10 +160,12 @@ def _egnn_layer_backward(g, h, x, edge_attr, PQ, hn, params, gh_out, gx_out, nee
     bwd = _C.egnn_edge_bwd if _PRECISIONS[_precision] is None else (_C.egnn_edge_bwd_ws if _edge_bwd_streams == 2 else _C.egnn_edge_bwd_tc)
     bwd(g, PQ, x, edge_attr, f, W1, W2, b2, W3, b3, w4, ghn, gx_out, gz1, gQ, gD, gxd, p_edge)
     # node_pre backward (source-side reduction through the CSC transpose)
-    gh = _new(h, n, H) if need_gh else None
+    gh = _new(h, n, f) if need_gh else None
     gx = _new(h, n, 3) if need_gx else None
     p_pre = _new(h, grid_n, 2 * H * f + H)
     (_C.egnn_node_pre_bwd_tc if tc else _C.egnn_node_pre_bwd)(gz1, gQ, gD, gxd, gx_out, gh_direct, g, h, W1, gh, gx, p_pre)
+    if g_attr is not None:
+        _C.egnn_edge_attr_grad(gz1, g, W1, f, g_attr, attr_accumulate)
     # deterministic reduction of the per-CTA weight-gradient partials
     r_post, r_edge, r_pre = _new(h, p_post.shape[1]), _new(h, p_edge.shape[1]), _new(h, p_pre.shape[1])
     _C.reduce_partials3((p_post, p_edge, p_pre), (r_post, r_edge, r_pre))
@@ -258,7 +262,9 @@ class _EGNNStack(torch.autograd.Function):
     """The whole ``for layer in self.GCN_layers`` loop (models/hybrid_models.py:89-90) as ONE autograd node:
     forward through the fused kernels (node side fused across layer boundaries on the tensor cores), backward
     layer by layer in reverse.  The last layer's coordinate branch is skipped, so its coord_mlp parameters get
-    ``None`` gradients exactly as in the reference.
+    ``None`` gradients exactly as in the reference.  Input gradients, as DGL's autograd gives them: ``x23`` [N, 23]
+    (residue features and coordinates) when it requires grad, ``edge_attr`` (summed over the layers) when it does;
+    neither costs anything when not requested.
 
     forward(graph, n_layers, x23, edge_attr, qkv_w, qkv_b, *flat_params) -> (h_final [N,64], QKV [N,192] or None)
 
@@ -302,13 +308,17 @@ class _EGNNStack(torch.autograd.Function):
             return (None,) * (6 + 11 * nl)
         gh = gh.contiguous()
         gx = None
+        need_x23 = ctx.needs_input_grad[2]
+        g_attr = _new(edge_attr, *edge_attr.shape) if ctx.needs_input_grad[3] else None
         for l in range(nl - 1, -1, -1):
             hl, xl, PQl, hnl, *pl = saved[1 + 15 * l:1 + 15 * (l + 1)]
-            need = l > 0                               # layer 0's inputs are data
-            gh, gx_in, gl = _egnn_layer_backward(ctx.graph, hl, xl, edge_attr, PQl, hnl, pl, gh, gx, need, need)
+            need = l > 0 or need_x23
+            gh, gx_in, gl = _egnn_layer_backward(ctx.graph, hl, xl, edge_attr, PQl, hnl, pl, gh, gx, need, need, g_attr,
+                                                 l != nl - 1)
             grads[11 * l:11 * l + 11] = gl
             gx = gx_in
-        return (None, None, None, None, gw, gb, *grads)
+        gx23 = torch.cat([gh, gx], 1) if need_x23 else None
+        return (None, None, gx23, g_attr, gw, gb, *grads)
 
 
 def egnn_stack(graph, x23, edge_attr, layer_params, qkv=None):

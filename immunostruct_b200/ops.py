@@ -324,30 +324,37 @@ def _(x23, edge_attr, params, graph, n_layers, n_edges, n_graphs, max_nodes, qkv
 
 @torch.library.custom_op("immunostruct_b200::egnn_stack_bwd", mutates_args=())
 def egnn_stack_bwd(gh: Tensor, edge_attr: Tensor, saved: List[Tensor], params: List[Tensor], graph: List[Tensor],
-                   n_layers: int, n_edges: int, n_graphs: int, max_nodes: int) -> List[Tensor]:
-    """-> 11 * n_layers parameter gradients (an empty tensor where the reference reports None: the last layer's coord_mlp)"""
+                   n_layers: int, n_edges: int, n_graphs: int, max_nodes: int, need_x23: bool,
+                   need_edge_attr: bool) -> List[Tensor]:
+    """-> 11 * n_layers parameter gradients (an empty tensor where the reference reports None: the last layer's coord_mlp),
+    then the gradients of x23 [N, 23] and of edge_attr (empty tensors where not requested)"""
     g = _graph_ns(graph, n_edges, n_graphs, max_nodes)
     edge_attr = edge_attr.contiguous()
     grads: list = [None] * (11 * n_layers)
     gx = None
+    g_attr = torch.empty_like(edge_attr) if need_edge_attr else None
     for l in range(n_layers - 1, -1, -1):
         hl, xl, pq, hn = saved[4 * l:4 * l + 4]
         pl = [t.contiguous() for t in params[11 * l:11 * l + 11]]
-        need = l > 0
-        gh, gx_in, gl = IF._egnn_layer_backward(g, hl, xl, edge_attr, pq, hn, pl, gh, gx, need, need)
+        need = l > 0 or need_x23
+        gh, gx_in, gl = IF._egnn_layer_backward(g, hl, xl, edge_attr, pq, hn, pl, gh, gx, need, need, g_attr,
+                                                l != n_layers - 1)
         grads[11 * l:11 * l + 11] = gl
         gx = gx_in
     # (the per-layer gradients are views of three reduction buffers, and registered operators may not return aliases --
     #  not even the same empty tensor twice)
-    return [edge_attr.new_empty(0) if t is None else t.clone() for t in grads]
+    out = [edge_attr.new_empty(0) if t is None else t.clone() for t in grads]
+    return out + [torch.cat([gh, gx], 1) if need_x23 else edge_attr.new_empty(0),
+                  g_attr if need_edge_attr else edge_attr.new_empty(0)]
 
 
 @egnn_stack_bwd.register_fake
-def _(gh, edge_attr, saved, params, graph, n_layers, n_edges, n_graphs, max_nodes):
+def _(gh, edge_attr, saved, params, graph, n_layers, n_edges, n_graphs, max_nodes, need_x23, need_edge_attr):
     out = [torch.empty_like(p) for p in params]
     for i in (4, 5, 6):                                  # the last layer's coord_mlp: no gradient
         out[11 * (n_layers - 1) + i] = gh.new_empty(0)
-    return out
+    return out + [gh.new_empty(gh.shape[0], 23) if need_x23 else gh.new_empty(0),
+                  torch.empty_like(edge_attr, memory_format=torch.contiguous_format) if need_edge_attr else gh.new_empty(0)]
 
 
 def _egnn_setup(ctx, inputs, output):
@@ -373,8 +380,11 @@ def _egnn_backward(ctx, grads):
         g_qkv_in = [gw, gb]
     if gh is None:
         return None, None, [None] * ctx.n_params, [None] * ctx.n_graph, None, None, None, None, g_qkv_in
-    gp = egnn_stack_bwd(gh.contiguous(), edge_attr, saved, params, graph, *ctx.cfg)
-    return (None, None, [None if g.numel() == 0 and p.numel() != 0 else g for g, p in zip(gp, params)], [None] * ctx.n_graph,
+    need_x23, need_attr = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
+    gp = egnn_stack_bwd(gh.contiguous(), edge_attr, saved, params, graph, *ctx.cfg, need_x23, need_attr)
+    gp, gx23, g_attr = gp[:ctx.n_params], gp[-2], gp[-1]
+    return (gx23 if need_x23 else None, g_attr if need_attr else None,
+            [None if g.numel() == 0 and p.numel() != 0 else g for g, p in zip(gp, params)], [None] * ctx.n_graph,
             None, None, None, None, g_qkv_in)
 
 

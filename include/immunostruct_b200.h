@@ -76,6 +76,8 @@ int is_egnn_node_post_pre_tc(const float* h, int64_t ldh, int F, const float* hn
                              float* PQn, int64_t n_nodes, int precision, int fast_act, int next_kind, void* stream);
 int is_egnn_node_post_fwd(const float* h, int64_t ldh, int F, const float* hn, const float* W5, const float* b5,
                           const float* W6, const float* b6, float* h_out, int64_t n_nodes, void* stream);
+/* gh_direct (the node_mlp's own gradient of h) and, in node_pre_bwd, gh (the gradient of the layer's input features) are
+ * [n_nodes, F] row-major or NULL: F = 64 for a hidden layer, F = 20 for layer 0 (input gradients, attribution). */
 int is_egnn_node_post_bwd(const float* gh_out, const float* h, int64_t ldh, int F, const float* hn,
                           const float* W5, const float* b5, const float* W6,
                           float* gh_direct, float* ghn, float* partials, int64_t n_nodes, void* stream);
@@ -120,6 +122,11 @@ int is_egnn_node_pre_bwd_tc(const float* gz1, const float* gQ, const float* gD, 
                          const float* gx_out, const float* gh_direct,
                          const int* outptr, const int* csc_pos, const float* h, int64_t ldh, int F,
                          const float* W1, float* gh, float* gx, float* partials, int64_t n_nodes, void* stream);
+/* gradient of the scalar edge features: g_attr[csr_eid[p]] = (accumulate ? g_attr[csr_eid[p]] : 0) + sum_k gz1[p,k] *
+ * W1[k, 2F+1] for every CSR position p.  gz1 [n_edges, 64] as written by the edge backward, g_attr [n_edges] in original
+ * edge order; one launch per layer (accumulate = 0 for the first), deterministic (no atomics). */
+int is_egnn_edge_attr_grad(const float* gz1, const int* csr_eid, const float* W1, int F, float* g_attr, int64_t n_edges,
+                           int accumulate, void* stream);
 int is_reduce_partials(const float* partials, int nparts, int64_t stride, float* out, void* stream);
 /* the three partial buffers of one layer's backward (node_post, edge, node_pre) reduced by one launch */
 int is_reduce_partials3(const float* p0, int n0, int64_t s0, float* o0, const float* p1, int n1, int64_t s1, float* o1,
