@@ -49,7 +49,7 @@ def exported_symbols():
             "is_segment_pool_fwd", "is_segment_pool_bwd", "is_contrastive_scratch_floats", "is_contrastive_fwd",
             "is_contrastive_bwd", "is_fused_adam", "is_rotate_coords", "is_mask_single_residue", "is_mask_rows", "is_gemm_tma_split_k",
             "is_split_planes", "is_gemm_planes_tma", "is_egnn_set_ws_buffers", "is_egnn_set_ws_variant", "is_reduce_partials3", "is_fused_adam_capturable",
-            "is_egnn_edge_attr_grad"]
+            "is_egnn_edge_attr_grad", "is_head_mc_infer"]
 
 
 def _check(rc: int, name: str):
@@ -115,7 +115,7 @@ def _current_device():
 _FN = {}              # launcher name -> ctypes function (restype set once)
 LAUNCHES = 0          # number of immunostruct_b200 kernels enqueued so far (bench.py reports the delta)
 _KERNELS_PER_CALL = {"is_collate_csr": 1, "is_egnn_edge_bwd_ws": 2, "is_loss_fwd": 2, "is_loss_bwd": 2, "is_contrastive_fwd": 9,
-                     "is_contrastive_bwd": 9}
+                     "is_contrastive_bwd": 9, "is_head_mc_infer": 2}
 
 
 def _call(name, *args):
@@ -471,6 +471,38 @@ def head_infer(pooled, Wc, bc, z_vae, coef, n_head, W1, b1, W2, b2):
           _t(coef, f32, "coef"), _i32(n_head), _t(W1, f32, "W1"), _t(b1, f32, "b1"), _t(W2, f32, "W2"), _t(b2, f32, "b2"),
           _i32(n_out), _t(x_gat, f32, "x_gat"), _t(out, f32, "out"), _i32(b), _stream())
     return x_gat, out
+
+
+def head_mc_infer(items, Wc, bc, coef, n_head, W1, b1, W2, b2):
+    """The eval-mode head over K reparameterisation draws (csrc/head.cu).  ``items``: one (pooled [B,64], mu [B,LD],
+    logvar [B,LD], z_vae [B,LD+PD], eps [K,B,LD]) tuple, or two for a cancer / wild-type pair (tokens item-major).
+    -> (logits [B,K], prob_mean [B], prob_std [B])."""
+    f32 = torch.float32
+    if len(items) not in (1, 2) or any(len(it) != 5 for it in items):
+        raise ValueError("head_mc_infer: one or two (pooled, mu, logvar, z_vae, eps) items")
+    b, ld = items[0][1].shape
+    k, lz = items[0][4].shape[0], items[0][3].shape[1]
+    for pooled, mu, logvar, zv, eps in items:
+        if (pooled.shape != (b, 64) or mu.shape != (b, ld) or logvar.shape != (b, ld) or zv.shape != (b, lz)
+                or eps.shape != (k, b, ld)):
+            raise ValueError("head_mc_infer: unexpected item shapes")
+    L = len(items) * (64 + lz)
+    if W1.shape != (32, L) or b1.shape != (32,) or W2.shape != (1, 32) or b2.shape != (1,) or lz < ld or L > 256:
+        raise ValueError("head_mc_infer: unexpected classifier shapes")
+    if (Wc is None) != (bc is None) or (Wc is not None and (Wc.shape != (64, 64) or bc.shape != (64,))):
+        raise ValueError("head_mc_infer: Wc / bc must both be None or [64,64] / [64]")
+    if coef is not None and (not 1 <= n_head <= 8 or coef.shape != (4 * n_head + 1,)):
+        raise ValueError("head_mc_infer: coef must hold 4 n_head + 1 values, 1 <= n_head <= 8")
+    dev = items[0][0].device
+    logits = torch.empty(b, k, dtype=f32, device=dev)
+    mean, std = torch.empty(b, dtype=f32, device=dev), torch.empty(b, dtype=f32, device=dev)
+    names = ("pooled", "mu", "logvar", "z_vae", "eps")
+    ptrs = [_t(t, f32, f"{n}{i}") for i, it in enumerate((items[0], items[1] if len(items) == 2 else (None,) * 5))
+            for t, n in zip(it, names)]
+    _call("is_head_mc_infer", *ptrs, _i32(len(items)), _i32(ld), _i32(lz - ld), _t(Wc, f32, "Wc"), _t(bc, f32, "bc"),
+          _t(coef, f32, "coef"), _i32(n_head), _t(W1, f32, "W1"), _t(b1, f32, "b1"), _t(W2, f32, "W2"), _t(b2, f32, "b2"),
+          _t(logits, f32, "logits"), _t(mean, f32, "prob_mean"), _t(std, f32, "prob_std"), _i32(b), _i32(k), _stream())
+    return logits, mean, std
 
 
 def unpack_nodes(aa, xyz, x):

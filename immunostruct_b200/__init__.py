@@ -12,7 +12,7 @@ from .packed import PackedGraphBatch, PackedGraphDataset, PackedSequence, pack_g
 from .optim import FusedAdam, FusedAdamW  # noqa: F401
 from .augment import TrainAugment  # noqa: F401
 from .graphed import CapturedStep  # noqa: F401
-from . import attribution, augment, dataloading, nn, optim, ops  # noqa: F401
+from . import attribution, augment, dataloading, nn, optim, ops, predictive  # noqa: F401
 from .ops import use_custom_ops  # noqa: F401
 from .functional import invalidate_caches  # noqa: F401
 

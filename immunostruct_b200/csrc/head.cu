@@ -130,6 +130,66 @@ vae_mid_infer_kernel(const float* __restrict__ h1, const float* __restrict__ pro
     }
 }
 
+// ---- head: shared arithmetic of head_infer and head_mc_infer ------------------------------------------------------
+// One copy of every rounding step, so that draw k of head_mc_infer is bit-identical to head_infer run on that draw.
+
+// x_gat row o = Wc[o] . pooled + bc[o], one warp: lanes over the 64 inputs (p0 = pooled[lane], p1 = pooled[32 + lane])
+__device__ __forceinline__ float head_xgat_row(const float* __restrict__ Wc, const float* __restrict__ bc, int o, float p0,
+                                               float p1, int lane) {
+    const float a = fmaf(__ldg(Wc + o * 64 + 32 + lane), p1, __ldg(Wc + o * 64 + lane) * p0);
+    return warp_sum(a) + __ldg(bc + o);
+}
+
+// closed-form fusion attention (fusion.cu): expectation of token i under head h over the L scalars c, whose extremes are
+// cmax / cmin.  Inference only: 2^(g2 c_j - m2) with ex2.approx, g2 = gamma log2 e (one FFMA + one MUFU per term; the
+// rounding of g2 moves an exponent of magnitude <= ~20 by ~1e-6, an order below the 1e-5 parity bound, as in the fast SiLU
+// of the inference EGNN kernels); two independent accumulator pairs
+__device__ __forceinline__ float head_fusion_expect(const float* c, int L, int i, const float* __restrict__ coef, int H, int h,
+                                                    float cmax, float cmin) {
+    const float gamma = coef[h] * c[i] + coef[H + h];
+    const float g2 = gamma * 1.4426950408889634f;
+    const float m2 = gamma > 0.0f ? g2 * cmax : g2 * cmin;
+    float Z0 = 0.0f, S0 = 0.0f, Z1 = 0.0f, S1 = 0.0f;
+    int j = 0;
+    for (; j + 1 < L; j += 2) {
+        const float c0 = c[j], c1 = c[j + 1];
+        float e0, e1;
+        asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e0) : "f"(fmaf(g2, c0, -m2)));
+        asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e1) : "f"(fmaf(g2, c1, -m2)));
+        Z0 += e0; S0 = fmaf(e0, c0, S0);
+        Z1 += e1; S1 = fmaf(e1, c1, S1);
+    }
+    if (j < L) {
+        const float c0 = c[j];
+        float e0;
+        asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e0) : "f"(fmaf(g2, c0, -m2)));
+        Z0 += e0; S0 = fmaf(e0, c0, S0);
+    }
+    return (S0 + S1) / (Z0 + Z1);
+}
+
+// fused feature of one token from its H head expectations Eh[0..H)
+__device__ __forceinline__ float head_fusion_out(const float* Eh, const float* __restrict__ coef, int H) {
+    float o = coef[4 * H];
+    for (int h = 0; h < H; ++h) o += coef[2 * H + h] * Eh[h] + coef[3 * H + h];
+    return o;
+}
+
+// classifier hidden unit o = relu(W1[o] . f + b1[o]), one warp: lanes strided over the L features
+__device__ __forceinline__ float head_hidden_row(const float* __restrict__ W1, const float* __restrict__ b1, const float* f,
+                                                 int L, int o, int lane) {
+    float a = 0.0f;
+    for (int k = lane; k < L; k += 32) a = fmaf(__ldg(W1 + o * L + k), f[k], a);
+    a = warp_sum(a);
+    return fmaxf(a + __ldg(b1 + o), 0.0f);
+}
+
+// classifier output r = W2[r] . hid + b2[r], one warp (lane = hidden unit)
+__device__ __forceinline__ float head_out_row(const float* __restrict__ W2, const float* __restrict__ b2, const float* hid,
+                                              int r, int lane) {
+    return warp_sum(__ldg(W2 + r * 32 + lane) * hid[lane]) + __ldg(b2 + r);
+}
+
 // ---- head: one CTA per sample ------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(IS_THREADS)
 head_infer_kernel(const float* __restrict__ pooled, const float* __restrict__ Wc, const float* __restrict__ bc,
@@ -148,9 +208,8 @@ head_infer_kernel(const float* __restrict__ pooled, const float* __restrict__ Wc
     if (Wc != nullptr) {
         const float p0 = __ldg(pooled + (int64_t)b * 64 + lane), p1 = __ldg(pooled + (int64_t)b * 64 + 32 + lane);
         for (int o = warp; o < 64; o += IS_THREADS / 32) {
-            float a = fmaf(__ldg(Wc + o * 64 + 32 + lane), p1, __ldg(Wc + o * 64 + lane) * p0);
-            a = warp_sum(a);
-            if (lane == 0) c[o] = a + __ldg(bc + o);
+            const float a = head_xgat_row(Wc, bc, o, p0, p1, lane);
+            if (lane == 0) c[o] = a;
         }
     } else if (tid < 64) {
         c[tid] = __ldg(pooled + (int64_t)b * 64 + tid);
@@ -174,55 +233,147 @@ head_infer_kernel(const float* __restrict__ pooled, const float* __restrict__ Wc
         const float cmax = s_mm[0], cmin = s_mm[1];
         for (int idx = tid; idx < L * H; idx += IS_THREADS) {
             const int i = idx / H, h = idx - i * H;
-            const float gamma = coef[h] * c[i] + coef[H + h];
-            // inference-only kernel: 2^(g2 c_j - m2) with ex2.approx, g2 = gamma log2 e (one FFMA + one MUFU per term; the
-            // rounding of g2 moves an exponent of magnitude <= ~20 by ~1e-6, an order below the 1e-5 parity bound, as in the
-            // fast SiLU of the inference EGNN kernels); two independent accumulator pairs
-            const float g2 = gamma * 1.4426950408889634f;
-            const float m2 = gamma > 0.0f ? g2 * cmax : g2 * cmin;
-            float Z0 = 0.0f, S0 = 0.0f, Z1 = 0.0f, S1 = 0.0f;
-            int j = 0;
-            for (; j + 1 < L; j += 2) {
-                const float c0 = c[j], c1 = c[j + 1];
-                float e0, e1;
-                asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e0) : "f"(fmaf(g2, c0, -m2)));
-                asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e1) : "f"(fmaf(g2, c1, -m2)));
-                Z0 += e0; S0 = fmaf(e0, c0, S0);
-                Z1 += e1; S1 = fmaf(e1, c1, S1);
-            }
-            if (j < L) {
-                const float c0 = c[j];
-                float e0;
-                asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e0) : "f"(fmaf(g2, c0, -m2)));
-                Z0 += e0; S0 = fmaf(e0, c0, S0);
-            }
-            Eh[idx] = (S0 + S1) / (Z0 + Z1);
+            Eh[idx] = head_fusion_expect(c, L, i, coef, H, h, cmax, cmin);
         }
         __syncthreads();
-        for (int i = tid; i < L; i += IS_THREADS) {
-            float o = coef[4 * H];
-            for (int h = 0; h < H; ++h) o += coef[2 * H + h] * Eh[i * H + h] + coef[3 * H + h];
-            f[i] = o;
-        }
+        for (int i = tid; i < L; i += IS_THREADS) f[i] = head_fusion_out(Eh + i * H, coef, H);
     } else {
         for (int i = tid; i < L; i += IS_THREADS) f[i] = c[i];
     }
     __syncthreads();
     // classifier: hid = relu(W1 f + b1) (32 rows, warp per 4 rows), out = W2 hid + b2 (or hid itself)
     for (int o = warp; o < 32; o += IS_THREADS / 32) {
-        float a = 0.0f;
-        for (int k = lane; k < L; k += 32) a = fmaf(__ldg(W1 + o * L + k), f[k], a);
-        a = warp_sum(a);
-        if (lane == 0) hid[o] = fmaxf(a + __ldg(b1 + o), 0.0f);
+        const float a = head_hidden_row(W1, b1, f, L, o, lane);
+        if (lane == 0) hid[o] = a;
     }
     __syncthreads();
     if (W2 != nullptr) {
         if (warp < n_out) {
-            float a = warp_sum(__ldg(W2 + warp * 32 + lane) * hid[lane]);
-            if (lane == 0) out[(int64_t)b * n_out + warp] = a + __ldg(b2 + warp);
+            const float a = head_out_row(W2, b2, hid, warp, lane);
+            if (lane == 0) out[(int64_t)b * n_out + warp] = a;
         }
     } else if (tid < 32) {
         out[(int64_t)b * 32 + tid] = hid[tid];
+    }
+}
+
+// ---- head over many reparameterisation draws: one CTA per (sample, chunk of MC_DRAWS draws) ----------------------
+// The tokens of one item are [x_gat | z | prop] (64 + LD + PD); only z = mu + eps exp(0.5 logvar) depends on the draw.
+// x_gat, mu, exp(0.5 logvar) and prop are computed once per CTA; the (draw, token, head) fusion work and the (draw, row)
+// classifier rows are spread over the whole CTA.  A logit depends on (sample, eps[k]) only, never on the chunking.
+constexpr int MC_DRAWS = 8;      // = warps per CTA: one warp per draw for the extremes and the output row
+
+struct McItem {
+    const float* pooled;         // [B, 64]
+    const float* mu;             // [B, LD]
+    const float* logvar;         // [B, LD]
+    const float* zv;             // [B, LD + PD] (the PD property columns are read)
+    const float* eps;            // [K, B, LD]
+};
+
+__global__ void __launch_bounds__(IS_THREADS)
+head_mc_infer_kernel(McItem it0, McItem it1, int n_items, int LD, int PD, const float* __restrict__ Wc,
+                     const float* __restrict__ bc, const float* __restrict__ coef, int H, const float* __restrict__ W1,
+                     const float* __restrict__ b1, const float* __restrict__ W2, const float* __restrict__ b2,
+                     float* __restrict__ logits, int B, int K, int n_chunks, int kc_max) {
+    extern __shared__ __align__(16) float sm[];
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int LZ = LD + PD, LI = 64 + LZ, L = n_items * LI, LH = coef != nullptr ? L * H : 0;
+    const int b = blockIdx.x / n_chunks, k0 = (blockIdx.x - b * n_chunks) * MC_DRAWS;
+    const int kc = min(MC_DRAWS, K - k0);
+    float* base = sm;                       // [L] draw-independent tokens (the z slots hold mu)
+    float* sdev = base + L;                 // [2][LD] exp(0.5 logvar)
+    float* c = sdev + 2 * LD;               // [kc_max][L] tokens of each draw
+    float* f = c + kc_max * L;              // [kc_max][L] fused features
+    float* hid = f + kc_max * L;            // [kc_max][32]
+    float* mm = hid + kc_max * 32;          // [kc_max][2] extremes of c
+    float* Eh = mm + kc_max * 2;            // [kc_max][L][H]
+    for (int r = warp; r < n_items * 64; r += IS_THREADS / 32) {
+        const int it = r >> 6, o = r & 63;
+        const float* pooled = (it ? it1 : it0).pooled + (int64_t)b * 64;
+        if (Wc != nullptr) {
+            const float a = head_xgat_row(Wc, bc, o, __ldg(pooled + lane), __ldg(pooled + 32 + lane), lane);
+            if (lane == 0) base[it * LI + o] = a;
+        } else if (lane == 0) {
+            base[it * LI + o] = __ldg(pooled + o);
+        }
+    }
+    for (int idx = tid; idx < n_items * LZ; idx += IS_THREADS) {
+        const int it = idx >= LZ, t = idx - it * LZ;
+        const McItem& m = it ? it1 : it0;
+        if (t < LD) {
+            base[it * LI + 64 + t] = __ldg(m.mu + (int64_t)b * LD + t);
+            sdev[it * LD + t] = expf(0.5f * __ldg(m.logvar + (int64_t)b * LD + t));
+        } else {
+            base[it * LI + 64 + t] = __ldg(m.zv + (int64_t)b * LZ + t);
+        }
+    }
+    __syncthreads();
+    // z = fmaf(eps, exp(0.5 logvar), mu): the arithmetic of vae_mid_infer_kernel
+    for (int idx = tid; idx < kc * L; idx += IS_THREADS) {
+        const int d = idx / L, t = idx - d * L, it = t >= LI, u = t - it * LI - 64;
+        float v = base[t];
+        if (u >= 0 && u < LD)
+            v = fmaf(__ldg((it ? it1 : it0).eps + ((int64_t)(k0 + d) * B + b) * LD + u), sdev[it * LD + u], v);
+        c[idx] = v;
+    }
+    __syncthreads();
+    const float* feat = c;
+    if (coef != nullptr) {
+        if (warp < kc) {
+            float lmax = -INFINITY, lmin = INFINITY;
+            for (int i = lane; i < L; i += 32) { lmax = fmaxf(lmax, c[warp * L + i]); lmin = fminf(lmin, c[warp * L + i]); }
+            lmax = warp_max(lmax); lmin = -warp_max(-lmin);
+            if (lane == 0) { mm[2 * warp] = lmax; mm[2 * warp + 1] = lmin; }
+        }
+        __syncthreads();
+        for (int idx = tid; idx < kc * LH; idx += IS_THREADS) {
+            const int d = idx / LH, r = idx - d * LH, i = r / H, h = r - i * H;
+            Eh[idx] = head_fusion_expect(c + d * L, L, i, coef, H, h, mm[2 * d], mm[2 * d + 1]);
+        }
+        __syncthreads();
+        for (int idx = tid; idx < kc * L; idx += IS_THREADS) f[idx] = head_fusion_out(Eh + idx * H, coef, H);
+        __syncthreads();
+        feat = f;
+    }
+    for (int r = warp; r < kc * 32; r += IS_THREADS / 32) {
+        const int d = r >> 5, o = r & 31;
+        const float a = head_hidden_row(W1, b1, feat + d * L, L, o, lane);
+        if (lane == 0) hid[r] = a;
+    }
+    __syncthreads();
+    if (warp < kc) {
+        const float a = head_out_row(W2, b2, hid + warp * 32, 0, lane);
+        if (lane == 0) logits[(int64_t)b * K + k0 + warp] = a;
+    }
+}
+
+// mean and population standard deviation of sigmoid(logit) over the K draws of each sample: one warp per sample, lanes
+// strided over the draws, fp64, two passes, fixed butterfly order (no atomics: the result depends on the logits only)
+__device__ __forceinline__ double warp_sum_f64(double v) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    return v;
+}
+
+__global__ void __launch_bounds__(IS_THREADS)
+head_mc_stats_kernel(const float* __restrict__ logits, int B, int K, float* __restrict__ prob_mean,
+                     float* __restrict__ prob_std) {
+    const int b = blockIdx.x * (IS_THREADS / 32) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    if (b >= B) return;
+    const float* row = logits + (int64_t)b * K;
+    double s = 0.0;
+    for (int k = lane; k < K; k += 32) s += 1.0 / (1.0 + exp(-(double)__ldg(row + k)));
+    const double mean = warp_sum_f64(s) / K;
+    double v = 0.0;
+    for (int k = lane; k < K; k += 32) {
+        const double p = 1.0 / (1.0 + exp(-(double)__ldg(row + k))) - mean;
+        v = fma(p, p, v);
+    }
+    const double var = warp_sum_f64(v) / K;
+    if (lane == 0) {
+        prob_mean[b] = (float)mean;
+        prob_std[b] = (float)sqrt(var);
     }
 }
 
@@ -263,6 +414,40 @@ int is_head_infer(const float* pooled, const float* Wc, const float* bc, const f
     if (W2 != nullptr && (n_out < 1 || n_out > 8)) return IS_ERR_ARG;
     head_infer_kernel<<<n_samples, IS_THREADS, 0, (cudaStream_t)stream>>>(pooled, Wc, bc, z_vae, LZ, coef, n_head, W1, b1, W2, b2,
                                                                           x_gat, out, n_out);
+    IS_LAUNCH_CHECK();
+    return IS_OK;
+}
+
+// K reparameterisation draws of the eval-mode head for B samples (see head_mc_infer_kernel): item i = (pooled_i [B,64],
+// mu_i / logvar_i [B,LD], z_vae_i [B,LD+PD] (property columns), eps_i [K,B,LD]); the tokens are item-major
+// [x_gat_0 | z_0 | prop_0 | x_gat_1 | ...] (L = n_items (64+LD+PD) <= IS_HEAD_LMAX); Wc / bc, coef and the classifier as
+// in is_head_infer, W2 [1,32] / b2 [1] required.  -> logits [B,K] (sample-major), prob_mean / prob_std [B] (mean and
+// population standard deviation of sigmoid(logit) over the draws).  Two kernels: the draws, then the statistics.
+int is_head_mc_infer(const float* pooled0, const float* mu0, const float* logvar0, const float* z_vae0, const float* eps0,
+                     const float* pooled1, const float* mu1, const float* logvar1, const float* z_vae1, const float* eps1,
+                     int n_items, int latent, int prop_dim, const float* Wc, const float* bc, const float* coef, int n_head,
+                     const float* W1, const float* b1, const float* W2, const float* b2, float* logits, float* prob_mean,
+                     float* prob_std, int n_samples, int n_draws, void* stream) {
+    if (n_samples <= 0 || n_draws <= 0 || latent <= 0 || prop_dim < 0 || (n_items != 1 && n_items != 2)) return IS_ERR_ARG;
+    if (n_items * (64 + latent + prop_dim) > IS_HEAD_LMAX) return IS_ERR_ARG;
+    if (coef != nullptr && (n_head < 1 || n_head > IS_HEAD_HMAX)) return IS_ERR_ARG;
+    if ((Wc == nullptr) != (bc == nullptr) || !W1 || !b1 || !W2 || !b2 || !logits || !prob_mean || !prob_std) return IS_ERR_ARG;
+    if (!pooled0 || !mu0 || !logvar0 || !z_vae0 || !eps0) return IS_ERR_ARG;
+    if (n_items == 2 && (!pooled1 || !mu1 || !logvar1 || !z_vae1 || !eps1)) return IS_ERR_ARG;
+    const int n_chunks = (n_draws + MC_DRAWS - 1) / MC_DRAWS, kc_max = n_draws < MC_DRAWS ? n_draws : MC_DRAWS;
+    if ((int64_t)n_samples * n_chunks > 0x7fffffff) return IS_ERR_UNSUPPORTED;
+    const int L = n_items * (64 + latent + prop_dim), H = coef != nullptr ? n_head : 0;
+    const size_t smem = sizeof(float) * ((size_t)L + 2 * latent + (size_t)kc_max * (2 * L + 32 + 2 + L * H));
+    if (smem > 227 * 1024) return IS_ERR_UNSUPPORTED;
+    cudaError_t e = cudaFuncSetAttribute(head_mc_infer_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return (int)e;
+    const McItem it0{pooled0, mu0, logvar0, z_vae0, eps0};
+    const McItem it1 = n_items == 2 ? McItem{pooled1, mu1, logvar1, z_vae1, eps1} : it0;
+    head_mc_infer_kernel<<<n_samples * n_chunks, IS_THREADS, smem, (cudaStream_t)stream>>>(
+        it0, it1, n_items, latent, prop_dim, Wc, bc, coef, n_head, W1, b1, W2, b2, logits, n_samples, n_draws, n_chunks, kc_max);
+    IS_LAUNCH_CHECK();
+    head_mc_stats_kernel<<<(n_samples + IS_THREADS / 32 - 1) / (IS_THREADS / 32), IS_THREADS, 0, (cudaStream_t)stream>>>(
+        logits, n_samples, n_draws, prob_mean, prob_std);
     IS_LAUNCH_CHECK();
     return IS_OK;
 }

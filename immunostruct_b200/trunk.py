@@ -117,12 +117,17 @@ class SequenceVAE:
         ``reparameterize`` (one standard-normal [B, latent] tensor).  -> (recon, mu, logvar, z_vae)."""
         h1 = _tc_linear(self.vae_fc1, sequence_data.reshape(-1, self.vae_input_dim), relu=True)
         eps = self.sample_eps(torch.empty(h1.shape[0], self.vae_latent_dim, dtype=h1.dtype, device=h1.device)).contiguous()
+        mu, logvar, z_vae, h3 = self.vae_mid_eval(h1, prop_mlp, peptide_property, eps)
+        return _tc_linear(self.vae_fc4, h3), mu, logvar, z_vae
+
+    def vae_mid_eval(self, h1, prop_mlp, peptide_property, eps):
+        """Property MLP, vae_fc21 / fc22, reparameterisation with ``eps`` [B, latent] and vae_fc3 + ReLU in one kernel
+        (csrc/head.cu, no autograd).  -> (mu, logvar, z_vae, h3)."""
         d = lambda t: t.detach()
-        mu, logvar, z_vae, h3 = IF._C.vae_mid_infer(
+        return IF._C.vae_mid_infer(
             h1, peptide_property.contiguous(), eps, d(prop_mlp[0].weight), d(prop_mlp[0].bias), d(prop_mlp[3].weight),
             d(prop_mlp[3].bias), d(self.vae_fc21.weight), d(self.vae_fc21.bias), d(self.vae_fc22.weight),
             d(self.vae_fc22.bias), d(self.vae_fc3.weight), d(self.vae_fc3.bias))
-        return _tc_linear(self.vae_fc4, h3), mu, logvar, z_vae
 
     def vae_branch(self, sequence_data, cond=None):
         mu, logvar = self.encode_vae(sequence_data.reshape(-1, self.vae_input_dim))

@@ -195,6 +195,18 @@ int is_vae_mid_infer(const float* h1, const float* prop, const float* eps, const
 int is_head_infer(const float* pooled, const float* Wc, const float* bc, const float* z_vae, int LZ, const float* coef,
                   int n_head, const float* W1, const float* b1, const float* W2, const float* b2, int n_out,
                   float* x_gat, float* out, int n_samples, void* stream);
+/* is_head_mc_infer: the head of is_head_infer (W2 [1,32] / b2 [1] required) for K reparameterisation draws of B samples.
+ * Item i (n_items 1, or 2 for a cancer / wild-type pair) supplies pooled_i [B,64], mu_i / logvar_i [B,latent], z_vae_i
+ * [B,latent+prop_dim] (only its property columns are read) and eps_i [K,B,latent]; z_i = mu_i + eps_i[k] exp(0.5
+ * logvar_i) with the arithmetic of is_vae_mid_infer, tokens item-major [x_gat_0 | z_0 | prop_0 | x_gat_1 | ...] (at most
+ * 256).  Draw k is bit-identical to is_head_infer on that draw.  -> logits [B,K], prob_mean / prob_std [B] (mean and
+ * population standard deviation of sigmoid(logit) over the draws, fp64 accumulation in a fixed order, no atomics).
+ * Item 1's pointers are ignored when n_items = 1. */
+int is_head_mc_infer(const float* pooled0, const float* mu0, const float* logvar0, const float* z_vae0, const float* eps0,
+                     const float* pooled1, const float* mu1, const float* logvar1, const float* z_vae1, const float* eps1,
+                     int n_items, int latent, int prop_dim, const float* Wc, const float* bc, const float* coef, int n_head,
+                     const float* W1, const float* b1, const float* W2, const float* b2, float* logits, float* prob_mean,
+                     float* prob_std, int n_samples, int n_draws, void* stream);
 /* Dense Linear layer on the tensor cores: C[M,N] = act(A[M,K] W[N,K]^T + bias), fp32 in / out, operands split
  * on the fly into three bf16 terms (precision 3, fp32-accurate) or rounded to bf16 (precision 0).  Replaces the
  * nn.Linear layers of the sequence VAE (reference models/hybrid_models.py:63-74: vae_fc1 with ReLU, vae_fc4) in the
