@@ -88,7 +88,7 @@ def test_structure_v2_golden():
     assert_grads_close(named_grads(model), gd["grads"], TOL)
 
 
-def _bench_shape_case(b, seed, n_pad=0, scale=1.0):
+def _bench_shape_case(b, seed, n_pad=0, scale=1.0, device=DEV):
     """HybridModelv2 at the BASELINE shape with default initialisation (at 200 nodes / in-degree 10 the
     logits already differ between graphs in the 2nd digit; scaling the EGNN weights up saturates the
     per-graph softmax and, from about 2x, overflows fp32 through the six un-normalised
@@ -96,7 +96,7 @@ def _bench_shape_case(b, seed, n_pad=0, scale=1.0):
     arr = synthetic_graph_arrays(b, 200, 10, seed=seed, n_pad=n_pad)
     dense = synthetic_dense(b, seed=seed)
     torch.manual_seed(seed)
-    model = I.model_map["HybridModelv2"](vae_input_dim=5943, device=DEV)
+    model = I.model_map["HybridModelv2"](vae_input_dim=5943, device=device)
     with torch.no_grad():
         for k, p in model.named_parameters():
             if k.startswith("GCN_layers") and k.endswith("weight"):
