@@ -49,7 +49,7 @@ def exported_symbols():
             "is_segment_pool_fwd", "is_segment_pool_bwd", "is_contrastive_scratch_floats", "is_contrastive_fwd",
             "is_contrastive_bwd", "is_fused_adam", "is_rotate_coords", "is_mask_single_residue", "is_mask_rows", "is_gemm_tma_split_k",
             "is_split_planes", "is_gemm_planes_tma", "is_egnn_set_ws_buffers", "is_egnn_set_ws_variant", "is_reduce_partials3", "is_fused_adam_capturable",
-            "is_egnn_edge_attr_grad", "is_head_mc_infer"]
+            "is_egnn_edge_attr_grad", "is_head_mc_infer", "is_mutscan_expand"]
 
 
 def _check(rc: int, name: str):
@@ -503,6 +503,29 @@ def head_mc_infer(items, Wc, bc, coef, n_head, W1, b1, W2, b2):
           _t(coef, f32, "coef"), _i32(n_head), _t(W1, f32, "W1"), _t(b1, f32, "b1"), _t(W2, f32, "W2"), _t(b2, f32, "b2"),
           _t(logits, f32, "logits"), _t(mean, f32, "prob_mean"), _t(std, f32, "prob_std"), _i32(b), _i32(k), _stream())
     return logits, mean, std
+
+
+def mutscan_expand(x23, node_off, node_index, seq, seq_index, seq_columns, sites, x23_out, seq_out, flag):
+    """One pass of an in-silico saturation scan (csrc/mutscan.cu): x23_out [r*N, 23] and seq_out [r*B, L, V] become r copies
+    of the base batch, copy k with the substitution sites[k] = (site p, residue column c) at node row node_off[b] +
+    node_index[b, p] and sequence row seq_index[b, p] of every sample b (-1 = absent site).  ``flag`` (int32 [1], zeroed by
+    the caller) is raised if a site row is not exactly one-hot or does not follow ``seq_columns``."""
+    f32, i64, i32 = torch.float32, torch.int64, torch.int32
+    if node_index.dim() != 2 or seq.dim() != 3 or x23.dim() != 2 or sites.dim() != 2:
+        raise ValueError("mutscan_expand: node_index [B,P], seq [B,L,V], x23 [N,23] and sites [r,2] expected")
+    b, p = node_index.shape
+    n, (_, L, V), r = x23.shape[0], seq.shape, sites.shape[0]
+    if (x23.shape[1] != 23 or node_off.shape != (b + 1,) or seq_index.shape != (b, p) or seq.shape[0] != b
+            or seq_columns.shape != (20,) or sites.shape[1] != 2 or r < 1 or p < 1):
+        raise ValueError("mutscan_expand: unexpected input shapes")
+    if x23_out.shape != (r * n, 23) or seq_out.shape != (r * b, L, V) or flag.shape != (1,):
+        raise ValueError("mutscan_expand: unexpected output shapes")
+    if r * b > 0x3fffffff or L * V > 0x7fffffff:
+        raise ValueError("mutscan_expand: r * B or L * V too large")
+    _call("is_mutscan_expand", _t(x23, f32, "x23"), _t(node_off, i64, "node_off"), _t(node_index, i64, "node_index"),
+          _t(seq, f32, "seq"), _t(seq_index, i64, "seq_index"), _t(seq_columns, i64, "seq_columns"), _t(sites, i32, "sites"),
+          _i32(r), _i32(b), _i32(p), _i64(n), _i32(L), _i32(V), _t(x23_out, f32, "x23_out"), _t(seq_out, f32, "seq_out"),
+          _t(flag, i32, "flag"), _stream())
 
 
 def unpack_nodes(aa, xyz, x):

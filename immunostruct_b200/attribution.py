@@ -38,16 +38,6 @@ class Attribution:
     completeness_gap: Tensor               # [B]
 
 
-def _replicate(graph: GraphBatch, r: int) -> GraphBatch:
-    """``r`` copies of the batch, collated on its device (the copies' features are replaced per pass)."""
-    ea = graph.edata["edge_attr"]
-    out = GraphBatch(graph.ndata["x"].detach().repeat(r, 1), graph._src_local.repeat(r), graph._dst_local.repeat(r),
-                     ea.detach().repeat(r, *([1] * (ea.dim() - 1))), graph._node_counts.repeat(r),
-                     graph._edge_counts.repeat(r), max_nodes=graph.max_nodes, collate_now=False)
-    out._collate()
-    return out
-
-
 def integrated_gradients(model, graph_data: GraphBatch, sequence_data: Optional[Tensor], peptide_property: Optional[Tensor],
                          *, steps: int = 32, eps: Optional[Tensor] = None, max_graphs: int = 4096) -> Attribution:
     """Integrated-gradients attribution of ``model(graph_data, sequence_data, peptide_property)[3]`` (the logit) to the 20
@@ -76,7 +66,7 @@ def integrated_gradients(model, graph_data: GraphBatch, sequence_data: Optional[
         to (x23, edge_attr, sequence, property) summed over the points (None where unused)."""
         r = len(alphas)
         if r not in graphs:
-            g = _replicate(graph_data, r)
+            g = graph_data.replicate(r)
             graphs[r] = (g, g.ndata["x"])
         g, x_rep = graphs[r]
         a = torch.tensor(alphas, dtype=x.dtype, device=dev)

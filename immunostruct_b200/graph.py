@@ -199,6 +199,16 @@ class GraphBatch:
         _raise_on_stats(max_deg, bad, max_nodes, n_empty, int(self.status.item()), self.max_nodes)
         return self
 
+    def replicate(self, r: int) -> "GraphBatch":
+        """``r`` copies of the batch, one after another, collated on its device (features detached; callers that evaluate
+        many variants of one batch replace the copies' features and keep the topology)."""
+        ea = self.edata["edge_attr"]
+        out = GraphBatch(self.ndata["x"].detach().repeat(r, 1), self._src_local.repeat(r), self._dst_local.repeat(r),
+                         ea.detach().repeat(r, *([1] * (ea.dim() - 1))), self._node_counts.repeat(r),
+                         self._edge_counts.repeat(r), max_nodes=self.max_nodes, collate_now=False)
+        out._collate()
+        return out
+
     # ---- DGL vocabulary -------------------------------------------------------------------------
     @property
     def device(self):

@@ -84,6 +84,18 @@ def _check(model, samples, kinds, what, names):
         raise ValueError("samples must be >= 1")
 
 
+def _pair_items(model, eps):
+    """Number of items the pair head reads (2 with ``use_wt_for_downstream``, else 1), after checking eps = (eps_c, eps_w)."""
+    if eps is not None and (not isinstance(eps, (tuple, list)) or len(eps) != 2):
+        raise ValueError("eps must be a pair (eps_c, eps_w)")
+    n = 2 if model.use_wt_for_downstream else 1
+    if eps is not None and any(e is None for e in eps[:n]):
+        raise ValueError("eps needs eps_c, and eps_w when use_wt_for_downstream is set")
+    if eps is not None and n == 2 and eps[0].shape[:1] != eps[1].shape[:1]:
+        raise ValueError("eps_c and eps_w must hold the same number of draws")
+    return n
+
+
 def predictive(model, graph_data, sequence_data, peptide_property, *, samples: int = 32,
                eps: Optional[Tensor] = None) -> Predictive:
     """K draws of ``model(graph_data, sequence_data, peptide_property)[3]`` (the logit), with K = ``samples`` or
@@ -117,13 +129,7 @@ def predictive_pair(model, graph_pair, sequence_pair, property_pair, *, samples:
     numbers that K sequential forwards would consume, only numbers of the same distribution.  Eval mode, no_grad and
     ``.grad`` as in ``predictive``."""
     _check(model, samples, _Comparative, "predictive_pair", _PAIR_CLASSES)
-    if eps is not None and (not isinstance(eps, (tuple, list)) or len(eps) != 2):
-        raise ValueError("eps must be a pair (eps_c, eps_w)")
-    n = 2 if model.use_wt_for_downstream else 1
-    if eps is not None and any(e is None for e in eps[:n]):
-        raise ValueError("eps needs eps_c, and eps_w when use_wt_for_downstream is set")
-    if eps is not None and n == 2 and eps[0].shape[:1] != eps[1].shape[:1]:
-        raise ValueError("eps_c and eps_w must hold the same number of draws")
+    n = _pair_items(model, eps)
     with torch.no_grad():
         params = _head_params(model)
         items = []

@@ -207,6 +207,17 @@ int is_head_mc_infer(const float* pooled0, const float* mu0, const float* logvar
                      int n_items, int latent, int prop_dim, const float* Wc, const float* bc, const float* coef, int n_head,
                      const float* W1, const float* b1, const float* W2, const float* b2, float* logits, float* prob_mean,
                      float* prob_std, int n_samples, int n_draws, void* stream);
+/* is_mutscan_expand (csrc/mutscan.cu): one pass of single-residue mutants for an in-silico saturation scan.  Copy k < r of
+ * the base batch (x23 [N,23], node_off [B+1], seq [B,L,V]) carries sites[k] = (p, c) (int32 pairs): x23_out [r N, 23] and
+ * seq_out [r B, L, V] are r copies of the base where, for every graph b with node_index[b,p] >= 0 (int64 [B,P], graph-local;
+ * < 0 = absent site, copy unmodified), node row node_off[b] + node_index[b,p] of copy k has residue columns one_hot_20(c)
+ * and sequence row seq_index[b,p] (int64 [B,P]) of sample b has one_hot_V(seq_columns[c]) (int64 [20]).  Bit-exact (copies
+ * and 0.0 / 1.0 only).  flag (int32 [1], zeroed by the caller, never cleared) is set to 1 if a base site row is not exactly
+ * one-hot, its sequence column is not seq_columns[its residue column], or an index is out of range (then that graph of
+ * that copy is not patched).  No atomics, no synchronisation. */
+int is_mutscan_expand(const float* x23, const int64_t* node_off, const int64_t* node_index, const float* seq,
+                      const int64_t* seq_index, const int64_t* seq_columns, const int* sites, int r, int n_graphs, int n_sites,
+                      int64_t n_nodes, int seq_len, int vocab, float* x23_out, float* seq_out, int* flag, void* stream);
 /* Dense Linear layer on the tensor cores: C[M,N] = act(A[M,K] W[N,K]^T + bias), fp32 in / out, operands split
  * on the fly into three bf16 terms (precision 3, fp32-accurate) or rounded to bf16 (precision 0).  Replaces the
  * nn.Linear layers of the sequence VAE (reference models/hybrid_models.py:63-74: vae_fc1 with ReLU, vae_fc4) in the
