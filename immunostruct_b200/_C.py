@@ -49,7 +49,7 @@ def exported_symbols():
             "is_segment_pool_fwd", "is_segment_pool_bwd", "is_contrastive_scratch_floats", "is_contrastive_fwd",
             "is_contrastive_bwd", "is_fused_adam", "is_rotate_coords", "is_mask_single_residue", "is_mask_rows", "is_gemm_tma_split_k",
             "is_split_planes", "is_gemm_planes_tma", "is_egnn_set_ws_buffers", "is_egnn_set_ws_variant", "is_reduce_partials3", "is_fused_adam_capturable",
-            "is_egnn_edge_attr_grad", "is_head_mc_infer", "is_mutscan_expand"]
+            "is_egnn_edge_attr_grad", "is_head_mc_infer", "is_mutscan_expand", "is_variant_expand"]
 
 
 def _check(rc: int, name: str):
@@ -526,6 +526,38 @@ def mutscan_expand(x23, node_off, node_index, seq, seq_index, seq_columns, sites
           _t(seq, f32, "seq"), _t(seq_index, i64, "seq_index"), _t(seq_columns, i64, "seq_columns"), _t(sites, i32, "sites"),
           _i32(r), _i32(b), _i32(p), _i64(n), _i32(L), _i32(V), _t(x23_out, f32, "x23_out"), _t(seq_out, f32, "seq_out"),
           _t(flag, i32, "flag"), _stream())
+
+
+def variant_expand(x23, node_off, edge_off, src_local, dst_local, edge_attr, seq, sample, offsets, node_index, seq_index,
+                   residue, seq_columns, node_out, edge_out, x23_out, src_out, dst_out, edge_attr_out, seq_out, flag):
+    """One pass of a variant library (csrc/mutscan.cu): variant v is a copy of base graph sample[v] (x23 rows from
+    node_out[v], graph-local edges from edge_out[v], sequence seq_out[v]) with the substitutions offsets[v] ..
+    offsets[v+1]-1 of (node_index, seq_index, residue) applied: residue columns one_hot_20(residue) at graph-local node row
+    node_index (-1 = not in the graph), one_hot_V(seq_columns[residue]) at sequence row seq_index.  ``flag`` (int32 [1],
+    zeroed by the caller) is raised if a replaced row is not exactly one-hot, contradicts ``seq_columns`` or an index is
+    out of range."""
+    f32, i64, i32 = torch.float32, torch.int64, torch.int32
+    if x23.dim() != 2 or seq.dim() != 3 or sample.dim() != 1 or offsets.dim() != 1 or node_index.dim() != 1:
+        raise ValueError("variant_expand: x23 [N,23], seq [B,L,V], sample [r], offsets [r+1] and node_index [S] expected")
+    b, L, V = seq.shape
+    r, s, e = sample.shape[0], node_index.shape[0], src_local.shape[0]
+    if (x23.shape[1] != 23 or node_off.shape != (b + 1,) or edge_off.shape != (b + 1,) or dst_local.shape != (e,)
+            or edge_attr.numel() != e or seq_index.shape != (s,) or residue.shape != (s,) or seq_columns.shape != (20,)
+            or offsets.shape != (r + 1,) or r < 1):
+        raise ValueError("variant_expand: unexpected input shapes")
+    n_out, e_out = x23_out.shape[0], src_out.shape[0]
+    if (x23_out.dim() != 2 or x23_out.shape[1] != 23 or node_out.shape != (r + 1,) or edge_out.shape != (r + 1,)
+            or dst_out.shape != (e_out,) or edge_attr_out.numel() != e_out or seq_out.shape != (r, L, V) or flag.shape != (1,)):
+        raise ValueError("variant_expand: unexpected output shapes")
+    if 3 * r > 0x7ffffffe:
+        raise ValueError("variant_expand: too many variants in one pass")
+    _call("is_variant_expand", _t(x23, f32, "x23"), _t(node_off, i64, "node_off"), _t(edge_off, i64, "edge_off"),
+          _t(src_local, i64, "src_local"), _t(dst_local, i64, "dst_local"), _t(edge_attr, f32, "edge_attr"), _t(seq, f32, "seq"),
+          _t(sample, i64, "sample"), _t(offsets, i64, "offsets"), _t(node_index, i64, "node_index"),
+          _t(seq_index, i64, "seq_index"), _t(residue, i64, "residue"), _t(seq_columns, i64, "seq_columns"),
+          _t(node_out, i64, "node_out"), _t(edge_out, i64, "edge_out"), _i32(r), _i32(b), _i64(s), _i32(L), _i32(V),
+          _i64(n_out), _i64(e_out), _t(x23_out, f32, "x23_out"), _t(src_out, i64, "src_out"), _t(dst_out, i64, "dst_out"),
+          _t(edge_attr_out, f32, "edge_attr_out"), _t(seq_out, f32, "seq_out"), _t(flag, i32, "flag"), _stream())
 
 
 def unpack_nodes(aa, xyz, x):

@@ -16,6 +16,12 @@ random numbers), so the difference between two variants is the effect of the sub
 An entry agrees with the fused eval forward of the B-sample mutant batch on the same draw to rounding, not bit for bit:
 where a graph sits in the batch changes two summation orders, the edge kernel's per-tile segment-sum MMA (a node's
 in-edges land at other positions of a 128-edge tile) and the K-slice count of the vae_fc1 GEMM (it follows the row count).
+
+``score_variants`` scores a caller's library instead: each variant is one sample of the batch with any list of
+substitutions (neoantigen candidates, anchor-modified designs, threaded peptides or HLA alleles).  A pass is a run of up to
+``max_graphs`` variants in the caller's order; ``is_variant_expand`` gathers their graphs, edges and sequences from the
+resident batch and applies the substitutions, the gathered topology is collated once per pass, and the trunk and the
+multi-draw head run as for the scan, each variant on the draws of its base sample.
 """
 from __future__ import annotations
 
@@ -26,6 +32,7 @@ import torch
 
 from . import functional as IF
 from .comparative_models import _Comparative
+from .graph import GraphBatch
 from .hybrid_models import _Hybrid
 from .predictive import _CLASSES, _PAIR_CLASSES, Predictive, _check, _draws, _encode, _head_params, _pair_items
 
@@ -58,6 +65,20 @@ def scan_sites(n_sites: int, device=None) -> Tensor:
     return torch.stack([p, c], 1).to(device)
 
 
+def _seq_columns(seq_columns, dev):
+    """seq_columns as int64 [20] on ``dev``, after the host checks of its type and shape."""
+    cols = torch.as_tensor(seq_columns)
+    if cols.dtype.is_floating_point or cols.dtype == torch.bool or cols.shape != (N_RESIDUES,):
+        raise ValueError("seq_columns must hold 20 integers: the sequence column of each residue-feature column")
+    return cols.to(dev, torch.int64).contiguous()
+
+
+def _columns_bad(cols, V):
+    """Device bool: seq_columns does not map the 20 residue columns to distinct sequence columns in [0, V)."""
+    s = cols.sort().values
+    return ((s < 0) | (s >= V)).any() | (s[1:] == s[:-1]).any()
+
+
 def _site_tables(graph, seq, node_index, seq_index, seq_columns):
     """Checked (node_index, seq_index, seq_columns) on the batch's device, int64.  One host read for all checks."""
     b = graph.n_graphs
@@ -68,16 +89,13 @@ def _site_tables(graph, seq, node_index, seq_index, seq_columns):
         raise ValueError("node_index and seq_index must have the same shape [B, P]")
     if not isinstance(seq, Tensor) or seq.dim() != 3 or seq.shape[0] != b:
         raise ValueError(f"sequence_data must be [B={b}, L, V]")
-    cols = torch.as_tensor(seq_columns)
-    if cols.dtype.is_floating_point or cols.dtype == torch.bool or cols.shape != (N_RESIDUES,):
-        raise ValueError("seq_columns must hold 20 integers: the sequence column of each residue-feature column")
     dev = graph.ndata["x"].device
-    ni, si, cols = node_index.to(dev), seq_index.to(dev), cols.to(dev, torch.int64)
+    cols = _seq_columns(seq_columns, dev)
+    ni, si = node_index.to(dev), seq_index.to(dev)
     L, V = seq.shape[1], seq.shape[2]
     counts = graph.batch_num_nodes().to(dev)
     bad = torch.stack([((ni == -1) != (si == -1)).any(), ((ni < -1) | (si < -1)).any(),
-                       (ni >= counts.unsqueeze(1)).any(), (si >= L).any(),
-                       ((cols < 0) | (cols >= V)).any() | (cols.unique().numel() != N_RESIDUES)]).tolist()
+                       (ni >= counts.unsqueeze(1)).any(), (si >= L).any(), _columns_bad(cols, V)]).tolist()
     if bad[0]:
         raise ValueError("a site is absent (-1) in node_index but not in seq_index, or the other way round")
     if bad[1]:
@@ -193,3 +211,177 @@ def mutational_scan_pair(model, graph_pair, sequence_pair, property_pair, node_i
 
         out = _run(model, gc, sequence_pair[0], property_pair[0], ni, si, cols, items[0][4], items_of, max_graphs)
     return Scan(*out, base)
+
+
+# ---- variant libraries: any substitution list on any sample -----------------------------------------------------------
+@dataclass
+class VariantScores:
+    """Scores of a library of multi-site residue variants, in the caller's order."""
+    logits: Tensor        # [V, K]  logit of variant v on draw k of its base sample
+    prob_mean: Tensor     # [V]     mean of sigmoid(logit) over the draws
+    prob_std: Tensor      # [V]     population standard deviation of sigmoid(logit) over the draws
+    base: Predictive      # the unmutated batch on the same draws
+
+
+def variant_passes(n_variants: int, max_graphs: int):
+    """(first variant, number of variants) of each pass: consecutive runs of at most ``max_graphs`` variants."""
+    if max_graphs < 1:
+        raise ValueError(f"max_graphs must be >= 1, got {max_graphs}")
+    return [(j, min(max_graphs, n_variants - j)) for j in range(0, n_variants, max_graphs)]
+
+
+def _variant_tables(graph, seq, sample, offsets, node_index, seq_index, residue, seq_columns, max_graphs):
+    """The checked library on the batch's device: (sample, offsets, node_index, seq_index, residue, seq_columns, node and
+    edge count of each variant, their running sums [V+1], every pass's node and edge totals).  One host read for all
+    checks and totals."""
+    b = graph.n_graphs
+    for name, t in (("sample", sample), ("offsets", offsets), ("node_index", node_index), ("seq_index", seq_index),
+                    ("residue", residue)):
+        if not isinstance(t, Tensor) or t.dtype != torch.int64 or t.dim() != 1:
+            raise ValueError(f"{name} must be a one-dimensional int64 tensor")
+    n_var, n_sub = sample.shape[0], node_index.shape[0]
+    if n_var < 1:
+        raise ValueError("the library needs at least one variant")
+    if offsets.shape[0] != n_var + 1:
+        raise ValueError(f"offsets must hold V + 1 = {n_var + 1} entries (the substitution CSR of the V variants)")
+    if seq_index.shape[0] != n_sub or residue.shape[0] != n_sub:
+        raise ValueError("node_index, seq_index and residue must hold one entry per substitution")
+    if not isinstance(seq, Tensor) or seq.dim() != 3 or seq.shape[0] != b:
+        raise ValueError(f"sequence_data must be [B={b}, L, V]")
+    passes = variant_passes(n_var, max_graphs)
+    dev = graph.ndata["x"].device
+    cols = _seq_columns(seq_columns, dev)
+    smp, off, ni, si, res = (t.to(dev).contiguous() for t in (sample, offsets, node_index, seq_index, residue))
+    L, V = seq.shape[1], seq.shape[2]
+    sb = smp.clamp(0, b - 1)
+    nv, ev = graph.batch_num_nodes().to(dev)[sb].contiguous(), graph.batch_num_edges().to(dev)[sb].contiguous()
+    zero = torch.zeros(1, dtype=torch.int64, device=dev)
+    ncs, ecs = torch.cat([zero, nv.cumsum(0)]), torch.cat([zero, ev.cumsum(0)])
+    owner = (torch.searchsorted(off, torch.arange(n_sub, device=dev), right=True) - 1).clamp(0, n_var - 1)
+    last = torch.arange(n_sub, device=dev)
+    twice = lambda key: (key.sort().values.diff() == 0).any()
+    node_key = torch.where(ni >= 0, owner * (int(graph.max_nodes) + 1) + ni, -1 - last)
+    seq_key = owner * L + si
+    first = torch.tensor([j for j, _ in passes], device=dev)
+    end = torch.tensor([j + r for j, r in passes], device=dev)
+    bad = torch.stack([((smp < 0) | (smp >= b)).any(), (off[0] != 0) | (off.diff() < 0).any() | (off[-1] != n_sub),
+                       ((ni < -1) | (ni >= nv[owner])).any(), ((si < 0) | (si >= L)).any(),
+                       ((res < 0) | (res >= N_RESIDUES)).any(), _columns_bad(cols, V), twice(node_key),
+                       twice(seq_key)]).long()
+    vals = torch.cat([bad, ncs[end] - ncs[first], ecs[end] - ecs[first]]).tolist()
+    if vals[0]:
+        raise ValueError(f"sample must index the batch: every entry in [0, B={b})")
+    if vals[1]:
+        raise ValueError(f"offsets must start at 0, never decrease and end at S={n_sub}")
+    if vals[2]:
+        raise ValueError("node_index must lie in [-1, n_b) of its variant's base graph (graph-local, -1 = not in the graph)")
+    if vals[3]:
+        raise ValueError(f"seq_index points outside the sequence length L={L}")
+    if vals[4]:
+        raise ValueError("residue must be a residue-feature column in [0, 20)")
+    if vals[5]:
+        raise ValueError(f"seq_columns must map the 20 residue columns to distinct sequence columns in [0, V={V})")
+    if vals[6]:
+        raise ValueError("a variant substitutes the same node row twice")
+    if vals[7]:
+        raise ValueError("a variant substitutes the same sequence row twice")
+    n_pass = len(passes)
+    return (smp, off, ni, si, res, cols, nv, ev, ncs, ecs, vals[8:8 + n_pass], vals[8 + n_pass:])
+
+
+def _run_variants(model, graph, seq, prop, tables, e, items_of, max_graphs):
+    """Every variant of the library in passes -> (logits [V,K], prob_mean [V], prob_std [V]).  ``items_of(item, s)`` turns
+    the mutant item of a pass whose variants have base samples ``s`` into the head's item list."""
+    smp, off, ni, si, res, cols, nv, ev, ncs, ecs, node_totals, edge_totals = tables
+    params = _head_params(model)
+    x = graph.ndata["x"].detach().contiguous()
+    ea = graph.edata["edge_attr"].detach().contiguous()
+    src, dst = graph._src_local.contiguous(), graph._dst_local.contiguous()
+    seq = seq.detach().contiguous()
+    prop = prop.detach().contiguous()
+    L, V, k = seq.shape[1], seq.shape[2], e.shape[0]
+    n_var = smp.shape[0]
+    f32 = dict(dtype=torch.float32, device=x.device)
+    logits, mean, std = torch.empty(n_var, k, **f32), torch.empty(n_var, **f32), torch.empty(n_var, **f32)
+    flag = torch.zeros(1, dtype=torch.int32, device=x.device)
+    for (j, r), n_p, e_p in zip(variant_passes(n_var, max_graphs), node_totals, edge_totals):
+        sp = smp[j:j + r]
+        x_p = torch.empty(n_p, 23, **f32)
+        src_p, dst_p = torch.empty(e_p, dtype=torch.int64, device=x.device), torch.empty(e_p, dtype=torch.int64, device=x.device)
+        ea_p = torch.empty(e_p, *ea.shape[1:], **f32)
+        seq_p = torch.empty(r, L, V, **f32)
+        IF._C.variant_expand(x, graph.node_off, graph.edge_off, src, dst, ea, seq, sp, off[j:j + r + 1], ni, si, res, cols,
+                             ncs[j:j + r + 1] - ncs[j], ecs[j:j + r + 1] - ecs[j], x_p, src_p, dst_p, ea_p, seq_p, flag)
+        # the pass's topology is gathered, not a replica of the batch: collated per pass
+        g = GraphBatch(x_p, src_p, dst_p, ea_p, nv[j:j + r], ev[j:j + r], max_nodes=graph.max_nodes, collate_now=False)
+        g._collate()
+        item = _encode(model, g, seq_p, prop[sp]) + (e[:, sp],)
+        lg, m, s = IF._C.head_mc_infer(items_of(item, sp), *params)
+        logits[j:j + r], mean[j:j + r], std[j:j + r] = lg, m, s
+    if flag.item():
+        raise ValueError("a substituted row is not exactly one-hot in the graph's residue columns or in the sequence, or "
+                         "its sequence column is not seq_columns[residue column] (a padded or masked row, or a wrong map)")
+    return logits, mean, std
+
+
+def score_variants(model, graph_data, sequence_data, peptide_property, sample: Tensor, offsets: Tensor,
+                   node_index: Tensor, seq_index: Tensor, residue: Tensor, *, seq_columns, eps: Optional[Tensor] = None,
+                   samples: int = 1, max_graphs: int = 4096) -> VariantScores:
+    """Scores of ``model(graph_data, sequence_data, peptide_property)[3]`` (the logit) for a library of V multi-site residue
+    variants of the batch's samples.
+
+    Variant v is sample ``sample[v]`` (int64 [V], any order, any number of times) with the substitutions
+    ``offsets[v]`` .. ``offsets[v+1] - 1`` (int64 [V+1], from 0 to S) of the int64 [S] tables: residue-feature column
+    ``residue[s]`` replaces the residue at graph-local node row ``node_index[s]`` (-1 when the graph does not hold that
+    residue, e.g. an HLA position present only in the sequence) and at sequence row ``seq_index[s]`` (always required),
+    written as column ``seq_columns[residue[s]]``.  A variant with no substitution is its base sample.  Coordinates and
+    contacts stay those of the base structure: nothing is re-folded.  No row may be substituted twice within a variant.
+
+    ``eps`` [K, B, latent] gives the draws, or one ``model.sample_eps`` call of [K*B, latent] (K = ``samples``) makes
+    them; variant v uses the draws of sample ``sample[v]``, so variants of one sample differ by their substitutions only.
+    The variants run in passes of at most ``max_graphs``, in the caller's order.  Classes, eval mode, no_grad and
+    ``.grad`` as in ``mutational_scan``."""
+    _check_scan(model, samples, (_Hybrid, _Comparative), "score_variants", _CLASSES)
+    tables = _variant_tables(graph_data, sequence_data, sample, offsets, node_index, seq_index, residue, seq_columns,
+                             max_graphs)
+    pair = isinstance(model, _Comparative) and model.use_wt_for_downstream
+    with torch.no_grad():
+        base_item = _encode(model, graph_data, sequence_data, peptide_property)
+        e = _draws(model, eps, samples, graph_data.n_graphs, base_item[1])
+        base_item += (e,)
+        base = Predictive(*IF._C.head_mc_infer([base_item, base_item] if pair else [base_item], *_head_params(model)))
+        out = _run_variants(model, graph_data, sequence_data, peptide_property, tables, e,
+                            lambda item, sp: [item, item] if pair else [item], max_graphs)
+    return VariantScores(*out, base)
+
+
+def score_variants_pair(model, graph_pair, sequence_pair, property_pair, sample: Tensor, offsets: Tensor,
+                        node_index: Tensor, seq_index: Tensor, residue: Tensor, *, seq_columns, eps=None, samples: int = 1,
+                        max_graphs: int = 4096) -> VariantScores:
+    """``score_variants`` of the cancer item of ``model.forward_comparative(graph_pair, sequence_pair, property_pair)``
+    against its fixed wild type, for the four comparative classes.  The library indexes the cancer item.
+
+    The wild type is encoded once, at batch B; each pass gathers its four encoded tensors and its draws by ``sample``.
+    ``eps`` = (eps_c, eps_w), each [K, B, latent], or one ``model.sample_eps`` call of [K*B, latent] per item, cancer
+    first.  Without ``use_wt_for_downstream`` the wild type is neither run nor drawn for.  ``base`` equals
+    ``predictive_pair`` on the same draws."""
+    _check_scan(model, samples, _Comparative, "score_variants_pair", _PAIR_CLASSES)
+    n = _pair_items(model, eps)
+    gc = graph_pair[0]
+    tables = _variant_tables(gc, sequence_pair[0], sample, offsets, node_index, seq_index, residue, seq_columns, max_graphs)
+    with torch.no_grad():
+        items = []
+        for i in range(n):
+            item = _encode(model, graph_pair[i], sequence_pair[i], property_pair[i])
+            k = samples if eps is None else eps[0].shape[0]
+            items.append(item + (_draws(model, None if eps is None else eps[i], k, item[1].shape[0], item[1]),))
+        base = Predictive(*IF._C.head_mc_infer(items, *_head_params(model)))
+        wt = items[1] if n == 2 else None
+
+        def items_of(item, sp):
+            if wt is None:
+                return [item]
+            return [item, tuple(t[:, sp] if t.dim() == 3 else t[sp] for t in wt)]
+
+        out = _run_variants(model, gc, sequence_pair[0], property_pair[0], tables, items[0][4], items_of, max_graphs)
+    return VariantScores(*out, base)

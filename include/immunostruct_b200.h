@@ -218,6 +218,27 @@ int is_head_mc_infer(const float* pooled0, const float* mu0, const float* logvar
 int is_mutscan_expand(const float* x23, const int64_t* node_off, const int64_t* node_index, const float* seq,
                       const int64_t* seq_index, const int64_t* seq_columns, const int* sites, int r, int n_graphs, int n_sites,
                       int64_t n_nodes, int seq_len, int vocab, float* x23_out, float* seq_out, int* flag, void* stream);
+/* is_variant_expand (csrc/mutscan.cu): one pass of a library of multi-site residue variants of a resident batch (x23
+ * [N,23], node_off / edge_off [B+1], graph-local src_local / dst_local int64 [E], edge_attr [E,1], seq [B,L,V]).
+ * Variant v < r is a copy of base graph b = sample[v] (int64 [r]): its x23 rows go to x23_out from row node_out[v], its
+ * edges (endpoints still graph-local, attributes) to src_out / dst_out / edge_attr_out from edge_out[v] (node_out /
+ * edge_out int64 [r+1]: the caller's running sums of the base counts), its sequence to seq_out[v] ([r,L,V]).  Then each
+ * substitution s in offsets[v] .. offsets[v+1]-1 (int64 [r+1], indices into the n_subs-long int64 node_index /
+ * seq_index / residue) writes one_hot_20(residue[s]) into the residue columns of node row node_index[s] (graph-local;
+ * -1 = the graph does not hold that residue) and one_hot_V(seq_columns[residue[s]]) (int64 [20]) into sequence row
+ * seq_index[s] (always required).  Bit-exact (copies and 0.0 / 1.0 only).  flag (int32 [1], zeroed by the caller, never
+ * cleared) is set to 1, and the substitution is not applied, if a base row it replaces is not exactly one-hot (the x23
+ * residue columns when node_index >= 0, the sequence row always), if both rows are present and the sequence's hot column
+ * is not seq_columns[the row's residue column], or if an index is out of range; a sample outside [0, B) or output
+ * offsets that disagree with the base counts or pass n_nodes_out / n_edges_out also raise it, and that variant is not
+ * written.  Within one variant no row may be substituted twice (the last one in table order wins).  No atomics, no
+ * synchronisation. */
+int is_variant_expand(const float* x23, const int64_t* node_off, const int64_t* edge_off, const int64_t* src_local,
+                      const int64_t* dst_local, const float* edge_attr, const float* seq, const int64_t* sample,
+                      const int64_t* offsets, const int64_t* node_index, const int64_t* seq_index, const int64_t* residue,
+                      const int64_t* seq_columns, const int64_t* node_out, const int64_t* edge_out, int r, int n_graphs,
+                      int64_t n_subs, int seq_len, int vocab, int64_t n_nodes_out, int64_t n_edges_out, float* x23_out,
+                      int64_t* src_out, int64_t* dst_out, float* edge_attr_out, float* seq_out, int* flag, void* stream);
 /* Dense Linear layer on the tensor cores: C[M,N] = act(A[M,K] W[N,K]^T + bias), fp32 in / out, operands split
  * on the fly into three bf16 terms (precision 3, fp32-accurate) or rounded to bf16 (precision 0).  Replaces the
  * nn.Linear layers of the sequence VAE (reference models/hybrid_models.py:63-74: vae_fc1 with ReLU, vae_fc4) in the
