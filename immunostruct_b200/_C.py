@@ -49,7 +49,8 @@ def exported_symbols():
             "is_segment_pool_fwd", "is_segment_pool_bwd", "is_contrastive_scratch_floats", "is_contrastive_fwd",
             "is_contrastive_bwd", "is_fused_adam", "is_rotate_coords", "is_mask_single_residue", "is_mask_rows", "is_gemm_tma_split_k",
             "is_split_planes", "is_gemm_planes_tma", "is_egnn_set_ws_buffers", "is_egnn_set_ws_variant", "is_reduce_partials3", "is_fused_adam_capturable",
-            "is_egnn_edge_attr_grad", "is_head_mc_infer", "is_mutscan_expand", "is_variant_expand"]
+            "is_egnn_edge_attr_grad", "is_head_mc_infer", "is_mutscan_expand", "is_variant_expand", "is_design_expand",
+            "is_design_select"]
 
 
 def _check(rc: int, name: str):
@@ -558,6 +559,76 @@ def variant_expand(x23, node_off, edge_off, src_local, dst_local, edge_attr, seq
           _t(node_out, i64, "node_out"), _t(edge_out, i64, "edge_out"), _i32(r), _i32(b), _i64(s), _i32(L), _i32(V),
           _i64(n_out), _i64(e_out), _t(x23_out, f32, "x23_out"), _t(src_out, i64, "src_out"), _t(dst_out, i64, "dst_out"),
           _t(edge_attr_out, f32, "edge_attr_out"), _t(seq_out, f32, "seq_out"), _t(flag, i32, "flag"), _stream())
+
+
+def design_expand(x23, node_off, node_index, seq, seq_index, seq_columns, beam, native, allowed, n_states, max_mutations,
+                  slot0, x23_out, seq_out, flag):
+    """One pass of a beam-search round (csrc/mutscan.cu): x23_out [r*N, 23] and seq_out [r*B, L, V] become r copies of the
+    base batch, copy k holding slot slot0 + k = (w P + p) 20 + c: state w of ``beam`` = (states [B,W,P], keys [B,W],
+    n_mut [B,W], valid [B,W] bool, ...) written at every present site, with residue column c at site p when the slot is
+    valid (``native`` [B,P], ``allowed`` [B,P,20] bool, the first ``n_states`` beam entries, ``max_mutations``).  ``flag``
+    (int32 [1], zeroed by the caller) is raised if the base rows of a slot's site are not exactly one-hot or do not
+    follow ``seq_columns``."""
+    f32, i64, i32, u8 = torch.float32, torch.int64, torch.int32, torch.bool
+    states, keys, n_mut, valid = beam[:4]
+    if node_index.dim() != 2 or seq.dim() != 3 or x23.dim() != 2 or states.dim() != 3:
+        raise ValueError("design_expand: node_index [B,P], seq [B,L,V], x23 [N,23] and states [B,W,P] expected")
+    b, p = node_index.shape
+    n, (_, L, V), w = x23.shape[0], seq.shape, states.shape[1]
+    if (x23.shape[1] != 23 or node_off.shape != (b + 1,) or seq_index.shape != (b, p) or seq.shape[0] != b
+            or seq_columns.shape != (20,) or states.shape != (b, w, p) or keys.shape != (b, w) or n_mut.shape != (b, w)
+            or valid.shape != (b, w) or native.shape != (b, p) or allowed.shape != (b, p, 20)):
+        raise ValueError("design_expand: unexpected input shapes")
+    r = seq_out.shape[0] // b
+    if r < 1 or x23_out.shape != (r * n, 23) or seq_out.shape != (r * b, L, V) or flag.shape != (1,):
+        raise ValueError("design_expand: unexpected output shapes")
+    if not (1 <= p <= 14 and 1 <= n_states <= w <= 32 and 0 <= slot0 and slot0 + r <= n_states * p * 20):
+        raise ValueError("design_expand: P <= 14, n_states <= W <= 32 and slots inside the round expected")
+    if r * b > 0x3fffffff or L * V > 0x7fffffff:
+        raise ValueError("design_expand: r * B or L * V too large")
+    _call("is_design_expand", _t(x23, f32, "x23"), _t(node_off, i64, "node_off"), _t(node_index, i64, "node_index"),
+          _t(seq, f32, "seq"), _t(seq_index, i64, "seq_index"), _t(seq_columns, i64, "seq_columns"),
+          _t(states, i64, "states"), _t(n_mut, i64, "n_mut"), _t(valid, u8, "valid"),
+          _t(native, i64, "native"), _t(allowed, u8, "allowed"), _i32(slot0), _i32(r), _i32(b), _i32(p), _i32(w),
+          _i32(n_states), _i32(max_mutations), _i64(n), _i32(L), _i32(V), _t(x23_out, f32, "x23_out"),
+          _t(seq_out, f32, "seq_out"), _t(flag, i32, "flag"), _stream())
+
+
+def design_select(beam, round_logits, round_mean, round_std, native, allowed, node_index, n_states, max_mutations, kappa,
+                  maximize, beam_out, best):
+    """Selection of a beam-search round (csrc/mutscan.cu), one CTA per sample: the next beam ``beam_out`` = (states
+    [B,W,P], keys [B,W], n_mut [B,W], valid [B,W] bool, logits [B,W,K], prob_mean, prob_std, objective [B,W]) is the top W
+    of the first ``n_states`` entries of ``beam`` (same tuple; its objective is not read) and the round's valid slots
+    (round_logits [n_states*P*20, B, K], round_mean / round_std [n_states*P*20, B]) by objective fmaf(kappa, std, mean),
+    descending when ``maximize``, ties to the smaller key, NaN never taken.  ``best`` [B] (any stride) gets the best
+    objective."""
+    f32, i64, u8 = torch.float32, torch.int64, torch.bool
+    if len(beam) != 8 or len(beam_out) != 8:
+        raise ValueError("design_select: beams are (states, keys, n_mut, valid, logits, prob_mean, prob_std, objective)")
+    states = beam[0]
+    if states.dim() != 3 or node_index.dim() != 2:
+        raise ValueError("design_select: states [B,W,P] and node_index [B,P] expected")
+    b, w, p = states.shape
+    k = beam[4].shape[-1]
+    shapes = ((b, w, p), (b, w), (b, w), (b, w), (b, w, k), (b, w), (b, w), (b, w))
+    n_slots = n_states * p * 20
+    if (any(tuple(t.shape) != s for t, s in zip(beam, shapes)) or any(tuple(t.shape) != s for t, s in zip(beam_out, shapes))
+            or round_logits.shape != (n_slots, b, k) or round_mean.shape != (n_slots, b)
+            or round_std.shape != (n_slots, b) or native.shape != (b, p) or allowed.shape != (b, p, 20)
+            or node_index.shape != (b, p) or best.shape != (b,)):
+        raise ValueError("design_select: unexpected shapes")
+    if not (1 <= p <= 14 and 1 <= n_states <= w <= 32):
+        raise ValueError("design_select: P <= 14 and n_states <= W <= 32 expected")
+    if any(x.data_ptr() == y.data_ptr() for x, y in zip(beam, beam_out)):
+        raise ValueError("design_select: beam_out must not alias beam")
+    names = ("states", "keys", "n_mut", "valid", "logits", "prob_mean", "prob_std", "objective")
+    types = (i64, i64, i64, u8, f32, f32, f32, f32)
+    _call("is_design_select", *(_t(t, d, n) for t, d, n in zip(beam[:7], types, names)),
+          _t(round_logits, f32, "round_logits"), _t(round_mean, f32, "round_mean"), _t(round_std, f32, "round_std"),
+          _t(native, i64, "native"), _t(allowed, u8, "allowed"), _t(node_index, i64, "node_index"), _i32(b), _i32(p),
+          _i32(w), _i32(n_states), _i32(k), _i32(max_mutations), _f32(kappa), _i32(1 if maximize else 0),
+          *(_t(t, d, n + "_out") for t, d, n in zip(beam_out, types, names)), _t(best, f32, "best", contiguous=False),
+          _i64(best.stride(0)), _stream())
 
 
 def unpack_nodes(aa, xyz, x):

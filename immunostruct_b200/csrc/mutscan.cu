@@ -216,6 +216,245 @@ __global__ void __launch_bounds__(VX_THREADS, VX_CTAS_PER_SM) variant_expand_ker
     }
 }
 
+// ---- beam search over residue substitutions (immunostruct_b200/design.py) ----------------------------------------------
+//
+// Sample b's beam holds W states of its P sites (int64 [B, W, P] residue columns, -1 at absent sites), their keys
+// sum_p digit(state[p]) 20^p (digit 0 at absent sites; they break ties), their Hamming distances to the native state and
+// a valid flag.
+// A round enumerates the slots (w, p, c) = "state w with site p set to residue c" of its first Wt states,
+// k = (w P + p) 20 + c; every slot is one copy of the whole batch.  design_slot_valid is the slot rule both kernels share.
+constexpr int DX_THREADS = 256;
+constexpr int DX_WARPS = DX_THREADS / 32;
+constexpr int DX_CTAS_PER_SM = 4;
+constexpr int DS_THREADS = 256;
+constexpr int DS_WARPS = DS_THREADS / 32;
+
+__device__ __forceinline__ int64_t design_digit(int64_t s) { return s < 0 ? 0 : s; }
+
+__device__ __forceinline__ int64_t pow20(int p) {
+    int64_t v = 1;
+    for (int i = 0; i < p; ++i) v *= 20;
+    return v;
+}
+
+// warp-wide (Wt <= 32; every lane gets the same answer): slot (w, p, c) of one sample is valid -- its parent w is valid,
+// site p is present, c is allowed there and differs from the parent's residue, the new state is within max_mut of the
+// native state, and it is canonical: no valid state l < Wt equals it, and none with l < w is one substitution away from
+// it (slot (l, p', c') yields the same state and comes first).  Lane l compares state l with the new state site by site:
+// two beam states two substitutions apart reach a common state at two different sites, which a comparison at site p
+// alone would miss.  Pointers are the sample's rows.
+__device__ __forceinline__ bool design_slot_valid(const int64_t* __restrict__ st, const int64_t* __restrict__ n_mut,
+                                                  const unsigned char* __restrict__ valid,
+                                                  const int64_t* __restrict__ native, const unsigned char* __restrict__ allowed,
+                                                  const int64_t* __restrict__ ni, int w, int p, int c, int P, int Wt,
+                                                  int max_mut, int lane) {
+    const int64_t* sw = st + (int64_t)w * P;
+    const int64_t sp = __ldg(sw + p);
+    if (!__ldg(valid + w) || __ldg(ni + p) < 0 || !__ldg(allowed + p * 20 + c) || sp == c) return false;
+    const int64_t nat = __ldg(native + p);
+    if (__ldg(n_mut + w) - (sp != nat) + (c != nat) > max_mut) return false;
+    bool dup = false;
+    if (lane < Wt && __ldg(valid + lane)) {
+        const int64_t* sl = st + (int64_t)lane * P;
+        int h = 0;
+        for (int q = 0; q < P; ++q) h += __ldg(sl + q) != (q == p ? (int64_t)c : __ldg(sw + q));
+        dup = h == 0 || (h == 1 && lane < w);
+    }
+    return !__any_sync(0xffffffffu, dup);
+}
+
+// One pass: copy k < r is slot slot0 + k.  Units (copy, graph, part) as in mutscan_expand_kernel; rows go in 32-row
+// chunks, one per warp, as in variant_expand_kernel.  Every present site of graph b gets the parent state's residue, and
+// site p the slot's residue c when the slot is valid (an invalid slot is written as its parent state).  Writing a residue
+// a row already holds is a bit-exact no-op, so only the mutated rows change.
+__global__ void __launch_bounds__(DX_THREADS, DX_CTAS_PER_SM) design_expand_kernel(
+        const float* __restrict__ x23, const int64_t* __restrict__ node_off, const int64_t* __restrict__ node_index,
+        const float* __restrict__ seq, const int64_t* __restrict__ seq_index, const int64_t* __restrict__ seq_columns,
+        const int64_t* __restrict__ states, const int64_t* __restrict__ n_mut, const unsigned char* __restrict__ valid,
+        const int64_t* __restrict__ native, const unsigned char* __restrict__ allowed, int slot0, int r, int B, int P, int W, int Wt, int max_mut,
+        int64_t N, int L, int V, float* __restrict__ x23_out, float* __restrict__ seq_out, int* __restrict__ flag) {
+    const int64_t units = 2 * (int64_t)r * B, LV = (int64_t)L * V;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    for (int64_t u = blockIdx.x; u < units; u += gridDim.x) {
+        const int part = (int)(u & 1);
+        const int kb = (int)(u >> 1), k = kb / B, b = kb - k * B;
+        const int s = slot0 + k, w = s / (P * 20), p = (s - w * P * 20) / 20, c = s - (w * P + p) * 20;
+        const int64_t n0 = __ldg(node_off + b), nb = __ldg(node_off + b + 1) - n0;
+        const int64_t* st = states + (int64_t)b * W * P;
+        const int64_t* ni = node_index + (int64_t)b * P;
+        const int64_t* si = seq_index + (int64_t)b * P;
+        const bool ok = design_slot_valid(st, n_mut + (int64_t)b * W, valid + (int64_t)b * W, native + (int64_t)b * P,
+                                          allowed + (int64_t)b * P * 20, ni, w, p, c, P, Wt, max_mut, lane);
+        const float* sbase = seq + b * LV;
+        if (part == 0 && warp == 0) {
+            const int64_t np = __ldg(ni + p), sq = __ldg(si + p);
+            if (np >= 0 && np < nb && sq >= 0 && sq < L &&
+                site_rows_bad(x23 + (n0 + np) * 23, sbase + sq * V, V, seq_columns, lane) && lane == 0)
+                *(volatile int*)flag = 1;
+        }
+        const int64_t n_rows = part == 0 ? nb : L;
+        const int Wd = part == 0 ? 23 : V;
+        const float* src = part == 0 ? x23 + n0 * 23 : sbase;
+        float* dst = part == 0 ? x23_out + ((int64_t)k * N + n0) * 23 : seq_out + ((int64_t)k * B + b) * LV;
+        for (int64_t c0 = (int64_t)warp * 32; c0 < n_rows; c0 += DX_WARPS * 32) {
+            int hot = -1;
+            for (int q = 0; q < P; ++q) {                                     // warp-uniform
+                const int64_t nq = __ldg(ni + q), sq = __ldg(si + q);
+                if (nq < 0) continue;                                         // absent site
+                const int64_t d = q == p && ok ? c : __ldg(st + (int64_t)w * P + q);
+                const int64_t sc = d >= 0 && d < 20 ? __ldg(seq_columns + d) : -1;
+                if (nq >= nb || sq < 0 || sq >= L || sc < 0 || sc >= V) {
+                    if (lane == 0) *(volatile int*)flag = 1;
+                    continue;
+                }
+                const int64_t row = part == 0 ? nq : sq;
+                if (lane == (int)(row - c0)) hot = part == 0 ? (int)d : (int)sc;
+            }
+            const int rows = (int)(n_rows - c0 < 32 ? n_rows - c0 : 32);
+            copy_chunk(src + c0 * Wd, dst + c0 * Wd, rows, Wd, part == 0 ? 20 : V, hot, lane);
+        }
+    }
+}
+
+// o1 / k1 ranks strictly before o2 / k2: the better objective, then the smaller key (keys in one pool are distinct)
+__device__ __forceinline__ bool design_before(float o1, int64_t k1, float o2, int64_t k2, bool maximize) {
+    return (maximize ? o1 > o2 : o1 < o2) || (o1 == o2 && k1 < k2);
+}
+
+// One CTA per sample.  The pool is the Wt carried states (with their scores) and the round's Wt P 20 slots; an entry is
+// eligible when it is valid (a valid beam state, or a valid slot) and its objective fmaf(kappa, std, mean) is not NaN.
+// The next beam is the first W eligible entries in design_before order, found by W block-wide arg-best passes over the
+// pool in shared memory (each pass takes the best entry ranked after the previous pick): deterministic, no atomics.
+__global__ void __launch_bounds__(DS_THREADS, 1) design_select_kernel(
+        const int64_t* __restrict__ states, const int64_t* __restrict__ keys, const int64_t* __restrict__ n_mut,
+        const unsigned char* __restrict__ valid, const float* __restrict__ logits, const float* __restrict__ mean,
+        const float* __restrict__ std_, const float* __restrict__ r_logits, const float* __restrict__ r_mean,
+        const float* __restrict__ r_std, const int64_t* __restrict__ native, const unsigned char* __restrict__ allowed,
+        const int64_t* __restrict__ node_index, int B, int P, int W, int Wt, int K, int max_mut, float kappa, int maximize,
+        int64_t* __restrict__ states_out, int64_t* __restrict__ keys_out, int64_t* __restrict__ n_mut_out,
+        unsigned char* __restrict__ valid_out, float* __restrict__ logits_out, float* __restrict__ mean_out,
+        float* __restrict__ std_out, float* __restrict__ obj_out, float* __restrict__ best, int64_t best_stride) {
+    extern __shared__ int64_t ds_smem[];
+    const int b = blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int n_slots = Wt * P * 20, n_pool = Wt + n_slots;
+    int64_t* pkey = ds_smem;
+    float* pobj = (float*)(ds_smem + n_pool);
+    __shared__ float red_o[DS_WARPS];
+    __shared__ int64_t red_k[DS_WARPS];
+    __shared__ int red_i[DS_WARPS];
+    __shared__ int sel[32];
+    const int64_t* st = states + (int64_t)b * W * P;
+    const int64_t* ky = keys + (int64_t)b * W;
+    const int64_t* nm = n_mut + (int64_t)b * W;
+    const unsigned char* vd = valid + (int64_t)b * W;
+    const int64_t* nat = native + (int64_t)b * P;
+    const float nan = __int_as_float(0x7fffffff);
+    for (int e = threadIdx.x; e < Wt; e += DS_THREADS) {
+        pkey[e] = __ldg(ky + e);
+        pobj[e] = __ldg(vd + e) ? fmaf(kappa, __ldg(std_ + (int64_t)b * W + e), __ldg(mean + (int64_t)b * W + e)) : nan;
+    }
+    for (int s = warp; s < n_slots; s += DS_WARPS) {                        // warp-uniform: the slot rule is warp-wide
+        const int w = s / (P * 20), p = (s - w * P * 20) / 20, c = s - (w * P + p) * 20;
+        const bool ok = design_slot_valid(st, nm, vd, nat, allowed + (int64_t)b * P * 20, node_index + (int64_t)b * P,
+                                          w, p, c, P, Wt, max_mut, lane);
+        if (lane == 0) {
+            pkey[Wt + s] = __ldg(ky + w) + (c - design_digit(__ldg(st + (int64_t)w * P + p))) * pow20(p);
+            pobj[Wt + s] = ok ? fmaf(kappa, __ldg(r_std + (int64_t)s * B + b), __ldg(r_mean + (int64_t)s * B + b)) : nan;
+        }
+    }
+    __syncthreads();
+    const bool mx = maximize != 0;
+    float prev_o = 0.0f;
+    int64_t prev_k = 0;
+    int n_sel = 0;
+    for (int j = 0; j < W; ++j) {
+        float bo = 0.0f;
+        int64_t bk = 0;
+        int bi = -1;
+        for (int e = threadIdx.x; e < n_pool; e += DS_THREADS) {
+            const float o = pobj[e];
+            if (o != o) continue;
+            const int64_t k = pkey[e];
+            if (j > 0 && !design_before(prev_o, prev_k, o, k, mx)) continue;
+            if (bi < 0 || design_before(o, k, bo, bk, mx)) { bo = o; bk = k; bi = e; }
+        }
+        for (int off = 16; off > 0; off >>= 1) {
+            const float oo = __shfl_down_sync(0xffffffffu, bo, off);
+            const int64_t ok_ = __shfl_down_sync(0xffffffffu, bk, off);
+            const int oi = __shfl_down_sync(0xffffffffu, bi, off);
+            if (oi >= 0 && (bi < 0 || design_before(oo, ok_, bo, bk, mx))) { bo = oo; bk = ok_; bi = oi; }
+        }
+        if (lane == 0) { red_o[warp] = bo; red_k[warp] = bk; red_i[warp] = bi; }
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            for (int i = 1; i < DS_WARPS; ++i)
+                if (red_i[i] >= 0 && (bi < 0 || design_before(red_o[i], red_k[i], bo, bk, mx))) {
+                    bo = red_o[i]; bk = red_k[i]; bi = red_i[i];
+                }
+            sel[j] = bi;
+            red_o[0] = bo; red_k[0] = bk; red_i[0] = bi;
+        }
+        __syncthreads();
+        bi = red_i[0];
+        prev_o = red_o[0];
+        prev_k = red_k[0];
+        __syncthreads();                                                      // red_* is rewritten by the next pass
+        if (bi < 0) break;
+        ++n_sel;
+    }
+    // the next beam: picks in order, then empty entries holding the native state (so a slot of theirs stays finite)
+    const int64_t bo_ = (int64_t)b * W;
+    for (int i = threadIdx.x; i < W * P; i += DS_THREADS) {
+        const int j = i / P, q = i - j * P;
+        int64_t v = __ldg(nat + q);
+        if (j < n_sel) {
+            const int e = sel[j];
+            const int w = e < Wt ? e : (e - Wt) / (P * 20);
+            v = __ldg(st + (int64_t)w * P + q);
+            if (e >= Wt && q == ((e - Wt) - w * P * 20) / 20) v = (e - Wt) % 20;
+        }
+        states_out[bo_ * P + i] = v;
+    }
+    for (int i = threadIdx.x; i < W * K; i += DS_THREADS) {
+        const int j = i / K, k = i - j * K;
+        float v = nan;
+        if (j < n_sel) {
+            const int e = sel[j];
+            v = e < Wt ? __ldg(logits + (bo_ + e) * K + k) : __ldg(r_logits + ((int64_t)(e - Wt) * B + b) * K + k);
+        }
+        logits_out[bo_ * K + i] = v;
+    }
+    for (int j = threadIdx.x; j < W; j += DS_THREADS) {
+        int64_t key = 0, nmut = 0;
+        float m = nan, sd = nan, o = nan;
+        if (j < n_sel) {
+            const int e = sel[j];
+            key = pkey[e];
+            o = pobj[e];
+            if (e < Wt) {
+                nmut = __ldg(nm + e);
+                m = __ldg(mean + bo_ + e);
+                sd = __ldg(std_ + bo_ + e);
+            } else {
+                const int s = e - Wt, w = s / (P * 20), p = (s - w * P * 20) / 20, c = s % 20;
+                const int64_t sp = __ldg(st + (int64_t)w * P + p), na = __ldg(nat + p);
+                nmut = __ldg(nm + w) - (sp != na) + (c != na);
+                m = __ldg(r_mean + (int64_t)s * B + b);
+                sd = __ldg(r_std + (int64_t)s * B + b);
+            }
+        } else {
+            for (int q = 0; q < P; ++q) key += design_digit(__ldg(nat + q)) * pow20(q);
+        }
+        keys_out[bo_ + j] = key;
+        n_mut_out[bo_ + j] = nmut;
+        valid_out[bo_ + j] = j < n_sel ? 1 : 0;
+        mean_out[bo_ + j] = m;
+        std_out[bo_ + j] = sd;
+        obj_out[bo_ + j] = o;
+    }
+    if (threadIdx.x == 0) best[(int64_t)b * best_stride] = n_sel > 0 ? pobj[sel[0]] : nan;
+}
+
 }  // namespace is
 
 using namespace is;
@@ -259,6 +498,52 @@ int is_variant_expand(const float* x23, const int64_t* node_off, const int64_t* 
         x23, node_off, edge_off, src_local, dst_local, edge_attr, seq, sample, offsets, node_index, seq_index, residue,
         seq_columns, node_out, edge_out, r, n_graphs, n_subs, seq_len, vocab, n_nodes_out, n_edges_out, x23_out, src_out,
         dst_out, edge_attr_out, seq_out, flag);
+    IS_LAUNCH_CHECK();
+    return IS_OK;
+}
+
+// grid: min(2 r B, 4 x SMs) CTAs of 256 threads, each looping over (copy, graph, part) units
+int is_design_expand(const float* x23, const int64_t* node_off, const int64_t* node_index, const float* seq,
+                     const int64_t* seq_index, const int64_t* seq_columns, const int64_t* states, const int64_t* n_mut,
+                     const unsigned char* valid, const int64_t* native, const unsigned char* allowed, int slot0, int r, int n_graphs, int n_sites, int beam, int n_states, int max_mutations, int64_t n_nodes,
+                     int seq_len, int vocab, float* x23_out, float* seq_out, int* flag, void* stream) {
+    if (r < 1 || n_graphs < 1 || n_sites < 1 || n_sites > 14 || beam < 1 || beam > 32 || n_states < 1 ||
+        n_states > beam || slot0 < 0 || slot0 + r > n_states * n_sites * 20 || n_nodes < 0 || seq_len < 1 || vocab < 1)
+        return IS_ERR_ARG;
+    if (!x23 || !node_off || !node_index || !seq || !seq_index || !seq_columns || !states || !n_mut || !valid || !native ||
+        !allowed || !x23_out || !seq_out || !flag)
+        return IS_ERR_ARG;
+    if ((int64_t)r * n_graphs > 0x3fffffff || (int64_t)seq_len * vocab > 0x7fffffff) return IS_ERR_UNSUPPORTED;
+    const int64_t units = 2 * (int64_t)r * n_graphs, cap = (int64_t)DX_CTAS_PER_SM * current_num_sms();
+    design_expand_kernel<<<(unsigned)(units < cap ? units : cap), DX_THREADS, 0, (cudaStream_t)stream>>>(
+        x23, node_off, node_index, seq, seq_index, seq_columns, states, n_mut, valid, native, allowed, slot0, r,
+        n_graphs, n_sites, beam, n_states, max_mutations, n_nodes, seq_len, vocab, x23_out, seq_out, flag);
+    IS_LAUNCH_CHECK();
+    return IS_OK;
+}
+
+// grid: one CTA of 256 threads per sample, (n_states (1 + 20 P)) x 12 bytes of dynamic shared memory (108 KB at the caps)
+int is_design_select(const int64_t* states, const int64_t* keys, const int64_t* n_mut, const unsigned char* valid,
+                     const float* logits, const float* prob_mean, const float* prob_std, const float* round_logits,
+                     const float* round_mean, const float* round_std, const int64_t* native, const unsigned char* allowed,
+                     const int64_t* node_index, int n_graphs, int n_sites, int beam, int n_states, int n_draws,
+                     int max_mutations, float kappa, int maximize, int64_t* states_out, int64_t* keys_out,
+                     int64_t* n_mut_out, unsigned char* valid_out, float* logits_out, float* mean_out, float* std_out,
+                     float* objective_out, float* best, int64_t best_stride, void* stream) {
+    if (n_graphs < 1 || n_sites < 1 || n_sites > 14 || beam < 1 || beam > 32 || n_states < 1 || n_states > beam ||
+        n_draws < 1 || best_stride < 1)
+        return IS_ERR_ARG;
+    if (!states || !keys || !n_mut || !valid || !logits || !prob_mean || !prob_std || !round_logits || !round_mean ||
+        !round_std || !native || !allowed || !node_index || !states_out || !keys_out || !n_mut_out || !valid_out ||
+        !logits_out || !mean_out || !std_out || !objective_out || !best)
+        return IS_ERR_ARG;
+    const size_t smem = (size_t)n_states * (1 + 20 * n_sites) * (sizeof(int64_t) + sizeof(float));
+    cudaError_t e = cudaFuncSetAttribute(design_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return (int)e;
+    design_select_kernel<<<(unsigned)n_graphs, DS_THREADS, smem, (cudaStream_t)stream>>>(
+        states, keys, n_mut, valid, logits, prob_mean, prob_std, round_logits, round_mean, round_std, native, allowed,
+        node_index, n_graphs, n_sites, beam, n_states, n_draws, max_mutations, kappa, maximize, states_out, keys_out,
+        n_mut_out, valid_out, logits_out, mean_out, std_out, objective_out, best, best_stride);
     IS_LAUNCH_CHECK();
     return IS_OK;
 }

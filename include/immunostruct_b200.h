@@ -239,6 +239,37 @@ int is_variant_expand(const float* x23, const int64_t* node_off, const int64_t* 
                       const int64_t* seq_columns, const int64_t* node_out, const int64_t* edge_out, int r, int n_graphs,
                       int64_t n_subs, int seq_len, int vocab, int64_t n_nodes_out, int64_t n_edges_out, float* x23_out,
                       int64_t* src_out, int64_t* dst_out, float* edge_attr_out, float* seq_out, int* flag, void* stream);
+/* is_design_expand / is_design_select (csrc/mutscan.cu): one round of a beam search over residue substitutions at the
+ * n_sites = P <= 14 sites of is_mutscan_expand (node_index / seq_index int64 [B,P], -1 in both = absent site).  The beam
+ * of sample b (beam = W <= 32 entries, of which the first n_states = Wt are read) is states int64 [B,W,P] (residue
+ * columns, -1 at absent sites), keys int64 [B,W] (sum_p digit_p 20^p, digit 0 at absent sites), n_mut int64 [B,W]
+ * (Hamming distance to native int64 [B,P]), valid uint8 [B,W]; allowed uint8 [B,P,20].  Slot k = (w P + p) 20 + c,
+ * k < Wt P 20, is state w with site p set to residue c; it is valid when valid[b,w], site p is present, allowed[b,p,c],
+ * c != states[b,w,p], the new state is within max_mutations of native, and no valid l < Wt equals the new state or,
+ * with l < w, differs from it at exactly one site (an earlier slot yields it).
+ * is_design_expand writes copies slot0 .. slot0 + r - 1 of the batch into x23_out [r N, 23] / seq_out [r B, L, V] (the
+ * layout of is_mutscan_expand): every present site of graph b gets the residue of state w, site p gets c if the slot is
+ * valid for b (an invalid slot is written as its parent state).  Bit-exact (copies and 0.0 / 1.0 only).  flag (int32 [1],
+ * zeroed by the caller, never cleared) is set to 1 if the base rows of site p are not exactly one-hot or contradict
+ * seq_columns, or an index or residue is out of range (that site is not written).
+ * is_design_select, one CTA per sample: the pool is the Wt carried entries (with logits [B,W,K], prob_mean / prob_std
+ * [B,W]) and the valid slots (round_logits [Wt P 20, B, K], round_mean / round_std [Wt P 20, B]); an entry's objective is
+ * fmaf(kappa, prob_std, prob_mean) in fp32, and entries whose objective is NaN (or that are invalid) are never taken.  The
+ * next beam (the *_out buffers, same shapes, must not alias the inputs) is the top W of the pool by objective
+ * (descending when maximize != 0, else ascending), ties to the smaller key; entries past the pool's size are invalid and
+ * hold the native state with NaN scores.  best[b * best_stride] = the objective of entry 0 (NaN if none).
+ * Deterministic, no atomics. */
+int is_design_expand(const float* x23, const int64_t* node_off, const int64_t* node_index, const float* seq,
+                     const int64_t* seq_index, const int64_t* seq_columns, const int64_t* states, const int64_t* n_mut,
+                     const unsigned char* valid, const int64_t* native, const unsigned char* allowed, int slot0, int r, int n_graphs, int n_sites, int beam, int n_states, int max_mutations, int64_t n_nodes,
+                     int seq_len, int vocab, float* x23_out, float* seq_out, int* flag, void* stream);
+int is_design_select(const int64_t* states, const int64_t* keys, const int64_t* n_mut, const unsigned char* valid,
+                     const float* logits, const float* prob_mean, const float* prob_std, const float* round_logits,
+                     const float* round_mean, const float* round_std, const int64_t* native, const unsigned char* allowed,
+                     const int64_t* node_index, int n_graphs, int n_sites, int beam, int n_states, int n_draws,
+                     int max_mutations, float kappa, int maximize, int64_t* states_out, int64_t* keys_out,
+                     int64_t* n_mut_out, unsigned char* valid_out, float* logits_out, float* mean_out, float* std_out,
+                     float* objective_out, float* best, int64_t best_stride, void* stream);
 /* Dense Linear layer on the tensor cores: C[M,N] = act(A[M,K] W[N,K]^T + bias), fp32 in / out, operands split
  * on the fly into three bf16 terms (precision 3, fp32-accurate) or rounded to bf16 (precision 0).  Replaces the
  * nn.Linear layers of the sequence VAE (reference models/hybrid_models.py:63-74: vae_fc1 with ReLU, vae_fc4) in the
