@@ -50,7 +50,7 @@ def exported_symbols():
             "is_contrastive_bwd", "is_fused_adam", "is_rotate_coords", "is_mask_single_residue", "is_mask_rows", "is_gemm_tma_split_k",
             "is_split_planes", "is_gemm_planes_tma", "is_egnn_set_ws_buffers", "is_egnn_set_ws_variant", "is_reduce_partials3", "is_fused_adam_capturable",
             "is_egnn_edge_attr_grad", "is_head_mc_infer", "is_mutscan_expand", "is_variant_expand", "is_design_expand",
-            "is_design_select"]
+            "is_design_select", "is_egnn_layer_fwd_fp16x2"]
 
 
 def _check(rc: int, name: str):
@@ -245,6 +245,22 @@ def egnn_edge_fwd_tc(g, PQ, x, edge_attr, F, W1, W2, b2, W3, b3, w4, update_coor
           _t(b3, f32, "b3"), _t(w4, f32, "w4"), _i32(1 if update_coords else 0), _i32(precision),
           _i32(1 if fast_act else 0), _t(hn, f32, "hn"), _t(x_out, f32, "x_out"), _i64(PQ.shape[0]), _t(g.status, torch.int32, "status"),
           _stream())
+
+
+def egnn_layer_fwd_fp16x2(g, PQ, x, edge_attr, W1, W2, b2, W3, b3, w4, update_coords, hn, x_out,
+                          h, W5, b5, W6, b6, h_out, W1n, b1n, PQn, next_kind=1):
+    """One whole EGNN layer of the fp16x2 inference forward in one launch (csrc/egnn_tc2.cu): egnn_edge_fwd_tc followed by
+    egnn_node_post_pre_tc, both in PREC_FP16X2, bit for bit.  ``h`` is the layer's input [N, F]; W1n / b1n / PQn and
+    next_kind as in egnn_node_post_pre_tc (next_kind 2, the QKV projections, only without ``update_coords``)."""
+    f32 = torch.float32
+    xp, ldx = _rows(x, "x")
+    hp, ldh = _rows(h, "h")
+    _call("is_egnn_layer_fwd_fp16x2", *_csr(g), _t(PQ, f32, "PQ"), xp, ldx, _t(edge_attr, f32, "edge_attr"),
+          _t(W1, f32, "W1"), _i32(h.shape[1]), _t(W2, f32, "W2"), _t(b2, f32, "b2"), _t(W3, f32, "W3"),
+          _t(b3, f32, "b3"), _t(w4, f32, "w4"), _i32(1 if update_coords else 0), _t(hn, f32, "hn"), _t(x_out, f32, "x_out"),
+          hp, ldh, _t(W5, f32, "W5"), _t(b5, f32, "b5"), _t(W6, f32, "W6"), _t(b6, f32, "b6"), _t(h_out, f32, "h_out"),
+          _t(W1n, f32, "W1n"), _t(b1n, f32, "b1n"), _t(PQn, f32, "PQn"), _i32(next_kind), _i64(PQ.shape[0]),
+          _t(g.status, torch.int32, "status"), _stream())
 
 
 def egnn_node_post_fwd(h, hn, W5, b5, W6, b6, h_out):

@@ -1,271 +1,64 @@
-// Node-side half of an EGNN layer on the tensor cores, fused across the layer boundary:
+// Node-side half of an EGNN layer on the tensor cores, fused across the layer boundary (the tile chain: egnn_node_tc.cuh):
 //
-//   node_post(l) :  h' = W6 silu(W5 [h | hn] + b5) + b6              (reference: EGNNConv node_mlp)
-//   node_pre(l+1):  P' = h' Ws'^T ,  Q' = h' Wd'^T + b1'              (first edge-MLP layer of layer l+1,
-//                                                                      split per node, see egnn.cu)
-//   or, after the LAST layer (next_kind = 2):  QKV = h' [Wq; Wk; Wv]^T + [bq; bk; bv]   (the three projections of
-//                                              the per-graph attention, models/layers.py:13-16 / :67-69)
-// Per tile of 128 nodes four chained tcgen05 GEMM groups run against weight blocks that stay resident
-// in shared memory for the CTA's lifetime; the activations never leave the SM between them:
-//   D1 = h W5h^T + hn W5n^T  -> +b5, SiLU -> D2 = t5 W6^T -> +b6 = h' (stored) -> D3 = h' [Ws'; Wd']^T (+b1')
-// A single A-operand buffer (one 64-wide K block) is re-staged between the groups.  Used by the
-// no-grad inference path (immunostruct_b200.functional.egnn_stack_infer); the training path keeps the
-// SIMT node kernels.  PREC_BF16 (bf16 mode) or PREC_BF16X3 (fp32 parity; the hi/lo tf32 form of the five
-// resident weight blocks would not fit in shared memory, the three-term bf16 form does: 138 KB).
-#include "tc_common.cuh"
+//   node_post(l) :  h' = W6 silu(W5 [h | hn] + b5) + b6
+//   node_pre(l+1):  P' = h' Ws'^T ,  Q' = h' Wd'^T + b1'   or, after the LAST layer (next_kind = 2), QKV = h' [Wq; Wk; Wv]^T + b
+//
+// One persistent CTA per SM (two at 256 threads) walks the groups of NTILE 128-node tiles; its weight blocks stay resident
+// in shared memory for the CTA's lifetime.  Used by the no-grad inference path in the precisions whose edge forward has no
+// node tail (bf16, bf16x3) and by the training forward; the fp16x2 inference forward runs the same chain as the tail of the
+// edge kernel (egnn_tc2.cu, egnn_layer_fwd).  PREC_BF16 (bf16 mode), PREC_FP16X2 or PREC_BF16X3 (fp32 parity; the hi/lo
+// tf32 form of the five resident weight blocks would not fit in shared memory, the three-term bf16 form does: 138 KB).
+#include "egnn_node_tc.cuh"
 
 namespace is {
 
 template <int PREC, int NT, bool FAST, int NEXT_KIND>
 __global__ void __launch_bounds__(NT, NT == 256 ? 2 : 1)
-node_post_pre_tc_kernel(const float* __restrict__ h, int64_t ldh, int F, const float* __restrict__ hn,
-                        const float* __restrict__ W5, const float* __restrict__ b5,
-                        const float* __restrict__ W6, const float* __restrict__ b6, float* __restrict__ h_out,
-                        const float* __restrict__ W1n /* next layer edge_mlp.0.weight [64,130] | [Wq;Wk;Wv] [192,64] | null */,
-                        const float* __restrict__ b1n, float* __restrict__ PQn, int64_t M) {
-    constexpr int next_kind = NEXT_KIND;
-    using C = TcCfg<PREC>;
-    constexpr int NW = NT / 32, CQ = NW / 4, CW = 64 / CQ;
-    constexpr int NBLK = NEXT_KIND == 2 ? 6 : 5;                          // resident weight blocks
-    constexpr uint32_t ASPL = C::A_BYTES, WSPL = NBLK * C::W_BYTES;       // split-term strides
+node_post_pre_tc_kernel(NodeArgs a, int64_t M) {
+    using NC = NodeCfg<PREC, NEXT_KIND>;
     extern __shared__ __align__(128) uint8_t smem_raw[];
-    // TWO_BUF (one- and two-term operand splits: the three-term tiles leave no room): a second A-operand buffer, so that h
-    // and hn are staged together (their row loads overlap) and D1 = h W5h^T + hn W5n^T is ONE MMA group with one hand-over
-    // instead of two; the epilogues then alternate between the buffers.
-    constexpr bool TWO_BUF = C::NSPLIT <= 2;
-    // NTILE (fp16x2: 2) tiles of 128 nodes share every hand-over: a tile's chain is a string of fixed latencies (barriers, MMA
-    // completion, the row loads' round trip) -- shortening its rows by 10 % did not change the kernel's time at all -- so two
-    // tiles per round halve the rounds (800 tiles on 148 CTAs: 6 -> 3) at little extra cost per round.  Needs both tiles'
-    // operand buffers (4 x 32 KB next to 96 KB of weights) and 2 x 256 TMEM columns.
-    constexpr int NTILE = (PREC == PREC_FP16X2 && NEXT_KIND == 1) ? 2 : 1;      // (the six blocks of the QKV tail leave no room)
-    constexpr uint32_t ABUF = C::NSPLIT * ASPL, ASTRIDE = (TWO_BUF ? 2 : 1) * ABUF, TCOLS = 256;
-    uint8_t* sA = smem_raw;                                   // [NTILE][1 or 2 buffers][NSPLIT][A_BYTES]
-    uint8_t* sA2 = TWO_BUF ? sA + ABUF : sA;
-    uint8_t* sW = sA + NTILE * ASTRIDE;                       // [NSPLIT][6 blocks][W_BYTES]: W5h W5n W6 | Ws' Wd' - or Wq Wk Wv
-    float* vec = reinterpret_cast<float*>(sW + C::NSPLIT * WSPL);   // b5, b6, next bias (64: b1' for Q' | 192: bq bk bv)
+    uint8_t* sA = smem_raw;
+    uint8_t* sW = sA + NC::A_REGION;
+    float* vec = reinterpret_cast<float*>(sW + NC::W_REGION);
     __shared__ __align__(8) uint64_t mbar;
     __shared__ uint32_t s_tmem;
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const bool has_next = W1n != nullptr;
-    const int K5 = F + 64;
+    const int tid = threadIdx.x, warp = tid >> 5;
 
-    if (warp == 0) tmem_alloc(&s_tmem, NTILE * TCOLS);
+    if (warp == 0) tmem_alloc(&s_tmem, NC::NTILE * NC::TCOLS);
     if (tid == 32) mbar_init(&mbar, 1);
-    // six resident weight blocks (16-byte chunk stores; W5's two K halves, W6, then the "next" weights)
-    stage_weight_block<PREC>(sW + 0 * C::W_BYTES, WSPL, W5, K5, 0, F, tid, NT);
-    stage_weight_block<PREC>(sW + 1 * C::W_BYTES, WSPL, W5, K5, F, 64, tid, NT);
-    stage_weight_block<PREC>(sW + 2 * C::W_BYTES, WSPL, W6, 64, 0, 64, tid, NT);
-    if (next_kind == 2) {
-        stage_weight_block<PREC>(sW + 3 * C::W_BYTES, WSPL, W1n, 64, 0, 64, tid, NT);
-        stage_weight_block<PREC>(sW + 4 * C::W_BYTES, WSPL, W1n + 4096, 64, 0, 64, tid, NT);
-        stage_weight_block<PREC>(sW + 5 * C::W_BYTES, WSPL, W1n + 8192, 64, 0, 64, tid, NT);
-    } else {
-        stage_weight_block<PREC>(sW + 3 * C::W_BYTES, WSPL, has_next ? W1n : nullptr, 130, 0, 64, tid, NT);
-        stage_weight_block<PREC>(sW + 4 * C::W_BYTES, WSPL, has_next ? W1n : nullptr, 130, 64, 64, tid, NT);
-    }
-    if (tid < 64) {
-        vec[tid] = b5[tid];
-        vec[64 + tid] = b6[tid];
-    }
-    if (tid < 192) vec[128 + tid] = !has_next ? 0.0f : next_kind == 2 ? b1n[tid] : (tid < 64 ? b1n[tid] : 0.0f);
+    node_stage_weights<PREC, NEXT_KIND>(a, sW, vec, tid, NT);
     fence_async_smem();
     fence_before_sync();
     __syncthreads();
     fence_after_sync();
     const uint32_t tmem = s_tmem;
-    const uint32_t a_addr = smem_u32(sA), a2_addr = smem_u32(sA2), w_addr = smem_u32(sW);
-    const int q = warp & 3, cq = warp >> 2, erow = 32 * q + lane;
-    const uint32_t t_lane = tmem + ((uint32_t)(32 * q) << 16);
-    const int rsub = lane >> 3, kc8 = lane & 7;
     uint32_t phase = 0;
-
-    // stage a [128 x 64] fp32 tile (rows m0.., `ncols` valid columns, row stride ld) as the A operand
-    auto stage_rows = [&](uint8_t* __restrict__ dstA, const float* __restrict__ src, int64_t ld, int ncols, int64_t m0) {
-#pragma unroll
-        for (int pass = 0; pass < IS_TM / (4 * NW); ++pass) {
-            const int r = pass * 4 * NW + warp * 4 + rsub;
-            const int64_t m = m0 + r;
-            float v[8];
-#pragma unroll
-            for (int i = 0; i < 8; ++i) v[i] = 0.0f;
-            if (m < M) {
-                const float* rp = src + m * ld + 8 * kc8;
-                if (ncols == 64 && (ld & 7) == 0 && (reinterpret_cast<uintptr_t>(src) & 31) == 0) {
-                    ldg256(rp, v);                                  // one sector-complete 32-byte access per lane
-                } else if (ncols == 64 && (ld & 3) == 0) {
-                    const float4 a = __ldg(reinterpret_cast<const float4*>(rp)), b = __ldg(reinterpret_cast<const float4*>(rp) + 1);
-                    v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = b.x; v[5] = b.y; v[6] = b.z; v[7] = b.w;
-                } else {
-#pragma unroll
-                    for (int i = 0; i < 8; ++i) v[i] = (8 * kc8 + i < ncols) ? __ldg(rp + i) : 0.0f;
-                }
-            }
-            store_operand8<PREC>(dstA, ASPL, r, kc8, v);
-        }
-    };
-    // publish the staged operands, let one elected lane issue `issue_fn` (MMAs of one hand-over) and wait for them
-    auto run_gemms = [&](auto&& issue_fn) {
-        fence_async_smem();
-        fence_before_sync();
-        __syncthreads();
-        if (tid < 32) {               // one elected lane of the converged warp issues (bare UTCHMMA, no election loop)
-            if (elect_one()) {
-                fence_after_sync();
-                issue_fn();
-                mma_commit(&mbar);
-            }
-            __syncwarp();
-            mbar_wait(&mbar, phase);
-        }
-        phase ^= 1;
-        __syncthreads();
-        fence_after_sync();
-    };
-    auto run_gemm = [&](uint32_t tmem_d, uint32_t a_tile, int wblock, uint32_t ncols, uint32_t accumulate) {
-        run_gemms([&] { issue_gemm<PREC, !FAST>(tmem_d, a_tile, ASPL, w_addr + wblock * C::W_BYTES, WSPL, ncols, accumulate); });
-    };
-
-    const int64_t ngroups = (M + NTILE * IS_TM - 1) / (NTILE * IS_TM);
-    for (int64_t t = blockIdx.x; t < ngroups; t += gridDim.x) {
-        const int64_t mg = t * NTILE * IS_TM;                 // first row of this group of NTILE tiles
-        // ---- D1 = h W5h^T + hn W5n^T ---------------------------------------------------------------
-        if (TWO_BUF) {
-#pragma unroll
-            for (int u = 0; u < NTILE; ++u) {
-                stage_rows(sA + u * ASTRIDE, h, ldh, F, mg + u * IS_TM);
-                stage_rows(sA2 + u * ASTRIDE, hn, 64, 64, mg + u * IS_TM);
-            }
-            run_gemms([&] {
-#pragma unroll
-                for (int u = 0; u < NTILE; ++u) {
-                    issue_gemm<PREC, !FAST>(tmem + u * TCOLS, a_addr + u * ASTRIDE, ASPL, w_addr + 0 * C::W_BYTES, WSPL, 64, 0);
-                    issue_gemm<PREC, !FAST>(tmem + u * TCOLS, a2_addr + u * ASTRIDE, ASPL, w_addr + 1 * C::W_BYTES, WSPL, 64, 1);
-                }
-            });
-        } else {
-            stage_rows(sA, h, ldh, F, mg);
-            run_gemm(tmem, a_addr, 0, 64, 0);
-            stage_rows(sA, hn, 64, 64, mg);
-            run_gemm(tmem, a_addr, 1, 64, 1);
-        }
-        // ---- t5 = silu(D1 + b5) -> A operand ; D2 = t5 W6^T -------------------------------------------
-#pragma unroll
-        for (int u = 0; u < NTILE; ++u) {
-            float z[CW];
-            tmem_ld<CW>(t_lane + u * TCOLS + CW * cq, z);
-#pragma unroll
-            for (int g = 0; g < CW / 8; ++g) {
-                float v[8];
-#pragma unroll
-                for (int i = 0; i < 8; ++i) v[i] = act<PREC, FAST>(z[8 * g + i] + vec[CW * cq + 8 * g + i]);
-                store_operand8<PREC>(sA + u * ASTRIDE, ASPL, erow, (CW / 8) * cq + g, v);
-            }
-        }
-        run_gemms([&] {
-#pragma unroll
-            for (int u = 0; u < NTILE; ++u)
-                issue_gemm<PREC, !FAST>(tmem + u * TCOLS + 64, a_addr + u * ASTRIDE, ASPL, w_addr + 2 * C::W_BYTES, WSPL, 64, 0);
-        });
-        // ---- h' = D2 + b6 -> global (+ A operand for the next layer's P/Q) ------------------------------
-#pragma unroll
-        for (int u = 0; u < NTILE; ++u) {
-            float z[CW];
-            tmem_ld<CW>(t_lane + u * TCOLS + 64 + CW * cq, z);
-            const int64_t m = mg + u * IS_TM + erow;
-#pragma unroll
-            for (int g = 0; g < CW / 8; ++g) {
-                float v[8];
-#pragma unroll
-                for (int i = 0; i < 8; ++i) v[i] = z[8 * g + i] + vec[64 + CW * cq + 8 * g + i];
-                if (m < M) stg256(h_out + m * 64 + CW * cq + 8 * g, v);
-                if (has_next) store_operand8<PREC>(sA2 + u * ASTRIDE, ASPL, erow, (CW / 8) * cq + g, v);
-            }
-        }
-        if (has_next && next_kind == 2) {
-            // ---- D3 = h' [Wq; Wk; Wv]^T (N = 192: blocks 3..5), written over the dead accumulators D1 / D2 ----
-            run_gemms([&] {
-#pragma unroll
-                for (int u = 0; u < NTILE; ++u)
-                    issue_gemm<PREC, !FAST>(tmem + u * TCOLS, a2_addr + u * ASTRIDE, ASPL, w_addr + 3 * C::W_BYTES, WSPL, 192, 0);
-            });
-#pragma unroll
-            for (int u = 0; u < NTILE; ++u) {
-                const int64_t m = mg + u * IS_TM + erow;
-#pragma unroll
-                for (int part = 0; part < 3; ++part) {
-                    float z[CW];
-                    tmem_ld<CW>(t_lane + u * TCOLS + 64 * part + CW * cq, z);
-                    if (m < M) {
-#pragma unroll
-                        for (int g = 0; g < CW / 8; ++g) {
-                            const int c = 64 * part + CW * cq + 8 * g;
-                            float o[8];
-#pragma unroll
-                            for (int i = 0; i < 8; ++i) o[i] = z[8 * g + i] + vec[128 + c + i];
-                            stg256(PQn + m * 192 + c, o);
-                        }
-                    }
-                }
-            }
-        } else if (has_next) {
-            // ---- D3 = h' [Ws'; Wd']^T (N = 128: weight blocks 3 and 4 are contiguous row groups) -------
-            run_gemms([&] {
-#pragma unroll
-                for (int u = 0; u < NTILE; ++u)
-                    issue_gemm<PREC, !FAST>(tmem + u * TCOLS + 128, a2_addr + u * ASTRIDE, ASPL, w_addr + 3 * C::W_BYTES, WSPL, 128, 0);
-            });
-#pragma unroll
-            for (int u = 0; u < NTILE; ++u) {
-                const int64_t m = mg + u * IS_TM + erow;
-#pragma unroll
-                for (int half = 0; half < 2; ++half) {
-                    float z[CW];
-                    tmem_ld<CW>(t_lane + u * TCOLS + 128 + 64 * half + CW * cq, z);
-                    if (m < M) {
-#pragma unroll
-                        for (int g = 0; g < CW / 8; ++g) {
-                            const int c = CW * cq + 8 * g;
-                            float o[8];
-#pragma unroll
-                            for (int i = 0; i < 8; ++i) o[i] = z[8 * g + i] + (half ? vec[128 + c + i] : 0.0f);
-                            stg256(PQn + m * 128 + 64 * half + c, o);
-                        }
-                    }
-                }
-            }
-        }
-        fence_before_sync();      // TMEM reads of this group are ordered before the next group's MMAs
-    }
+    constexpr int64_t GROUP = NC::NTILE * IS_TM;
+    node_chain<PREC, NT, FAST, NEXT_KIND>(a, sA, sW, vec, tmem, &mbar, phase, blockIdx.x * GROUP, gridDim.x * GROUP, M, tid, 0);
     fence_before_sync();
     __syncthreads();
-    if (warp == 0) tmem_dealloc(tmem, NTILE * TCOLS);
+    if (warp == 0) tmem_dealloc(tmem, NC::NTILE * NC::TCOLS);
 }
 
 template <int PREC, int NT, bool FAST, int NEXT_KIND>
-static int launch_node_tc2(const float* h, int64_t ldh, int F, const float* hn, const float* W5, const float* b5,
-                          const float* W6, const float* b6, float* h_out, const float* W1n, const float* b1n,
-                          float* PQn, int64_t M, cudaStream_t st) {
-    using C = TcCfg<PREC>;
-    constexpr int NTILE = (PREC == PREC_FP16X2 && NEXT_KIND == 1) ? 2 : 1;        // tiles per hand-over (see the kernel)
-    constexpr int NBLK = NEXT_KIND == 2 ? 6 : 5;
-    const size_t smem = (size_t)C::NSPLIT * (NTILE * (C::NSPLIT <= 2 ? 2 : 1) * C::A_BYTES + NBLK * C::W_BYTES) + 5 * 64 * sizeof(float) + 128;
+static int launch_node_tc2(const NodeArgs& a, int64_t M, cudaStream_t st) {
+    using NC = NodeCfg<PREC, NEXT_KIND>;
+    const size_t smem = (size_t)NC::A_REGION + NC::W_REGION + NC::VEC_BYTES + 128;
     cudaError_t e = cudaFuncSetAttribute(node_post_pre_tc_kernel<PREC, NT, FAST, NEXT_KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
     const int sms = current_num_sms();
-    int64_t tiles = (M + NTILE * IS_TM - 1) / (NTILE * IS_TM);
+    int64_t tiles = (M + NC::NTILE * IS_TM - 1) / (NC::NTILE * IS_TM);
     int64_t cap = (int64_t)sms * (NT == 256 ? 2 : 1);
     int grid = (int)(tiles < cap ? tiles : cap);
-    node_post_pre_tc_kernel<PREC, NT, FAST, NEXT_KIND><<<grid < 1 ? 1 : grid, NT, smem, st>>>(h, ldh, F, hn, W5, b5, W6, b6, h_out, W1n, b1n, PQn, M);
+    node_post_pre_tc_kernel<PREC, NT, FAST, NEXT_KIND><<<grid < 1 ? 1 : grid, NT, smem, st>>>(a, M);
     e = cudaGetLastError();
     return e == cudaSuccess ? 0 : (int)e;
 }
 
 template <int PREC, int NT, bool FAST>
-static int launch_node_tc(const float* h, int64_t ldh, int F, const float* hn, const float* W5, const float* b5,
-                          const float* W6, const float* b6, float* h_out, const float* W1n, const float* b1n,
-                          float* PQn, int64_t M, int next_kind, cudaStream_t st) {
-    if (next_kind == 2) return launch_node_tc2<PREC, NT, FAST, 2>(h, ldh, F, hn, W5, b5, W6, b6, h_out, W1n, b1n, PQn, M, st);
-    return launch_node_tc2<PREC, NT, FAST, 1>(h, ldh, F, hn, W5, b5, W6, b6, h_out, W1n, b1n, PQn, M, st);
+static int launch_node_tc(const NodeArgs& a, int64_t M, int next_kind, cudaStream_t st) {
+    if (next_kind == 2) return launch_node_tc2<PREC, NT, FAST, 2>(a, M, st);
+    return launch_node_tc2<PREC, NT, FAST, 1>(a, M, st);
 }
 
 }  // namespace is
@@ -287,14 +80,15 @@ int is_egnn_node_post_pre_tc(const float* h, int64_t ldh, int F, const float* hn
     if (W1n != nullptr && next_kind != 1 && next_kind != 2) return IS_ERR_ARG;
     if (((reinterpret_cast<uintptr_t>(h_out) | reinterpret_cast<uintptr_t>(PQn)) & 31) != 0) return IS_ERR_ARG;   // 256-bit stores
     cudaStream_t st = (cudaStream_t)stream;
+    const NodeArgs a{h, ldh, F, hn, W5, b5, W6, b6, h_out, W1n, b1n, PQn};
     if (precision == PREC_BF16)
-        return launch_node_tc<PREC_BF16, 256, true>(h, ldh, F, hn, W5, b5, W6, b6, h_out, W1n, b1n, PQn, n_nodes, next_kind, st);
+        return launch_node_tc<PREC_BF16, 256, true>(a, n_nodes, next_kind, st);
     if (precision == PREC_FP16X2)          // fp16 hi / lo operand split: inference forward only
-        return launch_node_tc<PREC_FP16X2, 512, true>(h, ldh, F, hn, W5, b5, W6, b6, h_out, W1n, b1n, PQn, n_nodes, next_kind, st);
+        return launch_node_tc<PREC_FP16X2, 512, true>(a, n_nodes, next_kind, st);
     if (precision == PREC_BF16X3 && fast_act)
-        return launch_node_tc<PREC_BF16X3, 512, true>(h, ldh, F, hn, W5, b5, W6, b6, h_out, W1n, b1n, PQn, n_nodes, next_kind, st);
+        return launch_node_tc<PREC_BF16X3, 512, true>(a, n_nodes, next_kind, st);
     if (precision == PREC_BF16X3)
-        return launch_node_tc<PREC_BF16X3, 512, false>(h, ldh, F, hn, W5, b5, W6, b6, h_out, W1n, b1n, PQn, n_nodes, next_kind, st);
+        return launch_node_tc<PREC_BF16X3, 512, false>(a, n_nodes, next_kind, st);
     return IS_ERR_ARG;
 }
 

@@ -22,7 +22,7 @@
 #include "common.cuh"
 #include "egnn_common.cuh"
 
-#include "tc_common.cuh"
+#include "egnn_node_tc.cuh"
 
 namespace is {
 
@@ -301,6 +301,19 @@ static int launch_tc(const EdgeCommon& c, float* hn, float* x_out, int grid, cud
 // warp-specialised asynchronous kernel (egnn_tc2.cu): bf16 / bf16x3, destination-side sums on the tensor cores
 int launch_edge_fwd_ws(const EdgeCommon& c, float* hn, float* x_out, int precision, bool update_coords, bool fast,
                        cudaStream_t st);
+// the same kernel with the node tail: one launch per fp16x2 inference layer
+int launch_layer_fwd_fp16x2(const EdgeCommon& c, float* hn, float* x_out, bool update_coords, const NodeArgs& nd, int next_kind,
+                            cudaStream_t st);
+
+static EdgeCommon edge_common(const int* indptr, const int* csr_src, const int* csr_dst, const int* csr_eid, const float* PQ,
+                              const float* x, int64_t ldx, const float* edge_attr, const float* W1, int F, const float* W2,
+                              const float* b2, const float* W3, const float* b3, const float* w4, int64_t n_nodes, int* status) {
+    EdgeCommon c;
+    c.indptr = indptr; c.csr_src = csr_src; c.csr_dst = csr_dst; c.csr_eid = csr_eid;
+    c.PQ = PQ; c.x = x; c.ldx = ldx; c.edge_attr = edge_attr; c.W1 = W1; c.F = F;
+    c.W2 = W2; c.b2 = b2; c.W3 = W3; c.b3 = b3; c.w4 = w4; c.n_nodes = (int)n_nodes; c.status = status;
+    return c;
+}
 
 }  // namespace is
 
@@ -322,10 +335,7 @@ int is_egnn_edge_fwd_tc(const int* indptr, const int* csr_src, const int* csr_ds
     precision &= ~16;
     if (precision != PREC_BF16 && precision != PREC_TF32X3 && precision != PREC_BF16X3 && precision != PREC_FP16X2) return IS_ERR_ARG;
     if (precision == PREC_FP16X2 && legacy) return IS_ERR_ARG;          // the fp16 hi / lo split exists in the warp-specialised kernel only
-    EdgeCommon c;
-    c.indptr = indptr; c.csr_src = csr_src; c.csr_dst = csr_dst; c.csr_eid = csr_eid;
-    c.PQ = PQ; c.x = x; c.ldx = ldx; c.edge_attr = edge_attr; c.W1 = W1; c.F = F;
-    c.W2 = W2; c.b2 = b2; c.W3 = W3; c.b3 = b3; c.w4 = w4; c.n_nodes = (int)n_nodes; c.status = status;
+    const EdgeCommon c = edge_common(indptr, csr_src, csr_dst, csr_eid, PQ, x, ldx, edge_attr, W1, F, W2, b2, W3, b3, w4, n_nodes, status);
     const int sms = current_num_sms();
     const int per_sm = precision == PREC_BF16 ? 3 : precision == PREC_BF16X3 ? 2 : 1;
     int64_t g = (n_nodes + 31) / 32;
@@ -339,6 +349,29 @@ int is_egnn_edge_fwd_tc(const int* indptr, const int* csr_src, const int* csr_ds
     if (precision == PREC_BF16X3)
         return update_coords ? launch_tc<PREC_BF16X3, true, 256>(c, hn, x_out, grid, st, fast_act != 0) : launch_tc<PREC_BF16X3, false, 256>(c, hn, x_out, grid, st, fast_act != 0);
     return update_coords ? launch_tc<PREC_TF32X3, true, 512>(c, hn, x_out, grid, st, fast_act != 0) : launch_tc<PREC_TF32X3, false, 512>(c, hn, x_out, grid, st, fast_act != 0);
+}
+
+// One whole EGNN layer of the fp16x2 inference forward in one launch: is_egnn_edge_fwd_tc (precision 4) followed by
+// is_egnn_node_post_pre_tc (precision 4) on the same arguments, with bit-identical results.  h / ldh / F is the layer's input
+// (the node MLP reads h and the hn this launch computes); update_coords = 0 needs next_kind 2 (W1n = [Wq;Wk;Wv]) or W1n NULL,
+// update_coords = 1 needs next_kind 1.
+int is_egnn_layer_fwd_fp16x2(const int* indptr, const int* csr_src, const int* csr_dst, const int* csr_eid,
+                             const float* PQ, const float* x, int64_t ldx, const float* edge_attr,
+                             const float* W1, int F, const float* W2, const float* b2,
+                             const float* W3, const float* b3, const float* w4, int update_coords, float* hn, float* x_out,
+                             const float* h, int64_t ldh, const float* W5, const float* b5, const float* W6, const float* b6,
+                             float* h_out, const float* W1n, const float* b1n, float* PQn, int next_kind,
+                             int64_t n_nodes, int* status, void* stream) {
+    if (!(F == 20 || F == 64) || n_nodes <= 0 || n_nodes > 0x7fffffff) return IS_ERR_ARG;
+    if ((W1n == nullptr) != (PQn == nullptr)) return IS_ERR_ARG;
+    if (next_kind != 1 && next_kind != 2) return IS_ERR_ARG;
+    if (update_coords && (next_kind != 1 || x_out == nullptr)) return IS_ERR_ARG;
+    if (!update_coords && next_kind == 1 && W1n != nullptr) return IS_ERR_ARG;
+    if (((reinterpret_cast<uintptr_t>(PQ) | reinterpret_cast<uintptr_t>(hn) | reinterpret_cast<uintptr_t>(h_out) |
+          reinterpret_cast<uintptr_t>(PQn)) & 31) != 0) return IS_ERR_ARG;          // 256-bit accesses
+    const EdgeCommon c = edge_common(indptr, csr_src, csr_dst, csr_eid, PQ, x, ldx, edge_attr, W1, F, W2, b2, W3, b3, w4, n_nodes, status);
+    const NodeArgs nd{h, ldh, F, hn, W5, b5, W6, b6, h_out, W1n, b1n, PQn};
+    return launch_layer_fwd_fp16x2(c, hn, x_out, update_coords != 0, nd, next_kind, (cudaStream_t)stream);
 }
 
 }  // extern "C"

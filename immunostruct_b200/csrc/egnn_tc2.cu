@@ -29,7 +29,7 @@
 #include "common.cuh"
 #include "egnn_common.cuh"
 
-#include "tc_common.cuh"
+#include "egnn_node_tc.cuh"
 
 namespace is {
 
@@ -121,7 +121,16 @@ __device__ __forceinline__ void issue_segsum(uint32_t tmem_d, uint32_t s_addr, u
 //   m_full[2]     epilog  -> MMA           acc2_full[2]  MMA2 commit -> epilog
 //   hn_full[2]    MMA3 commit -> epilog (hn rows) and gather (operand buffer + S free again)
 // TMEM: acc1[2] | acc2[2] | hn[2], 64 columns each (512 allocated).  Shared memory: two operand buffers
-// (bf16x3: 2 x 48 KB), W2 / W3 once (48 KB), two selector tiles, four scalar stages: 175 KB.
+// (bf16x3: 2 x 48 KB), W2 / W3 once (48 KB; no W3 without the coordinate branch), two selector tiles, four scalar stages:
+// 175 KB.
+//
+// NODE != 0 (fp16x2 inference forward, egnn_layer_fwd): the kernel is the whole EGNN layer.  A CTA's tiles cover its node
+// range [nbeg, nend) and hold every in-edge of those nodes, so when its last tile is done the CTA has the complete hn of
+// exactly its own nodes -- all the node MLP and the next layer's projections need (node_chain, egnn_node_tc.cuh).  After a
+// CTA barrier warps 0-15 run that chain over [nbeg, nend), in the TMEM allocation and over the operand region of the edge
+// phase; its weight blocks were staged next to W2 / W3 in the prologue.  NODE = 1: P' / Q' of the next layer (or nothing
+// when nd.W1n is null); NODE = 2: the fused QKV projections after the last layer.  The only dependency across the grid is
+// the next layer's gather of P'[src] / Q'[dst], which is the next launch.
 // =====================================================================================================
 namespace e3 {
 using namespace e2;
@@ -172,24 +181,52 @@ __device__ __forceinline__ void meta_edge(const EdgeCommon& p, Meta3& m, int j, 
 // copy of m stays for MMA 3, which reads it transposed as its B operand.
 // The gather maps a quarter-warp to ONE row (8 lanes x 32 bytes = the row's 256 contiguous bytes of P or Q, two whole
 // 128-byte lines per quarter-warp and instruction); with LBO = 144 its eight 16-byte operand stores are conflict free.
-template <int PREC, bool HAS_COORD, bool FAST, bool TSA>
+template <int PREC, bool HAS_COORD>
+__host__ __device__ constexpr uint32_t ws_edge_bytes() {
+    using namespace e3;
+    return 2 * S_BYTES + TcCfg<PREC>::NSPLIT * (2 * A_BYTES + (HAS_COORD ? 2 : 1) * W_BYTES) + sizeof(float) * (5 * 64 + 4 * IS_TM) +
+           NM * sizeof(Meta3);
+}
+
+// shared memory of the node tail: the operand buffers reuse the edge region (which they may outgrow), the weight blocks and
+// biases follow it
+template <int PREC, bool HAS_COORD, int NODE>
+__host__ __device__ constexpr uint32_t ws_node_offset() {
+    using NC = NodeCfg<PREC, NODE>;
+    constexpr uint32_t e = ws_edge_bytes<PREC, HAS_COORD>();
+    return NODE == 0 ? 0u : ((e > NC::A_REGION ? e : NC::A_REGION) + 127u) / 128u * 128u;
+}
+
+template <int PREC, bool HAS_COORD, int NODE>
+__host__ __device__ constexpr uint32_t ws_smem_bytes() {
+    using NC = NodeCfg<PREC, NODE>;
+    return NODE == 0 ? ws_edge_bytes<PREC, HAS_COORD>() : ws_node_offset<PREC, HAS_COORD, NODE>() + NC::W_REGION + NC::VEC_BYTES;
+}
+
+template <int PREC, bool HAS_COORD, bool FAST, bool TSA, int NODE>
 __global__ void __launch_bounds__(e3::NT3, 1)
-edge_fwd_ws_kernel(EdgeCommon p, float* __restrict__ hn, float* __restrict__ x_out) {
+edge_fwd_ws_kernel(EdgeCommon p, float* __restrict__ hn, float* __restrict__ x_out, NodeArgs nd) {
     using namespace e3;
     using C = TcCfg<PREC>;
     constexpr int NS = C::NSPLIT;
     constexpr int CW = 32;                      // accumulator columns per epilogue thread (two column halves)
     constexpr uint32_t ABUF = NS * A_BYTES;     // one operand buffer (all split terms)
     constexpr bool TS2 = TSA && HAS_COORD;      // MMA 2 exists and takes m from TMEM
+    static_assert(NODE == 0 || (PREC == PREC_FP16X2 && FAST), "the node tail is the fp16x2 inference chain");
+    static_assert(ws_smem_bytes<PREC, HAS_COORD, NODE>() <= 227 * 1024 - 1024, "shared memory (+ the static mbarriers)");
     extern __shared__ __align__(128) uint8_t smem_raw[];
     uint8_t* sS = smem_raw;                                            // [2][S_BYTES]; rows 32..63 of a tile alias what follows
     uint8_t* sA = sS + 2 * S_BYTES;                                    // [2][NS][A_BYTES] t1, then m
     uint8_t* sW2 = sA + 2 * ABUF;                                      // [NS][W_BYTES]
-    uint8_t* sW3 = sW2 + NS * W_BYTES;
-    float* vec = reinterpret_cast<float*>(sW3 + NS * W_BYTES);         // b2, b3, w4, wr, wa
+    uint8_t* sW3 = sW2 + NS * W_BYTES;                                 // [NS][W_BYTES] (coordinate branch only)
+    float* vec = reinterpret_cast<float*>(sW3 + (HAS_COORD ? NS * W_BYTES : 0));   // b2, b3, w4, wr, wa
     float* e_c = vec + 5 * 64;                                         // [2 buffers][2 halves][128] partial c
     Meta3* meta = reinterpret_cast<Meta3*>(e_c + 4 * IS_TM);           // [NM]
+    uint8_t* sNW = smem_raw + ws_node_offset<PREC, HAS_COORD, NODE>(); // node tail: [NS][NBLK][W_BYTES], then its biases
+    float* nvec = reinterpret_cast<float*>(sNW + NodeCfg<PREC, NODE>::W_REGION);
     __shared__ __align__(8) uint64_t meta_full[NM], meta_free[NM], a_full[2], acc1_full[2], m_full[2], acc2_full[2], hn_full[2];
+    __shared__ __align__(8) uint64_t node_bar;
+    __shared__ NodeArgs s_nd;     // the tail reads its arguments from here: kept in registers across the edge phase they spill
     __shared__ uint32_t s_tmem;
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -201,9 +238,11 @@ edge_fwd_ws_kernel(EdgeCommon p, float* __restrict__ hn, float* __restrict__ x_o
             mbar_init(&a_full[i], NW_PROD); mbar_init(&m_full[i], NW_EPI);
             mbar_init(&acc1_full[i], 1); mbar_init(&acc2_full[i], 1); mbar_init(&hn_full[i], 1);
         }
+        if (NODE != 0) { mbar_init(&node_bar, 1); s_nd = nd; }
     }
     stage_weight_block<PREC>(sW2, W_BYTES, p.W2, 64, 0, 64, tid, NT3);                 // W2 / W3 as B operands
-    stage_weight_block<PREC>(sW3, W_BYTES, HAS_COORD ? p.W3 : nullptr, 64, 0, 64, tid, NT3);
+    if (HAS_COORD) stage_weight_block<PREC>(sW3, W_BYTES, p.W3, 64, 0, 64, tid, NT3);
+    if (NODE != 0) node_stage_weights<PREC, NODE>(nd, sNW, nvec, tid, NT3);
     if (tid < 64) {
         vec[tid] = p.b2[tid];
         vec[64 + tid] = HAS_COORD ? p.b3[tid] : 0.0f;
@@ -456,26 +495,34 @@ edge_fwd_ws_kernel(EdgeCommon p, float* __restrict__ hn, float* __restrict__ x_o
             if (done) break;
         }
     }
+    if (NODE != 0) {
+        // every MMA of the edge phase has been observed complete through its commit mbarrier by the epilogue warps (acc2_full /
+        // hn_full of the last tile) and every tcgen05.ld / st has been waited for: TMEM and the operand region are free
+        constexpr int NT_NODE = 512;                 // warps 0-15: the epilogue and gather warps
+        static_assert(NodeCfg<PREC, NODE>::NTILE * NodeCfg<PREC, NODE>::TCOLS <= 512, "TMEM columns");
+        fence_before_sync();
+        __syncthreads();
+        fence_after_sync();
+        if (tid < NT_NODE) {
+            uint32_t phase = 0;
+            node_chain<PREC, NT_NODE, FAST, NODE>(s_nd, smem_raw, sNW, nvec, tmem, &node_bar, phase, nbeg,
+                                                  NodeCfg<PREC, NODE>::NTILE * IS_TM, nend, tid, 2);
+        }
+    }
     fence_before_sync();
     __syncthreads();
     if (warp == 0) tmem_dealloc(tmem, 512);
 }
 
-template <int PREC>
-static size_t ws_smem_bytes() {
-    using namespace e3;
-    return 2 * (size_t)S_BYTES + (size_t)TcCfg<PREC>::NSPLIT * (2 * A_BYTES + 2 * W_BYTES) + sizeof(float) * (5 * 64 + 4 * IS_TM) + NM * sizeof(Meta3);
-}
-
 // variant bits of the warp-specialised kernel (is_egnn_set_ws_variant): bit 0 = A operand of MMA 2 from tensor memory
 int g_ws_variant = 1;
 
-template <int PREC, bool HAS_COORD, bool FAST, bool TSA>
-static int launch_wsk_v(const EdgeCommon& c, float* hn, float* x_out, int grid, cudaStream_t st) {
-    const size_t smem = ws_smem_bytes<PREC>();
-    cudaError_t e = cudaFuncSetAttribute(edge_fwd_ws_kernel<PREC, HAS_COORD, FAST, TSA>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+template <int PREC, bool HAS_COORD, bool FAST, bool TSA, int NODE = 0>
+static int launch_wsk_v(const EdgeCommon& c, float* hn, float* x_out, int grid, cudaStream_t st, const NodeArgs& nd = NodeArgs{}) {
+    const size_t smem = ws_smem_bytes<PREC, HAS_COORD, NODE>();
+    cudaError_t e = cudaFuncSetAttribute(edge_fwd_ws_kernel<PREC, HAS_COORD, FAST, TSA, NODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
-    edge_fwd_ws_kernel<PREC, HAS_COORD, FAST, TSA><<<grid, e3::NT3, smem, st>>>(c, hn, x_out);
+    edge_fwd_ws_kernel<PREC, HAS_COORD, FAST, TSA, NODE><<<grid, e3::NT3, smem, st>>>(c, hn, x_out, nd);
     e = cudaGetLastError();
     return e == cudaSuccess ? 0 : (int)e;
 }
@@ -486,13 +533,17 @@ static int launch_wsk(const EdgeCommon& c, float* hn, float* x_out, int grid, cu
     return launch_wsk_v<PREC, HAS_COORD, FAST, false>(c, hn, x_out, grid, st);
 }
 
+static int ws_grid(int n_nodes) {
+    const int sms = current_num_sms();
+    int64_t g = ((int64_t)n_nodes + 31) / 32;
+    if (g > sms) g = sms;
+    return (int)(g < 1 ? 1 : g);
+}
+
 // entry used by is_egnn_edge_fwd_tc (egnn_tc.cu) for the bf16 / bf16x3 precisions: warp-specialised kernel
 int launch_edge_fwd_ws(const EdgeCommon& c, float* hn, float* x_out, int precision, bool update_coords, bool fast,
                        cudaStream_t st) {
-    const int sms = current_num_sms();
-    int64_t g = ((int64_t)c.n_nodes + 31) / 32;
-    if (g > sms) g = sms;
-    const int grid = (int)(g < 1 ? 1 : g);
+    const int grid = ws_grid(c.n_nodes);
     if (precision == PREC_BF16)
         return update_coords ? launch_wsk<PREC_BF16, true, true>(c, hn, x_out, grid, st)
                              : launch_wsk<PREC_BF16, false, true>(c, hn, x_out, grid, st);
@@ -504,6 +555,17 @@ int launch_edge_fwd_ws(const EdgeCommon& c, float* hn, float* x_out, int precisi
                              : launch_wsk<PREC_BF16X3, false, true>(c, hn, x_out, grid, st);
     return update_coords ? launch_wsk<PREC_BF16X3, true, false>(c, hn, x_out, grid, st)
                          : launch_wsk<PREC_BF16X3, false, false>(c, hn, x_out, grid, st);
+}
+
+// the whole fp16x2 inference layer in one launch (is_egnn_layer_fwd_fp16x2): edge phase with the node tail.  With the
+// coordinate branch: P' / Q' of the next layer; without: the QKV projections (next_kind 2) or P' / Q' (W1n null: h' only).
+// MMA 2 always takes m from tensor memory (the default variant of the two-kernel path).
+int launch_layer_fwd_fp16x2(const EdgeCommon& c, float* hn, float* x_out, bool update_coords, const NodeArgs& nd, int next_kind,
+                            cudaStream_t st) {
+    const int grid = ws_grid(c.n_nodes);
+    if (update_coords) return launch_wsk_v<PREC_FP16X2, true, true, true, 1>(c, hn, x_out, grid, st, nd);
+    if (next_kind == 2) return launch_wsk_v<PREC_FP16X2, false, true, false, 2>(c, hn, x_out, grid, st, nd);
+    return launch_wsk_v<PREC_FP16X2, false, true, false, 1>(c, hn, x_out, grid, st, nd);
 }
 
 }  // namespace is

@@ -203,6 +203,9 @@ def _egnn_stack_forward(graph, x23, edge_attr, params, fast_act, keep, qkv=None)
         prec = _C.PREC_BF16X3                  # training: the backward kernels recompute the forward in the bf16x3 split
     node_prec = {None: None, _C.PREC_BF16: _C.PREC_BF16, _C.PREC_TF32X3: _C.PREC_BF16X3, _C.PREC_BF16X3: _C.PREC_BF16X3,
                  _C.PREC_FP16X2: _C.PREC_FP16X2}[prec]
+    # fp16x2 inference: one launch per layer, the node kernel's chain runs as the tail of the edge kernel (same arithmetic,
+    # bit-identical).  The CPU kernel contracts (tests) model the two launches.
+    fused = prec == _C.PREC_FP16X2 and not _C.lib_is_patched()
     # (training forward: the fused tensor-core node kernel with the accurate SiLU and all eight bf16x3 partial
     #  products, fast_act = False -- with six products a handful of parameter gradients landed at 1.0-1.3e-5 of
     #  their scale on the B200, just outside the 1e-5 gradient tolerance)
@@ -215,24 +218,31 @@ def _egnn_stack_forward(graph, x23, edge_attr, params, fast_act, keep, qkv=None)
         upd = l != last
         hn, h_out = _new(h, n, H), _new(h, n, H)
         x_out = _new(h, n, 3) if upd else None
-        if prec is None:
-            _C.egnn_edge_fwd(graph, PQ, x, edge_attr, f, W1, W2, b2, W3, b3, w4, upd, hn, x_out)
-        else:
-            _C.egnn_edge_fwd_tc(graph, PQ, x, edge_attr, f, W1, W2, b2, W3, b3, w4, upd, prec, hn, x_out,
-                                fast_act=fast_act)
         nxt = params[l + 1] if upd else None
         PQ_next = _new(h, n, 2 * H) if upd else None
-        if node_prec is None:
+        if fused:
+            if not upd and qkv is not None:
+                QKV = _new(h, n, 3 * H)
+                W1n, b1n, PQn, kind = qkv[0], qkv[1], QKV, 2
+            else:
+                W1n, b1n, PQn, kind = (nxt[0], nxt[1], PQ_next, 1) if upd else (None, None, None, 1)
+            _C.egnn_layer_fwd_fp16x2(graph, PQ, x, edge_attr, W1, W2, b2, W3, b3, w4, upd, hn, x_out,
+                                     h, W5, b5, W6, b6, h_out, W1n, b1n, PQn, next_kind=kind)
+        elif prec is None:
+            _C.egnn_edge_fwd(graph, PQ, x, edge_attr, f, W1, W2, b2, W3, b3, w4, upd, hn, x_out)
             _C.egnn_node_post_fwd(h, hn, W5, b5, W6, b6, h_out)
             if upd:
                 _C.egnn_node_pre_fwd(h_out, nxt[0], nxt[1], PQ_next)
-        elif not upd and qkv is not None:
-            QKV = _new(h, n, 3 * H)
-            _C.egnn_node_post_pre_tc(h, hn, W5, b5, W6, b6, h_out, qkv[0], qkv[1], QKV, node_prec,
-                                     fast_act=fast_act, next_kind=2)
         else:
-            _C.egnn_node_post_pre_tc(h, hn, W5, b5, W6, b6, h_out, nxt[0] if upd else None,
-                                     nxt[1] if upd else None, PQ_next, node_prec, fast_act=fast_act)
+            _C.egnn_edge_fwd_tc(graph, PQ, x, edge_attr, f, W1, W2, b2, W3, b3, w4, upd, prec, hn, x_out,
+                                fast_act=fast_act)
+            if not upd and qkv is not None:
+                QKV = _new(h, n, 3 * H)
+                _C.egnn_node_post_pre_tc(h, hn, W5, b5, W6, b6, h_out, qkv[0], qkv[1], QKV, node_prec,
+                                         fast_act=fast_act, next_kind=2)
+            else:
+                _C.egnn_node_post_pre_tc(h, hn, W5, b5, W6, b6, h_out, nxt[0] if upd else None,
+                                         nxt[1] if upd else None, PQ_next, node_prec, fast_act=fast_act)
         if keep is not None:
             keep.append((h, x, PQ, hn))
         h, PQ = h_out, PQ_next

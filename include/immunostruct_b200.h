@@ -60,6 +60,18 @@ int is_egnn_edge_fwd_tc(const int* indptr, const int* csr_src, const int* csr_ds
                         const float* W1, int F, const float* W2, const float* b2,
                         const float* W3, const float* b3, const float* w4, int update_coords, int precision,
                         int fast_act, float* hn, float* x_out, int64_t n_nodes, int* status, void* stream);
+/* One whole EGNN layer of the fp16x2 inference forward in one launch (csrc/egnn_tc2.cu): is_egnn_edge_fwd_tc with precision 4
+ * followed by is_egnn_node_post_pre_tc with precision 4, bit-identical.  Each CTA runs the node MLP and the next projections of
+ * its own destination nodes once its edge tiles are done, so hn is written and read back within the launch.  h / ldh / F =
+ * the layer's input features; update_coords 1 needs next_kind 1 (W1n = next edge_mlp.0.weight [64,130], PQn [n,128]);
+ * update_coords 0 takes next_kind 2 (W1n = [Wq;Wk;Wv] [192,64], PQn = QKV [n,192]) or W1n / b1n / PQn NULL. */
+int is_egnn_layer_fwd_fp16x2(const int* indptr, const int* csr_src, const int* csr_dst, const int* csr_eid,
+                             const float* PQ, const float* x, int64_t ldx, const float* edge_attr,
+                             const float* W1, int F, const float* W2, const float* b2,
+                             const float* W3, const float* b3, const float* w4, int update_coords, float* hn, float* x_out,
+                             const float* h, int64_t ldh, const float* W5, const float* b5, const float* W6, const float* b6,
+                             float* h_out, const float* W1n, const float* b1n, float* PQn, int next_kind,
+                             int64_t n_nodes, int* status, void* stream);
 /* operand-buffer depth of the warp-specialised edge forward kernel (csrc/egnn_tc2.cu): only 2 is accepted (a third
    buffer was measured without gain and no longer fits next to the padded operand tiles) */
 int is_egnn_set_ws_buffers(int n);
