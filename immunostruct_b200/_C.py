@@ -50,7 +50,7 @@ def exported_symbols():
             "is_contrastive_bwd", "is_fused_adam", "is_rotate_coords", "is_mask_single_residue", "is_mask_rows", "is_gemm_tma_split_k",
             "is_split_planes", "is_gemm_planes_tma", "is_egnn_set_ws_buffers", "is_egnn_set_ws_variant", "is_reduce_partials3", "is_fused_adam_capturable",
             "is_egnn_edge_attr_grad", "is_head_mc_infer", "is_mutscan_expand", "is_variant_expand", "is_design_expand",
-            "is_design_select", "is_egnn_layer_fwd_fp16x2"]
+            "is_design_select", "is_egnn_layer_fwd_fp16x2", "is_occlusion_expand"]
 
 
 def _check(rc: int, name: str):
@@ -645,6 +645,34 @@ def design_select(beam, round_logits, round_mean, round_std, native, allowed, no
           _i32(w), _i32(n_states), _i32(k), _i32(max_mutations), _f32(kappa), _i32(1 if maximize else 0),
           *(_t(t, d, n + "_out") for t, d, n in zip(beam_out, types, names)), _t(best, f32, "best", contiguous=False),
           _i64(best.stride(0)), _stream())
+
+
+def occlusion_expand(x23, node_off, edge_off, src_local, dst_local, edge_attr, sample, node_a, node_b, node_out, edge_out,
+                     x23_out, src_out, dst_out, edge_attr_out, flag):
+    """One pass of structural occlusion variants (csrc/occlusion.cu): variant v is base graph sample[v] with row node_a[v]
+    and its edges removed (node_b[v] == -1: the row's 23 floats become 0.0) or with every edge of the contact
+    {node_a[v], node_b[v]} removed; x23 rows from node_out[v], the kept edges in base order (graph-local endpoints,
+    attributes) from edge_out[v].  ``flag`` (int32 [1], zeroed by the caller) is raised, and the variant not written, for
+    an index out of range, node_b == node_a, or output offsets that disagree with the node count or the kept edge count."""
+    f32, i64, i32 = torch.float32, torch.int64, torch.int32
+    if x23.dim() != 2 or sample.dim() != 1:
+        raise ValueError("occlusion_expand: x23 [N,23] and sample [r] expected")
+    b, r, e = node_off.shape[0] - 1, sample.shape[0], src_local.shape[0]
+    if (x23.shape[1] != 23 or b < 1 or edge_off.shape != (b + 1,) or dst_local.shape != (e,) or edge_attr.numel() != e
+            or node_a.shape != (r,) or node_b.shape != (r,) or r < 1):
+        raise ValueError("occlusion_expand: unexpected input shapes")
+    n_out, e_out = x23_out.shape[0], src_out.shape[0]
+    if (x23_out.dim() != 2 or x23_out.shape[1] != 23 or node_out.shape != (r + 1,) or edge_out.shape != (r + 1,)
+            or dst_out.shape != (e_out,) or edge_attr_out.numel() != e_out or flag.shape != (1,)):
+        raise ValueError("occlusion_expand: unexpected output shapes")
+    if 2 * r > 0x7ffffffe:
+        raise ValueError("occlusion_expand: too many variants in one pass")
+    _call("is_occlusion_expand", _t(x23, f32, "x23"), _t(node_off, i64, "node_off"), _t(edge_off, i64, "edge_off"),
+          _t(src_local, i64, "src_local"), _t(dst_local, i64, "dst_local"), _t(edge_attr, f32, "edge_attr"),
+          _t(sample, i64, "sample"), _t(node_a, i64, "node_a"), _t(node_b, i64, "node_b"), _t(node_out, i64, "node_out"),
+          _t(edge_out, i64, "edge_out"), _i32(r), _i32(b), _i64(n_out), _i64(e_out), _t(x23_out, f32, "x23_out"),
+          _t(src_out, i64, "src_out"), _t(dst_out, i64, "dst_out"), _t(edge_attr_out, f32, "edge_attr_out"),
+          _t(flag, i32, "flag"), _stream())
 
 
 def unpack_nodes(aa, xyz, x):

@@ -282,6 +282,22 @@ int is_design_select(const int64_t* states, const int64_t* keys, const int64_t* 
                      int max_mutations, float kappa, int maximize, int64_t* states_out, int64_t* keys_out,
                      int64_t* n_mut_out, unsigned char* valid_out, float* logits_out, float* mean_out, float* std_out,
                      float* objective_out, float* best, int64_t best_stride, void* stream);
+/* is_occlusion_expand (csrc/occlusion.cu): one pass of single-removal structural variants of a resident batch (x23
+ * [N,23], node_off / edge_off [B+1], graph-local src_local / dst_local int64 [E], edge_attr [E,1]).  Variant v < r is a
+ * copy of base graph b = sample[v] (int64 [r]) with one removal: node_b[v] == -1 occludes graph-local row a = node_a[v]
+ * (its 23 floats become 0.0 and every edge with src == a or dst == a is dropped), node_b[v] >= 0 occludes the contact
+ * {a, node_b[v]} (every edge a -> node_b or node_b -> a is dropped; rows unchanged, self-loops never dropped).  Its x23
+ * rows go to x23_out from row node_out[v], its kept edges, in base order, with graph-local endpoints and their
+ * attributes, to src_out / dst_out / edge_attr_out from edge_out[v] (node_out / edge_out int64 [r+1]: the caller's
+ * running sums of the node counts and of the kept edge counts).  Bit-exact (copies and 0.0 only).  flag (int32 [1],
+ * zeroed by the caller, never cleared) is set to 1, and that variant is not written, for a sample outside [0, B), node_a
+ * outside [0, n_b), node_b outside [-1, n_b) or equal to node_a, node_out[v+1] - node_out[v] != n_b, a kept count that
+ * is not edge_out[v+1] - edge_out[v], or offsets past n_nodes_out / n_edges_out.  No atomics. */
+int is_occlusion_expand(const float* x23, const int64_t* node_off, const int64_t* edge_off, const int64_t* src_local,
+                        const int64_t* dst_local, const float* edge_attr, const int64_t* sample, const int64_t* node_a,
+                        const int64_t* node_b, const int64_t* node_out, const int64_t* edge_out, int r, int n_graphs,
+                        int64_t n_nodes_out, int64_t n_edges_out, float* x23_out, int64_t* src_out, int64_t* dst_out,
+                        float* edge_attr_out, int* flag, void* stream);
 /* Dense Linear layer on the tensor cores: C[M,N] = act(A[M,K] W[N,K]^T + bias), fp32 in / out, operands split
  * on the fly into three bf16 terms (precision 3, fp32-accurate) or rounded to bf16 (precision 0).  Replaces the
  * nn.Linear layers of the sequence VAE (reference models/hybrid_models.py:63-74: vae_fc1 with ReLU, vae_fc4) in the
