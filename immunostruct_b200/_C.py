@@ -50,7 +50,7 @@ def exported_symbols():
             "is_contrastive_bwd", "is_fused_adam", "is_rotate_coords", "is_mask_single_residue", "is_mask_rows", "is_gemm_tma_split_k",
             "is_split_planes", "is_gemm_planes_tma", "is_egnn_set_ws_buffers", "is_egnn_set_ws_variant", "is_reduce_partials3", "is_fused_adam_capturable",
             "is_egnn_edge_attr_grad", "is_head_mc_infer", "is_mutscan_expand", "is_variant_expand", "is_design_expand",
-            "is_design_select", "is_egnn_layer_fwd_fp16x2", "is_occlusion_expand"]
+            "is_design_select", "is_egnn_layer_fwd_fp16x2", "is_occlusion_expand", "is_coord_noise_expand"]
 
 
 def _check(rc: int, name: str):
@@ -673,6 +673,33 @@ def occlusion_expand(x23, node_off, edge_off, src_local, dst_local, edge_attr, s
           _t(edge_out, i64, "edge_out"), _i32(r), _i32(b), _i64(n_out), _i64(e_out), _t(x23_out, f32, "x23_out"),
           _t(src_out, i64, "src_out"), _t(dst_out, i64, "dst_out"), _t(edge_attr_out, f32, "edge_attr_out"),
           _t(flag, i32, "flag"), _stream())
+
+
+def coord_noise_expand(x23, node_off, sigma, seed, item, draw0, x23_out):
+    """One pass of seeded coordinate perturbations (csrc/coordnoise.cu): x23_out [r*N, 23] becomes r copies of the base
+    batch in the layout of ``GraphBatch.replicate(r)``, copy k being structure draw m = draw0 + k: columns 20..22 of
+    graph-local row a of graph b get ``fmaf(sigma[i], z, x)``, z the Philox4x32-10 / Box-Muller normals of the key
+    (seed, item, m, b, a); columns 0..19 and rows with sigma 0 are copied.  Every argument is checked here: the kernel
+    has no flag."""
+    f32, i64 = torch.float32, torch.int64
+    if x23.dim() != 2 or x23.shape[1] != 23 or node_off.dim() != 1 or node_off.shape[0] < 2:
+        raise ValueError("coord_noise_expand: x23 [N,23] and node_off [B+1] expected")
+    n, b = x23.shape[0], node_off.shape[0] - 1
+    if sigma.shape != (n,):
+        raise ValueError("coord_noise_expand: sigma [N] expected")
+    if x23_out.dim() != 2 or x23_out.shape[1] != 23 or x23_out.shape[0] < n or (n and x23_out.shape[0] % n):
+        raise ValueError("coord_noise_expand: x23_out [r*N, 23] expected")
+    r = x23_out.shape[0] // n if n else 1
+    if not (isinstance(seed, int) and 0 <= seed < 2 ** 64 and isinstance(item, int) and 0 <= item < 2 ** 32
+            and isinstance(draw0, int) and 0 <= draw0 and draw0 + r <= 2 ** 32):
+        raise ValueError("coord_noise_expand: seed in [0, 2^64), item in [0, 2^32) and draw0 + r <= 2^32 expected")
+    if r * b > 0x7fffffff:
+        raise ValueError("coord_noise_expand: r * B too large")
+    if x23_out.data_ptr() == x23.data_ptr():
+        raise ValueError("coord_noise_expand: x23_out must not alias x23")
+    _call("is_coord_noise_expand", _t(x23, f32, "x23"), _t(node_off, i64, "node_off"), _t(sigma, f32, "sigma"), _i32(r),
+          _i32(b), _i64(n), ctypes.c_uint64(seed), ctypes.c_uint32(item), ctypes.c_uint32(draw0),
+          _t(x23_out, f32, "x23_out"), _stream())
 
 
 def unpack_nodes(aa, xyz, x):

@@ -298,6 +298,15 @@ int is_occlusion_expand(const float* x23, const int64_t* node_off, const int64_t
                         const int64_t* node_b, const int64_t* node_out, const int64_t* edge_out, int r, int n_graphs,
                         int64_t n_nodes_out, int64_t n_edges_out, float* x23_out, int64_t* src_out, int64_t* dst_out,
                         float* edge_attr_out, int* flag, void* stream);
+/* is_coord_noise_expand (csrc/coordnoise.cu): one pass of r seeded coordinate perturbations of a resident batch (x23
+ * [N,23], node_off [B+1], sigma fp32 [N] per node row), in the layout of GraphBatch.replicate(r): x23_out [r N, 23],
+ * copy k of graph b at rows k N + node_off[b].  Copy k is structure draw m = draw0 + k: graph-local row a of graph b
+ * keeps columns 0..19 and gets x_c + sigma z_c (fmaf) in columns 20..22, z = three standard normals of Philox4x32-10
+ * with counter (a, b, m, item) and key (low, high 32 bits of seed), by Box-Muller on u_j = ((v_j >> 8) + 0.5) 2^-24:
+ * z0 = sqrt(-2 log u0) cospi(2 u1), z1 = sqrt(-2 log u0) sinpi(2 u1), z2 = sqrt(-2 log u2) cospi(2 u3).  Rows with
+ * sigma == 0 are copied bit-exact.  No device flag: the caller checks every argument (draw0 + r <= 2^32).  No atomics. */
+int is_coord_noise_expand(const float* x23, const int64_t* node_off, const float* sigma, int r, int n_graphs,
+                          int64_t n_nodes, uint64_t seed, uint32_t item, uint32_t draw0, float* x23_out, void* stream);
 /* Dense Linear layer on the tensor cores: C[M,N] = act(A[M,K] W[N,K]^T + bias), fp32 in / out, operands split
  * on the fly into three bf16 terms (precision 3, fp32-accurate) or rounded to bf16 (precision 0).  Replaces the
  * nn.Linear layers of the sequence VAE (reference models/hybrid_models.py:63-74: vae_fc1 with ReLU, vae_fc4) in the
