@@ -33,8 +33,8 @@ import torch
 from . import functional as IF
 from .comparative_models import _Comparative
 from .hybrid_models import _Hybrid
-from .mutagenesis import _check_scan, scan_passes
-from .predictive import _CLASSES, _PAIR_CLASSES, Predictive, _draws, _encode, _head_params, _pair_items
+from .predictive import _CLASSES, _PAIR_CLASSES, Predictive, _check, _repeat, _scorer, _scorer_pair
+from .resident import replicas, scan_passes, score_replicas
 
 Tensor = torch.Tensor
 
@@ -101,30 +101,22 @@ def _statistics(logits):
     return tuple(t.float() for t in (mean, std, std_s, std_l))
 
 
-def _run(model, perturbed, fixed, layout, passes, structures, seed, b, k):
-    """Every structure draw in passes -> logits [B, M, K].
+def _ensemble(model, scorer, perturbed, passes, seed):
+    """Every structure draw in replica passes -> logits [B, M, K].  ``perturbed``: (graph, sigma) of the scored item and,
+    when the wild type is perturbed too, of the wild type; item i draws from stream item i.  A wild type that is not
+    perturbed stays the scorer's fixed one."""
+    encoded = [scorer.item[1:], None if scorer.wt is None else scorer.wt[1:]]
+    reps = replicas(passes, lambda r: [(g.replicate(r), tuple(_repeat(t, r) for t in enc))
+                                       for (g, _), enc in zip(perturbed, encoded)])
+    bases = [(g.ndata["x"].detach().contiguous(), g.node_off, s) for g, s in perturbed]
 
-    ``perturbed``: one (graph, sigma, item id, (mu, logvar, z_vae, eps)) per perturbed item; ``fixed``: the (pooled, mu,
-    logvar, z_vae, eps) of a wild type that is not perturbed, or None; ``layout``: the head's items, each an index into
-    ``perturbed`` or -1 for ``fixed``.  Replicas and repeated tensors are built for every distinct r before the first
-    pass, so the loop holds no collation and no host read."""
-    params = _head_params(model)
-    dev = perturbed[0][0].ndata["x"].device
-    reps = {}
-    for r in sorted({r for _, r in passes}):
-        rep = lambda t: t.repeat(1, r, 1) if t.dim() == 3 else t.repeat(r, 1)
-        reps[r] = ([(g.replicate(r), tuple(rep(t) for t in enc)) for g, _, _, enc in perturbed],
-                   None if fixed is None else tuple(rep(t) for t in fixed))
-    bases = [(g.ndata["x"].detach().contiguous(), g.node_off, s, item) for g, s, item, _ in perturbed]
-    logits = torch.empty(structures, b, k, dtype=torch.float32, device=dev)
-    for j, r in passes:
-        copies, wt = reps[r]
-        for (x, node_off, s, item), (g, _) in zip(bases, copies):
+    def run_pass(j, r, *copies):
+        for item, ((x, node_off, s), (g, _)) in enumerate(zip(bases, copies)):
             IF._C.coord_noise_expand(x, node_off, s, seed, item, j, g.ndata["x"])
         items = [(model.structure_embedding(g, project=False)[0].contiguous(),) + enc for g, enc in copies]
-        lg, _, _ = IF._C.head_mc_infer([wt if i < 0 else items[i] for i in layout], *params)
-        logits[j:j + r] = lg.reshape(r, b, k)
-    return logits.permute(1, 0, 2).contiguous()
+        return scorer.score(items[0], r=r, wt=items[1] if len(items) == 2 else None)
+
+    return score_replicas(scorer, passes, reps, run_pass)[0].permute(1, 0, 2).contiguous()
 
 
 def _result(logits, seed, base):
@@ -144,20 +136,13 @@ def coordinate_ensemble(model, graph, seq, prop, *, sigma, structures: int = 16,
     of a sample share its draws.  Structures run in passes of at most ``max_graphs`` graphs.  Follows ``model.forward``
     for the eight classes ``predictive`` supports; the model must be in eval mode; no_grad, and every ``.grad`` is left
     untouched.  ``prob_std^2 = std_structure^2 + std_latent^2`` (the law of total variance, computed in fp64)."""
-    _check_scan(model, samples, (_Hybrid, _Comparative), "coordinate_ensemble", _CLASSES)
+    _check(model, samples, (_Hybrid, _Comparative), "coordinate_ensemble", _CLASSES)
     s, bad = _sigma(sigma, graph, "sigma")
-    b = graph.n_graphs
-    seed, passes = _checked(structures, seed, b, max_graphs, [("sigma", bad)])
-    pair = isinstance(model, _Comparative) and model.use_wt_for_downstream
+    seed, passes = _checked(structures, seed, graph.n_graphs, max_graphs, [("sigma", bad)])
     with torch.no_grad():
-        e = _draws(model, eps, samples, b, graph.ndata["x"])
-        pooled, mu, logvar, z_vae = _encode(model, graph, seq, prop)
-        item = (pooled, mu, logvar, z_vae, e)
-        base = Predictive(*IF._C.head_mc_infer([item, item] if pair else [item], *_head_params(model)))
-        # model.forward of a pair-wide head repeats the one item
-        logits = _run(model, [(graph, s, 0, item[1:])], None, [0, 0] if pair else [0], passes, structures, seed, b,
-                      e.shape[0])
-    return _result(logits, seed, base)
+        scorer = _scorer(model, graph, seq, prop, eps, samples)
+        logits = _ensemble(model, scorer, [(graph, s)], passes, seed)
+    return _result(logits, seed, scorer.base)
 
 
 def coordinate_ensemble_pair(model, graph_pair, seq_pair, prop_pair, *, sigma, structures: int = 16,
@@ -172,28 +157,19 @@ def coordinate_ensemble_pair(model, graph_pair, seq_pair, prop_pair, *, sigma, s
     Without ``use_wt_for_downstream`` the wild type is neither run nor drawn for, and sigma_w must be None.  ``eps`` =
     (eps_c, eps_w), each [K, B, latent], or one ``model.sample_eps`` call of [K*B, latent] per item, cancer first.
     ``base`` equals ``predictive_pair`` on the same draws."""
-    _check_scan(model, samples, _Comparative, "coordinate_ensemble_pair", _PAIR_CLASSES)
-    n = _pair_items(model, eps)
+    _check(model, samples, _Comparative, "coordinate_ensemble_pair", _PAIR_CLASSES)
     if not isinstance(sigma, (tuple, list)) or len(sigma) != 2 or sigma[0] is None:
         raise ValueError("sigma must be a pair (sigma_c, sigma_w); sigma_w may be None")
-    if n == 1 and sigma[1] is not None:
+    if not model.use_wt_for_downstream and sigma[1] is not None:
         raise ValueError("sigma_w needs use_wt_for_downstream: without it the wild type does not enter the score")
     gc = graph_pair[0]
     b = gc.n_graphs
-    if n == 2 and graph_pair[1].n_graphs != b:
+    if model.use_wt_for_downstream and graph_pair[1].n_graphs != b:
         raise ValueError("the cancer and wild-type batches must hold the same number of graphs")
     s_c, bad_c = _sigma(sigma[0], gc, "sigma_c")
     s_w, bad_w = (None, None) if sigma[1] is None else _sigma(sigma[1], graph_pair[1], "sigma_w")
     seed, passes = _checked(structures, seed, b, max_graphs, [("sigma_c", bad_c), ("sigma_w", bad_w)])
     with torch.no_grad():
-        k = samples if eps is None else eps[0].shape[0]
-        draws = [_draws(model, None if eps is None else eps[i], k, b, graph_pair[i].ndata["x"]) for i in range(n)]
-        items = [_encode(model, graph_pair[i], seq_pair[i], prop_pair[i]) + (draws[i],) for i in range(n)]
-        base = Predictive(*IF._C.head_mc_infer(items, *_head_params(model)))
-        perturbed = [(gc, s_c, 0, items[0][1:])]
-        if s_w is not None:
-            perturbed.append((graph_pair[1], s_w, 1, items[1][1:]))
-        layout = [0] if n == 1 else [0, 1 if s_w is not None else -1]
-        logits = _run(model, perturbed, items[1] if n == 2 and s_w is None else None, layout, passes, structures,
-                      seed, b, k)
-    return _result(logits, seed, base)
+        scorer = _scorer_pair(model, graph_pair, seq_pair, prop_pair, eps, samples)
+        logits = _ensemble(model, scorer, [(gc, s_c)] + ([] if s_w is None else [(graph_pair[1], s_w)]), passes, seed)
+    return _result(logits, seed, scorer.base)

@@ -34,8 +34,10 @@ import torch
 from . import functional as IF
 from .comparative_models import _Comparative
 from .hybrid_models import _Hybrid
-from .mutagenesis import N_RESIDUES, _check_scan, _site_tables, scan_passes
-from .predictive import _CLASSES, _PAIR_CLASSES, Predictive, _draws, _encode, _head_params, _pair_items
+from .mutagenesis import _site_tables
+from .predictive import _CLASSES, _PAIR_CLASSES, Predictive, _check, _encode, _scorer, _scorer_pair
+from .resident import (N_RESIDUES, check_one_hot, native_residues, replicas, scan_passes, score_replicas,
+                       sequence_replica)
 
 Tensor = torch.Tensor
 MAX_SITES = 14            # keys sum_p state[p] 20^p must fit int64
@@ -84,19 +86,15 @@ def _design_args(b, n_sites, allowed, max_mutations, beam, rounds, kappa, dev):
     return allowed.to(dev).expand(b, n_sites, N_RESIDUES), m, t, float(torch.tensor(float(kappa), dtype=torch.float32))
 
 
-def _search(model, graph, seq, prop, ni, si, cols, allowed, max_mut, beam, rounds, maximize, kappa, e, base, items_of,
-            max_graphs):
-    """The rounds of one search -> Design fields without ``base``.  ``items_of(item, r)`` turns the mutant item of an
-    r-copy pass into the head's item list."""
-    params = _head_params(model)
+def _search(model, scorer, graph, seq, prop, ni, si, cols, allowed, max_mut, beam, rounds, maximize, kappa, max_graphs):
+    """The rounds of one search -> Design fields without ``base``."""
+    base = scorer.base
     b, n_sites = ni.shape
     x = graph.ndata["x"].detach().contiguous()
     seq = seq.detach().contiguous()
-    prop = prop.detach().contiguous()
-    L, V, k, dev = seq.shape[1], seq.shape[2], e.shape[0], x.device
+    k, dev = scorer.item[4].shape[0], x.device
     f32, i64 = dict(dtype=torch.float32, device=dev), dict(dtype=torch.int64, device=dev)
-    rows = graph.node_off[:-1].unsqueeze(1) + ni.clamp_min(0)
-    native = torch.where(ni < 0, -1, x[rows.reshape(-1), :N_RESIDUES].argmax(1).reshape(b, n_sites)).contiguous()
+    native = native_residues(graph, ni)
     allowed = allowed.clone()
     allowed.scatter_(2, native.clamp_min(0).unsqueeze(2), torch.ones(b, n_sites, 1, dtype=torch.bool, device=dev))
     nan = float("nan")
@@ -118,27 +116,22 @@ def _search(model, graph, seq, prop, ni, si, cols, allowed, max_mut, beam, round
     history[:, 0] = obj0
     sizes = round_slots(n_sites, beam, rounds)
     plans = {s: scan_passes(s, b, max_graphs) for s in set(sizes)}
-    passes = {}
-    for r in sorted({r for plan in plans.values() for _, r in plan}):    # topology of r copies, collated before round 1
-        passes[r] = (graph.replicate(r), torch.empty(r * b, L, V, **f32), prop.repeat(r, 1), e.repeat(1, r, 1))
-    n_max = max(sizes)
-    r_logits, r_mean, r_std = torch.empty(n_max, b, k, **f32), torch.empty(n_max, b, **f32), torch.empty(n_max, b, **f32)
+    # topology of r copies, collated before round 1
+    reps = replicas([p for plan in plans.values() for p in plan], sequence_replica(graph, seq, prop, scorer.item[4]))
     flag = torch.zeros(1, dtype=torch.int32, device=dev)
+
+    def run_pass(j, r, g, seq_r, prop_r, e_r):             # slots j .. j+r-1 of the current round
+        IF._C.design_expand(x, graph.node_off, ni, seq, si, cols, cur, native, allowed, n_states, max_mut, j,
+                            g.ndata["x"], seq_r, flag)
+        return scorer.score(_encode(model, g, seq_r, prop_r) + (e_r,), r=r)
+
     for t, n_slots in enumerate(sizes, 1):
         n_states = 1 if t == 1 else beam
-        for j, r in plans[n_slots]:
-            g, seq_r, prop_r, e_r = passes[r]
-            IF._C.design_expand(x, graph.node_off, ni, seq, si, cols, cur, native, allowed, n_states, max_mut, j,
-                                g.ndata["x"], seq_r, flag)
-            item = _encode(model, g, seq_r, prop_r) + (e_r,)
-            lg, m, s = IF._C.head_mc_infer(items_of(item, r), *params)
-            r_logits[j:j + r], r_mean[j:j + r], r_std[j:j + r] = lg.reshape(r, b, k), m.reshape(r, b), s.reshape(r, b)
-        IF._C.design_select(cur, r_logits[:n_slots], r_mean[:n_slots], r_std[:n_slots], native, allowed, ni, n_states,
-                            max_mut, kappa, maximize, nxt, history[:, t])
+        r_logits, r_mean, r_std = score_replicas(scorer, plans[n_slots], reps, run_pass)
+        IF._C.design_select(cur, r_logits, r_mean, r_std, native, allowed, ni, n_states, max_mut, kappa, maximize, nxt,
+                            history[:, t])
         cur, nxt = nxt, cur
-    if flag.item():
-        raise ValueError("a site row is not exactly one-hot in the graph's residue columns or in the sequence, or its "
-                         "sequence column is not seq_columns[residue column] (a padded or masked row, or a wrong map)")
+    check_one_hot(flag, "a site row")
     states, _, n_mut, valid, logits, mean, std, obj = cur
     return states, n_mut, valid, logits, mean, std, obj, history
 
@@ -165,18 +158,14 @@ def beam_search(model, graph_data, sequence_data, peptide_property, node_index: 
     (K = ``samples``) makes them; every candidate of sample b uses sample b's draws.  Rounds run in passes of at most
     ``max_graphs`` graphs.  Follows ``model.forward`` for the eight classes ``predictive`` supports; the model must be in
     eval mode; no_grad, and every ``.grad`` is left untouched."""
-    _check_scan(model, samples, (_Hybrid, _Comparative), "beam_search", _CLASSES)
+    _check(model, samples, (_Hybrid, _Comparative), "beam_search", _CLASSES)
     ni, si, cols, allowed, max_mut, rounds, kappa = _prepare(graph_data, sequence_data, node_index, seq_index, seq_columns,
                                                              allowed, max_mutations, beam, rounds, kappa, max_graphs)
-    pair = isinstance(model, _Comparative) and model.use_wt_for_downstream
     with torch.no_grad():
-        base_item = _encode(model, graph_data, sequence_data, peptide_property)
-        e = _draws(model, eps, samples, graph_data.n_graphs, base_item[1])
-        base_item += (e,)
-        base = Predictive(*IF._C.head_mc_infer([base_item, base_item] if pair else [base_item], *_head_params(model)))
-        out = _search(model, graph_data, sequence_data, peptide_property, ni, si, cols, allowed, max_mut, beam, rounds,
-                      maximize, kappa, e, base, lambda item, r: [item, item] if pair else [item], max_graphs)
-    return Design(*out, base)
+        scorer = _scorer(model, graph_data, sequence_data, peptide_property, eps, samples)
+        out = _search(model, scorer, graph_data, sequence_data, peptide_property, ni, si, cols, allowed, max_mut, beam,
+                      rounds, maximize, kappa, max_graphs)
+    return Design(*out, scorer.base)
 
 
 def beam_search_pair(model, graph_pair, sequence_pair, property_pair, node_index: Tensor, seq_index: Tensor, *,
@@ -190,28 +179,12 @@ def beam_search_pair(model, graph_pair, sequence_pair, property_pair, node_index
     eps_w), each [K, B, latent], or one ``model.sample_eps`` call of [K*B, latent] per item, cancer first.  Without
     ``use_wt_for_downstream`` the wild type is neither run nor drawn for.  ``base`` equals ``predictive_pair`` on the same
     draws."""
-    _check_scan(model, samples, _Comparative, "beam_search_pair", _PAIR_CLASSES)
-    n = _pair_items(model, eps)
+    _check(model, samples, _Comparative, "beam_search_pair", _PAIR_CLASSES)
     gc = graph_pair[0]
     ni, si, cols, allowed, max_mut, rounds, kappa = _prepare(gc, sequence_pair[0], node_index, seq_index, seq_columns,
                                                              allowed, max_mutations, beam, rounds, kappa, max_graphs)
     with torch.no_grad():
-        items = []
-        for i in range(n):
-            item = _encode(model, graph_pair[i], sequence_pair[i], property_pair[i])
-            k = samples if eps is None else eps[0].shape[0]
-            items.append(item + (_draws(model, None if eps is None else eps[i], k, item[1].shape[0], item[1]),))
-        base = Predictive(*IF._C.head_mc_infer(items, *_head_params(model)))
-        wt = items[1] if n == 2 else None
-        wt_r = {}
-
-        def items_of(item, r):
-            if wt is None:
-                return [item]
-            if r not in wt_r:
-                wt_r[r] = tuple(t.repeat(1, r, 1) if t.dim() == 3 else t.repeat(r, 1) for t in wt)
-            return [item, wt_r[r]]
-
-        out = _search(model, gc, sequence_pair[0], property_pair[0], ni, si, cols, allowed, max_mut, beam, rounds,
-                      maximize, kappa, items[0][4], base, items_of, max_graphs)
-    return Design(*out, base)
+        scorer = _scorer_pair(model, graph_pair, sequence_pair, property_pair, eps, samples)
+        out = _search(model, scorer, gc, sequence_pair[0], property_pair[0], ni, si, cols, allowed, max_mut, beam, rounds,
+                      maximize, kappa, max_graphs)
+    return Design(*out, scorer.base)

@@ -9,9 +9,10 @@ rejects a site row that is not exactly one-hot (a padded or masked row) or that 
 
 The P x 20 variants of the batch run in passes of r = min(remaining, max_graphs // B) copies of the whole batch: one
 kernel writes a pass's mutant features from the resident batch (``is_mutscan_expand``, csrc/mutscan.cu), the copies'
-topology is collated once per distinct r, the trunk and the VAE encoder run once per pass and the multi-draw head
-(``is_head_mc_infer``) scores every draw.  The reparameterisation noise is common to all variants of a sample (common
-random numbers), so the difference between two variants is the effect of the substitution alone.
+topology is collated once per distinct r before the first pass (``resident``'s replica passes), the trunk and the VAE
+encoder run once per pass and the multi-draw head (``is_head_mc_infer``) scores every draw.  The reparameterisation
+noise is common to all variants of a sample (common random numbers), so the difference between two variants is the
+effect of the substitution alone.
 
 An entry agrees with the fused eval forward of the B-sample mutant batch on the same draw to rounding, not bit for bit:
 where a graph sits in the batch changes two summation orders, the edge kernel's per-tile segment-sum MMA (a node's
@@ -20,8 +21,8 @@ in-edges land at other positions of a 128-edge tile) and the K-slice count of th
 ``score_variants`` scores a caller's library instead: each variant is one sample of the batch with any list of
 substitutions (neoantigen candidates, anchor-modified designs, threaded peptides or HLA alleles).  A pass is a run of up to
 ``max_graphs`` variants in the caller's order; ``is_variant_expand`` gathers their graphs, edges and sequences from the
-resident batch and applies the substitutions, the gathered topology is collated once per pass, and the trunk and the
-multi-draw head run as for the scan, each variant on the draws of its base sample.
+resident batch and applies the substitutions, the gathered topology is collated once per pass (``resident``'s gathered
+passes), and the trunk and the multi-draw head run as for the scan, each variant on the draws of its base sample.
 """
 from __future__ import annotations
 
@@ -32,12 +33,12 @@ import torch
 
 from . import functional as IF
 from .comparative_models import _Comparative
-from .graph import GraphBatch
 from .hybrid_models import _Hybrid
-from .predictive import _CLASSES, _PAIR_CLASSES, Predictive, _check, _draws, _encode, _head_params, _pair_items
+from .predictive import _CLASSES, _PAIR_CLASSES, Predictive, _check, _encode, _scorer, _scorer_pair
+from .resident import (N_RESIDUES, check_one_hot, native_residues, pass_totals, replicas, scan_passes, score_gathered,
+                       score_replicas, sequence_replica, variant_passes)
 
 Tensor = torch.Tensor
-N_RESIDUES = 20
 
 
 @dataclass
@@ -48,14 +49,6 @@ class Scan:
     prob_std: Tensor      # [B, P, 20]     population standard deviation of sigmoid(logit) over the draws
     native: Tensor        # [B, P]         residue column of the input at the site, -1 = absent site
     base: Predictive      # the unmutated batch on the same draws
-
-
-def scan_passes(n_copies: int, b: int, max_graphs: int):
-    """(first copy, number of copies) of each pass: r = min(remaining, max_graphs // B) copies of the B-graph batch."""
-    if b > max_graphs:
-        raise ValueError(f"the batch has {b} graphs, more than max_graphs={max_graphs}")
-    per = max_graphs // b
-    return [(j, min(per, n_copies - j)) for j in range(0, n_copies, per)]
 
 
 def scan_sites(n_sites: int, device=None) -> Tensor:
@@ -109,50 +102,30 @@ def _site_tables(graph, seq, node_index, seq_index, seq_columns):
     return ni.contiguous(), si.contiguous(), cols.contiguous()
 
 
-def _check_scan(model, samples, kinds, what, names):
-    _check(model, samples, kinds, what, names)
-    if model.training:
-        raise RuntimeError(f"{what} needs model.eval(): dropout would change the function between variants")
-
-
-def _run(model, graph, seq, prop, ni, si, cols, e, items_of, max_graphs):
-    """Every variant of ``graph`` in passes -> (logits [B,P,20,K], prob_mean, prob_std, native).  ``items_of(item, r)``
-    turns the mutant item of an r-copy pass into the head's item list."""
-    params = _head_params(model)
+def _scan(model, scorer, graph, seq, prop, ni, si, cols, max_graphs):
+    """Every variant of ``graph`` in replica passes -> (logits [B,P,20,K], prob_mean, prob_std, native)."""
     b, n_sites = ni.shape
     x = graph.ndata["x"].detach().contiguous()
     seq = seq.detach().contiguous()
-    prop = prop.detach().contiguous()
-    L, V, k = seq.shape[1], seq.shape[2], e.shape[0]
     sites = scan_sites(n_sites, x.device)
-    n_copies = sites.shape[0]
-    logits = torch.empty(n_copies, b, k, dtype=torch.float32, device=x.device)
-    mean = torch.empty(n_copies, b, dtype=torch.float32, device=x.device)
-    std = torch.empty_like(mean)
+    passes = scan_passes(sites.shape[0], b, max_graphs)
     flag = torch.zeros(1, dtype=torch.int32, device=x.device)
-    passes = {}
-    for j, r in scan_passes(n_copies, b, max_graphs):
-        if r not in passes:                     # topology of r copies, collated once; only the features change per pass
-            passes[r] = (graph.replicate(r), torch.empty(r * b, L, V, dtype=torch.float32, device=x.device),
-                         prop.repeat(r, 1))
-        g, seq_r, prop_r = passes[r]
+
+    def run_pass(j, r, g, seq_r, prop_r, e_r):
         IF._C.mutscan_expand(x, graph.node_off, ni, seq, si, cols, sites[j:j + r], g.ndata["x"], seq_r, flag)
-        item = _encode(model, g, seq_r, prop_r) + (e.repeat(1, r, 1),)
-        lg, m, s = IF._C.head_mc_infer(items_of(item, r), *params)
-        logits[j:j + r], mean[j:j + r], std[j:j + r] = lg.reshape(r, b, k), m.reshape(r, b), s.reshape(r, b)
-    if flag.item():
-        raise ValueError("a site row is not exactly one-hot in the graph's residue columns or in the sequence, or its "
-                         "sequence column is not seq_columns[residue column] (a padded or masked row, or a wrong map)")
+        return scorer.score(_encode(model, g, seq_r, prop_r) + (e_r,), r=r)
+
+    reps = replicas(passes, sequence_replica(graph, seq, prop, scorer.item[4]))
+    logits, mean, std = score_replicas(scorer, passes, reps, run_pass)
+    check_one_hot(flag, "a site row")
     absent = ni < 0
     shape = (n_sites, N_RESIDUES, b)
-    logits = logits.reshape(*shape, k).permute(2, 0, 1, 3).contiguous()
+    logits = logits.reshape(*shape, logits.shape[2]).permute(2, 0, 1, 3).contiguous()
     mean = mean.reshape(shape).permute(2, 0, 1).contiguous()
     std = std.reshape(shape).permute(2, 0, 1).contiguous()
     for t in (logits, mean, std):
         t[absent] = float("nan")
-    rows = graph.node_off[:-1].unsqueeze(1) + ni.clamp_min(0)
-    native = torch.where(absent, -1, x[rows.reshape(-1), :N_RESIDUES].argmax(1).reshape(b, n_sites))
-    return logits, mean, std, native
+    return logits, mean, std, native_residues(graph, ni)
 
 
 def mutational_scan(model, graph_data, sequence_data, peptide_property, node_index: Tensor, seq_index: Tensor, *,
@@ -167,18 +140,13 @@ def mutational_scan(model, graph_data, sequence_data, peptide_property, node_ind
     ``max_graphs`` graphs.  Follows ``model.forward`` for the eight classes ``predictive`` supports; the model must be in
     eval mode; no_grad, and every ``.grad`` is left untouched.  The native residue's column is scored like any other and
     equals ``base`` up to rounding."""
-    _check_scan(model, samples, (_Hybrid, _Comparative), "mutational_scan", _CLASSES)
+    _check(model, samples, (_Hybrid, _Comparative), "mutational_scan", _CLASSES)
     ni, si, cols = _site_tables(graph_data, sequence_data, node_index, seq_index, seq_columns)
     scan_passes(1, graph_data.n_graphs, max_graphs)
-    pair = isinstance(model, _Comparative) and model.use_wt_for_downstream
     with torch.no_grad():
-        base_item = _encode(model, graph_data, sequence_data, peptide_property)
-        e = _draws(model, eps, samples, graph_data.n_graphs, base_item[1])
-        base_item += (e,)
-        base = Predictive(*IF._C.head_mc_infer([base_item, base_item] if pair else [base_item], *_head_params(model)))
-        out = _run(model, graph_data, sequence_data, peptide_property, ni, si, cols, e,
-                   lambda item, r: [item, item] if pair else [item], max_graphs)
-    return Scan(*out, base)
+        scorer = _scorer(model, graph_data, sequence_data, peptide_property, eps, samples)
+        out = _scan(model, scorer, graph_data, sequence_data, peptide_property, ni, si, cols, max_graphs)
+    return Scan(*out, scorer.base)
 
 
 def mutational_scan_pair(model, graph_pair, sequence_pair, property_pair, node_index: Tensor, seq_index: Tensor, *,
@@ -190,27 +158,14 @@ def mutational_scan_pair(model, graph_pair, sequence_pair, property_pair, node_i
     eps_w), each [K, B, latent], or one ``model.sample_eps`` call of [K*B, latent] per item, cancer first.  Without
     ``use_wt_for_downstream`` the wild type is neither run nor drawn for.  ``base`` equals ``predictive_pair`` on the same
     draws."""
-    _check_scan(model, samples, _Comparative, "mutational_scan_pair", _PAIR_CLASSES)
-    n = _pair_items(model, eps)
+    _check(model, samples, _Comparative, "mutational_scan_pair", _PAIR_CLASSES)
     gc = graph_pair[0]
     ni, si, cols = _site_tables(gc, sequence_pair[0], node_index, seq_index, seq_columns)
     scan_passes(1, gc.n_graphs, max_graphs)
     with torch.no_grad():
-        items = []
-        for i in range(n):
-            item = _encode(model, graph_pair[i], sequence_pair[i], property_pair[i])
-            k = samples if eps is None else eps[0].shape[0]
-            items.append(item + (_draws(model, None if eps is None else eps[i], k, item[1].shape[0], item[1]),))
-        base = Predictive(*IF._C.head_mc_infer(items, *_head_params(model)))
-        wt = items[1] if n == 2 else None
-
-        def items_of(item, r):
-            if wt is None:
-                return [item]
-            return [item, tuple(t.repeat(1, r, 1) if t.dim() == 3 else t.repeat(r, 1) for t in wt)]
-
-        out = _run(model, gc, sequence_pair[0], property_pair[0], ni, si, cols, items[0][4], items_of, max_graphs)
-    return Scan(*out, base)
+        scorer = _scorer_pair(model, graph_pair, sequence_pair, property_pair, eps, samples)
+        out = _scan(model, scorer, gc, sequence_pair[0], property_pair[0], ni, si, cols, max_graphs)
+    return Scan(*out, scorer.base)
 
 
 # ---- variant libraries: any substitution list on any sample -----------------------------------------------------------
@@ -223,17 +178,10 @@ class VariantScores:
     base: Predictive      # the unmutated batch on the same draws
 
 
-def variant_passes(n_variants: int, max_graphs: int):
-    """(first variant, number of variants) of each pass: consecutive runs of at most ``max_graphs`` variants."""
-    if max_graphs < 1:
-        raise ValueError(f"max_graphs must be >= 1, got {max_graphs}")
-    return [(j, min(max_graphs, n_variants - j)) for j in range(0, n_variants, max_graphs)]
-
-
 def _variant_tables(graph, seq, sample, offsets, node_index, seq_index, residue, seq_columns, max_graphs):
     """The checked library on the batch's device: (sample, offsets, node_index, seq_index, residue, seq_columns, node and
-    edge count of each variant, their running sums [V+1], every pass's node and edge totals).  One host read for all
-    checks and totals."""
+    edge count of each variant, their running sums [V+1], the passes, every pass's node and edge totals).  One host read
+    for all checks and totals."""
     b = graph.n_graphs
     for name, t in (("sample", sample), ("offsets", offsets), ("node_index", node_index), ("seq_index", seq_index),
                     ("residue", residue)):
@@ -255,20 +203,17 @@ def _variant_tables(graph, seq, sample, offsets, node_index, seq_index, residue,
     L, V = seq.shape[1], seq.shape[2]
     sb = smp.clamp(0, b - 1)
     nv, ev = graph.batch_num_nodes().to(dev)[sb].contiguous(), graph.batch_num_edges().to(dev)[sb].contiguous()
-    zero = torch.zeros(1, dtype=torch.int64, device=dev)
-    ncs, ecs = torch.cat([zero, nv.cumsum(0)]), torch.cat([zero, ev.cumsum(0)])
+    ncs, ecs, node_tot, edge_tot = pass_totals(nv, ev, n_var, len(passes), max_graphs)
     owner = (torch.searchsorted(off, torch.arange(n_sub, device=dev), right=True) - 1).clamp(0, n_var - 1)
     last = torch.arange(n_sub, device=dev)
     twice = lambda key: (key.sort().values.diff() == 0).any()
     node_key = torch.where(ni >= 0, owner * (int(graph.max_nodes) + 1) + ni, -1 - last)
     seq_key = owner * L + si
-    first = torch.tensor([j for j, _ in passes], device=dev)
-    end = torch.tensor([j + r for j, r in passes], device=dev)
     bad = torch.stack([((smp < 0) | (smp >= b)).any(), (off[0] != 0) | (off.diff() < 0).any() | (off[-1] != n_sub),
                        ((ni < -1) | (ni >= nv[owner])).any(), ((si < 0) | (si >= L)).any(),
                        ((res < 0) | (res >= N_RESIDUES)).any(), _columns_bad(cols, V), twice(node_key),
                        twice(seq_key)]).long()
-    vals = torch.cat([bad, ncs[end] - ncs[first], ecs[end] - ecs[first]]).tolist()
+    vals = torch.cat([bad, node_tot, edge_tot]).tolist()
     if vals[0]:
         raise ValueError(f"sample must index the batch: every entry in [0, B={b})")
     if vals[1]:
@@ -286,42 +231,26 @@ def _variant_tables(graph, seq, sample, offsets, node_index, seq_index, residue,
     if vals[7]:
         raise ValueError("a variant substitutes the same sequence row twice")
     n_pass = len(passes)
-    return (smp, off, ni, si, res, cols, nv, ev, ncs, ecs, vals[8:8 + n_pass], vals[8 + n_pass:])
+    return (smp, off, ni, si, res, cols, nv, ev, ncs, ecs, passes, vals[8:8 + n_pass], vals[8 + n_pass:])
 
 
-def _run_variants(model, graph, seq, prop, tables, e, items_of, max_graphs):
-    """Every variant of the library in passes -> (logits [V,K], prob_mean [V], prob_std [V]).  ``items_of(item, s)`` turns
-    the mutant item of a pass whose variants have base samples ``s`` into the head's item list."""
-    smp, off, ni, si, res, cols, nv, ev, ncs, ecs, node_totals, edge_totals = tables
-    params = _head_params(model)
-    x = graph.ndata["x"].detach().contiguous()
-    ea = graph.edata["edge_attr"].detach().contiguous()
-    src, dst = graph._src_local.contiguous(), graph._dst_local.contiguous()
+def _score_variants(model, scorer, graph, seq, prop, tables):
+    """Every variant of the library in gathered passes -> (logits [V,K], prob_mean [V], prob_std [V])."""
+    smp, off, ni, si, res, cols, nv, ev, ncs, ecs, passes, node_totals, edge_totals = tables
     seq = seq.detach().contiguous()
     prop = prop.detach().contiguous()
-    L, V, k = seq.shape[1], seq.shape[2], e.shape[0]
-    n_var = smp.shape[0]
-    f32 = dict(dtype=torch.float32, device=x.device)
-    logits, mean, std = torch.empty(n_var, k, **f32), torch.empty(n_var, **f32), torch.empty(n_var, **f32)
-    flag = torch.zeros(1, dtype=torch.int32, device=x.device)
-    for (j, r), n_p, e_p in zip(variant_passes(n_var, max_graphs), node_totals, edge_totals):
-        sp = smp[j:j + r]
-        x_p = torch.empty(n_p, 23, **f32)
-        src_p, dst_p = torch.empty(e_p, dtype=torch.int64, device=x.device), torch.empty(e_p, dtype=torch.int64, device=x.device)
-        ea_p = torch.empty(e_p, *ea.shape[1:], **f32)
-        seq_p = torch.empty(r, L, V, **f32)
-        IF._C.variant_expand(x, graph.node_off, graph.edge_off, src, dst, ea, seq, sp, off[j:j + r + 1], ni, si, res, cols,
-                             ncs[j:j + r + 1] - ncs[j], ecs[j:j + r + 1] - ecs[j], x_p, src_p, dst_p, ea_p, seq_p, flag)
-        # the pass's topology is gathered, not a replica of the batch: collated per pass
-        g = GraphBatch(x_p, src_p, dst_p, ea_p, nv[j:j + r], ev[j:j + r], max_nodes=graph.max_nodes, collate_now=False)
-        g._collate()
-        item = _encode(model, g, seq_p, prop[sp]) + (e[:, sp],)
-        lg, m, s = IF._C.head_mc_infer(items_of(item, sp), *params)
-        logits[j:j + r], mean[j:j + r], std[j:j + r] = lg, m, s
-    if flag.item():
-        raise ValueError("a substituted row is not exactly one-hot in the graph's residue columns or in the sequence, or "
-                         "its sequence column is not seq_columns[residue column] (a padded or masked row, or a wrong map)")
-    return logits, mean, std
+    e = scorer.item[4]
+    flag = torch.zeros(1, dtype=torch.int32, device=smp.device)
+
+    def expand(j, r, inputs, outputs):
+        seq_p = torch.empty(r, *seq.shape[1:], dtype=torch.float32, device=smp.device)
+        IF._C.variant_expand(*inputs, seq, smp[j:j + r], off[j:j + r + 1], ni, si, res, cols, *outputs, seq_p, flag)
+        return seq_p
+
+    out = score_gathered(scorer, graph, smp, nv, ev, ncs, ecs, passes, node_totals, edge_totals, expand,
+                         lambda g, sp, seq_p: _encode(model, g, seq_p, prop[sp]) + (e[:, sp],))
+    check_one_hot(flag, "a substituted row")
+    return out
 
 
 def score_variants(model, graph_data, sequence_data, peptide_property, sample: Tensor, offsets: Tensor,
@@ -341,18 +270,13 @@ def score_variants(model, graph_data, sequence_data, peptide_property, sample: T
     them; variant v uses the draws of sample ``sample[v]``, so variants of one sample differ by their substitutions only.
     The variants run in passes of at most ``max_graphs``, in the caller's order.  Classes, eval mode, no_grad and
     ``.grad`` as in ``mutational_scan``."""
-    _check_scan(model, samples, (_Hybrid, _Comparative), "score_variants", _CLASSES)
+    _check(model, samples, (_Hybrid, _Comparative), "score_variants", _CLASSES)
     tables = _variant_tables(graph_data, sequence_data, sample, offsets, node_index, seq_index, residue, seq_columns,
                              max_graphs)
-    pair = isinstance(model, _Comparative) and model.use_wt_for_downstream
     with torch.no_grad():
-        base_item = _encode(model, graph_data, sequence_data, peptide_property)
-        e = _draws(model, eps, samples, graph_data.n_graphs, base_item[1])
-        base_item += (e,)
-        base = Predictive(*IF._C.head_mc_infer([base_item, base_item] if pair else [base_item], *_head_params(model)))
-        out = _run_variants(model, graph_data, sequence_data, peptide_property, tables, e,
-                            lambda item, sp: [item, item] if pair else [item], max_graphs)
-    return VariantScores(*out, base)
+        scorer = _scorer(model, graph_data, sequence_data, peptide_property, eps, samples)
+        out = _score_variants(model, scorer, graph_data, sequence_data, peptide_property, tables)
+    return VariantScores(*out, scorer.base)
 
 
 def score_variants_pair(model, graph_pair, sequence_pair, property_pair, sample: Tensor, offsets: Tensor,
@@ -365,23 +289,10 @@ def score_variants_pair(model, graph_pair, sequence_pair, property_pair, sample:
     ``eps`` = (eps_c, eps_w), each [K, B, latent], or one ``model.sample_eps`` call of [K*B, latent] per item, cancer
     first.  Without ``use_wt_for_downstream`` the wild type is neither run nor drawn for.  ``base`` equals
     ``predictive_pair`` on the same draws."""
-    _check_scan(model, samples, _Comparative, "score_variants_pair", _PAIR_CLASSES)
-    n = _pair_items(model, eps)
+    _check(model, samples, _Comparative, "score_variants_pair", _PAIR_CLASSES)
     gc = graph_pair[0]
     tables = _variant_tables(gc, sequence_pair[0], sample, offsets, node_index, seq_index, residue, seq_columns, max_graphs)
     with torch.no_grad():
-        items = []
-        for i in range(n):
-            item = _encode(model, graph_pair[i], sequence_pair[i], property_pair[i])
-            k = samples if eps is None else eps[0].shape[0]
-            items.append(item + (_draws(model, None if eps is None else eps[i], k, item[1].shape[0], item[1]),))
-        base = Predictive(*IF._C.head_mc_infer(items, *_head_params(model)))
-        wt = items[1] if n == 2 else None
-
-        def items_of(item, sp):
-            if wt is None:
-                return [item]
-            return [item, tuple(t[:, sp] if t.dim() == 3 else t[sp] for t in wt)]
-
-        out = _run_variants(model, gc, sequence_pair[0], property_pair[0], tables, items[0][4], items_of, max_graphs)
-    return VariantScores(*out, base)
+        scorer = _scorer_pair(model, graph_pair, sequence_pair, property_pair, eps, samples)
+        out = _score_variants(model, scorer, gc, sequence_pair[0], property_pair[0], tables)
+    return VariantScores(*out, scorer.base)

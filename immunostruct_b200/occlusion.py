@@ -34,10 +34,9 @@ import torch
 
 from . import functional as IF
 from .comparative_models import _Comparative
-from .graph import GraphBatch
 from .hybrid_models import _Hybrid
-from .mutagenesis import _check_scan, variant_passes
-from .predictive import _CLASSES, _PAIR_CLASSES, Predictive, _draws, _encode, _head_params, _pair_items
+from .predictive import _CLASSES, _PAIR_CLASSES, Predictive, _check, _scorer, _scorer_pair
+from .resident import pass_totals, score_gathered, variant_passes
 
 Tensor = torch.Tensor
 
@@ -89,24 +88,11 @@ def _first_selected(keep):
     return torch.sort((~keep).to(torch.int32), stable=True).indices
 
 
-def _pass_totals(n_var, ncs, ecs, n_slots, max_graphs):
-    """Node and edge totals of every possible pass (the first n_slots runs of max_graphs variants), from the running sums
-    ``ncs`` / ``ecs`` and the device count ``n_var``; runs past n_var total 0."""
-    dev = ncs.device
-    first = torch.arange(n_slots, device=dev) * max_graphs
-    end = torch.minimum(first + max_graphs, n_var)
-    first = torch.minimum(first, n_var)
-    return ncs[end] - ncs[first], ecs[end] - ecs[first]
-
-
 def _finish_tables(graph, smp, na, nb, kept, n_var, n_slots, max_graphs, what):
     """Running sums and the one host read -> (sample, node_a, node_b, node count, kept edges, node offsets, edge offsets,
     passes, pass node totals, pass edge totals, C), trimmed to the C variants."""
-    dev = smp.device
-    nv = graph.batch_num_nodes().to(dev)[smp]
-    zero = torch.zeros(1, dtype=torch.int64, device=dev)
-    ncs, ecs = torch.cat([zero, nv.cumsum(0)]), torch.cat([zero, kept.cumsum(0)])
-    node_tot, edge_tot = _pass_totals(n_var, ncs, ecs, n_slots, max_graphs)
+    nv = graph.batch_num_nodes().to(smp.device)[smp]
+    ncs, ecs, node_tot, edge_tot = pass_totals(nv, kept, n_var, n_slots, max_graphs)
     vals = torch.cat([n_var.reshape(1), node_tot, edge_tot]).tolist()
     c = vals[0]
     if c == 0:
@@ -161,69 +147,23 @@ def _contact_tables(graph, nodes, max_graphs):
     return tables, edge_contact
 
 
-def _run(model, graph, tables, enc, e, items_of):
-    """Every variant in passes -> (logits [C,K], prob_mean [C], prob_std [C]).  ``enc`` = (mu, logvar, z_vae) of the base
-    batch; ``items_of(item, sp)`` turns the occluded item of a pass whose variants have base samples ``sp`` into the
-    head's item list."""
-    smp, na, nb, nv, kept, ncs, ecs, passes, node_totals, edge_totals, n_var = tables
-    mu, logvar, z_vae = enc
-    params = _head_params(model)
-    x = graph.ndata["x"].detach().contiguous()
-    ea = graph.edata["edge_attr"].detach().contiguous()
-    src, dst = graph._src_local.contiguous(), graph._dst_local.contiguous()
-    k = e.shape[0]
-    f32 = dict(dtype=torch.float32, device=x.device)
-    i64 = dict(dtype=torch.int64, device=x.device)
-    logits, mean, std = torch.empty(n_var, k, **f32), torch.empty(n_var, **f32), torch.empty(n_var, **f32)
-    flag = torch.zeros(1, dtype=torch.int32, device=x.device)
-    for (j, r), n_p, e_p in zip(passes, node_totals, edge_totals):
-        sp = smp[j:j + r]
-        x_p = torch.empty(n_p, 23, **f32)
-        src_p, dst_p = torch.empty(e_p, **i64), torch.empty(e_p, **i64)
-        ea_p = torch.empty(e_p, *ea.shape[1:], **f32)
-        IF._C.occlusion_expand(x, graph.node_off, graph.edge_off, src, dst, ea, sp, na[j:j + r], nb[j:j + r],
-                               ncs[j:j + r + 1] - ncs[j], ecs[j:j + r + 1] - ecs[j], x_p, src_p, dst_p, ea_p, flag)
-        # the pass's topology differs from the batch's: collated per pass
-        g = GraphBatch(x_p, src_p, dst_p, ea_p, nv[j:j + r], kept[j:j + r], max_nodes=graph.max_nodes, collate_now=False)
-        g._collate()
-        pooled = model.structure_embedding(g, project=False)[0].contiguous()
-        item = (pooled, mu[sp], logvar[sp], z_vae[sp], e[:, sp])
-        logits[j:j + r], mean[j:j + r], std[j:j + r] = IF._C.head_mc_infer(items_of(item, sp), *params)
+def _occlude(model, scorer, graph, tables):
+    """Every variant in gathered passes -> (logits [C,K], prob_mean [C], prob_std [C]).  The sequence branch is not
+    touched: a pass gathers the base's encoded tensors and draws by sample instead of re-encoding."""
+    smp, na, nb, nv, kept, ncs, ecs, passes, node_totals, edge_totals, _ = tables
+    mu, logvar, z_vae, e = scorer.item[1:]
+    flag = torch.zeros(1, dtype=torch.int32, device=smp.device)
+
+    def expand(j, r, inputs, outputs):
+        IF._C.occlusion_expand(*inputs, smp[j:j + r], na[j:j + r], nb[j:j + r], *outputs, flag)
+
+    def pass_item(g, sp, _):
+        return model.structure_embedding(g, project=False)[0].contiguous(), mu[sp], logvar[sp], z_vae[sp], e[:, sp]
+
+    out = score_gathered(scorer, graph, smp, nv, kept, ncs, ecs, passes, node_totals, edge_totals, expand, pass_item)
     if flag.item():
         raise RuntimeError("is_occlusion_expand rejected a variant: its indices or offsets disagree with the batch")
-    return logits, mean, std
-
-
-def _single(model, graph, seq, prop, tables, eps, samples):
-    """Base and passes of the single-item forms -> (base, (logits, prob_mean, prob_std))."""
-    pair = isinstance(model, _Comparative) and model.use_wt_for_downstream
-    with torch.no_grad():
-        e = _draws(model, eps, samples, graph.n_graphs, graph.ndata["x"])
-        pooled, mu, logvar, z_vae = _encode(model, graph, seq, prop)
-        item = (pooled, mu, logvar, z_vae, e)
-        base = Predictive(*IF._C.head_mc_infer([item, item] if pair else [item], *_head_params(model)))
-        out = _run(model, graph, tables, (mu, logvar, z_vae), e, lambda it, sp: [it, it] if pair else [it])
-    return base, out
-
-
-def _pair(model, graph_pair, sequence_pair, property_pair, tables, eps, samples, n):
-    """Base and passes of the pair forms: the cancer item occluded against the fixed wild type, encoded once at batch B
-    and gathered by sample per pass (never run or drawn for without use_wt_for_downstream)."""
-    with torch.no_grad():
-        k = samples if eps is None else eps[0].shape[0]
-        draws = [_draws(model, None if eps is None else eps[i], k, graph_pair[i].n_graphs, graph_pair[i].ndata["x"])
-                 for i in range(n)]
-        items = [_encode(model, graph_pair[i], sequence_pair[i], property_pair[i]) + (draws[i],) for i in range(n)]
-        base = Predictive(*IF._C.head_mc_infer(items, *_head_params(model)))
-        wt = items[1] if n == 2 else None
-
-        def items_of(item, sp):
-            if wt is None:
-                return [item]
-            return [item, tuple(t[:, sp] if t.dim() == 3 else t[sp] for t in wt)]
-
-        out = _run(model, graph_pair[0], tables, items[0][1:4], items[0][4], items_of)
-    return base, out
+    return out
 
 
 def _residue_result(graph, rows, out, base):
@@ -248,10 +188,11 @@ def occlude_residues(model, graph, seq, prop, *, nodes: Optional[Tensor] = None,
     variant uses the draws of its sample.  Variants run in row order, in passes of at most ``max_graphs``.  Follows
     ``model.forward`` for the eight classes ``predictive`` supports; the model must be in eval mode; no_grad, and every
     ``.grad`` is left untouched.  The result is aligned with the rows; rows not scanned are NaN."""
-    _check_scan(model, samples, (_Hybrid, _Comparative), "occlude_residues", _CLASSES)
+    _check(model, samples, (_Hybrid, _Comparative), "occlude_residues", _CLASSES)
     tables, rows = _residue_tables(graph, nodes, max_graphs)
-    base, out = _single(model, graph, seq, prop, tables, eps, samples)
-    return _residue_result(graph, rows, out, base)
+    with torch.no_grad():
+        scorer = _scorer(model, graph, seq, prop, eps, samples)
+        return _residue_result(graph, rows, _occlude(model, scorer, graph, tables), scorer.base)
 
 
 def occlude_contacts(model, graph, seq, prop, *, nodes: Optional[Tensor] = None, eps: Optional[Tensor] = None,
@@ -263,10 +204,11 @@ def occlude_contacts(model, graph, seq, prop, *, nodes: Optional[Tensor] = None,
     contacts with at least one selected endpoint (e.g. the peptide rows: the peptide-HLA interface and the peptide's own
     contacts), by default every contact.  Entries are ordered by (sample, u, v); ``edge_contact`` maps each edge of the
     batch to its contact.  Draws, passes, classes, eval mode, no_grad and ``.grad`` as in ``occlude_residues``."""
-    _check_scan(model, samples, (_Hybrid, _Comparative), "occlude_contacts", _CLASSES)
+    _check(model, samples, (_Hybrid, _Comparative), "occlude_contacts", _CLASSES)
     tables, edge_contact = _contact_tables(graph, nodes, max_graphs)
-    base, out = _single(model, graph, seq, prop, tables, eps, samples)
-    return _contact_result(tables, edge_contact, out, base)
+    with torch.no_grad():
+        scorer = _scorer(model, graph, seq, prop, eps, samples)
+        return _contact_result(tables, edge_contact, _occlude(model, scorer, graph, tables), scorer.base)
 
 
 def occlude_residues_pair(model, graph_pair, seq_pair, prop_pair, *, nodes: Optional[Tensor] = None, eps=None,
@@ -278,19 +220,19 @@ def occlude_residues_pair(model, graph_pair, seq_pair, prop_pair, *, nodes: Opti
     (eps_c, eps_w), each [K, B, latent], or one ``model.sample_eps`` call of [K*B, latent] per item, cancer first.
     Without ``use_wt_for_downstream`` the wild type is neither run nor drawn for.  ``base`` equals ``predictive_pair`` on
     the same draws."""
-    _check_scan(model, samples, _Comparative, "occlude_residues_pair", _PAIR_CLASSES)
-    n = _pair_items(model, eps)
+    _check(model, samples, _Comparative, "occlude_residues_pair", _PAIR_CLASSES)
     tables, rows = _residue_tables(graph_pair[0], nodes, max_graphs)
-    base, out = _pair(model, graph_pair, seq_pair, prop_pair, tables, eps, samples, n)
-    return _residue_result(graph_pair[0], rows, out, base)
+    with torch.no_grad():
+        scorer = _scorer_pair(model, graph_pair, seq_pair, prop_pair, eps, samples)
+        return _residue_result(graph_pair[0], rows, _occlude(model, scorer, graph_pair[0], tables), scorer.base)
 
 
 def occlude_contacts_pair(model, graph_pair, seq_pair, prop_pair, *, nodes: Optional[Tensor] = None, eps=None,
                           samples: int = 1, max_graphs: int = 4096) -> ContactOcclusion:
     """``occlude_contacts`` of the cancer item of ``model.forward_comparative`` against its fixed wild type; the wild
     type as in ``occlude_residues_pair``."""
-    _check_scan(model, samples, _Comparative, "occlude_contacts_pair", _PAIR_CLASSES)
-    n = _pair_items(model, eps)
+    _check(model, samples, _Comparative, "occlude_contacts_pair", _PAIR_CLASSES)
     tables, edge_contact = _contact_tables(graph_pair[0], nodes, max_graphs)
-    base, out = _pair(model, graph_pair, seq_pair, prop_pair, tables, eps, samples, n)
-    return _contact_result(tables, edge_contact, out, base)
+    with torch.no_grad():
+        scorer = _scorer_pair(model, graph_pair, seq_pair, prop_pair, eps, samples)
+        return _contact_result(tables, edge_contact, _occlude(model, scorer, graph_pair[0], tables), scorer.base)

@@ -12,7 +12,7 @@ output of the shared ``vae_mid_infer`` kernel is discarded).
 """
 from __future__ import annotations
 
-from dataclasses import dataclass
+from dataclasses import dataclass, field
 from typing import Optional
 
 import torch
@@ -39,8 +39,6 @@ class Predictive:
 
 def _head_params(model):
     """Weights of the fused head, after checking that the model has one: (Wc, bc, coef, n_head, W1, b1, W2, b2)."""
-    if model.training:
-        raise RuntimeError("predictive needs model.eval(): dropout would change the function between draws")
     if model.gat_hidden_channels != 64 or model.mlp_features != 32:
         raise NotImplementedError("the fused head needs gat_hidden_channels = 64 and mlp_features = 32")
     fus = model.combined_attention if model._fusion_dim else None
@@ -82,6 +80,8 @@ def _check(model, samples, kinds, what, names):
         raise NotImplementedError(f"{what} supports {names}; {type(model).__name__} is not one of them")
     if samples < 1:
         raise ValueError("samples must be >= 1")
+    if model.training:
+        raise RuntimeError(f"{what} needs model.eval(): dropout would change the function between draws and variants")
 
 
 def _pair_items(model, eps):
@@ -94,6 +94,65 @@ def _pair_items(model, eps):
     if eps is not None and n == 2 and eps[0].shape[:1] != eps[1].shape[:1]:
         raise ValueError("eps_c and eps_w must hold the same number of draws")
     return n
+
+
+def _repeat(t, r):
+    """A tensor of an item or of the batch, [B, ...] or draws-first [K, B, latent], repeated for r copies of the batch."""
+    return t.repeat(1, r, 1) if t.dim() == 3 else t.repeat(r, 1)
+
+
+@dataclass
+class _Scorer:
+    """The base of a batch on the device and the head that scores its variants.  ``item`` = (pooled, mu, logvar, z_vae,
+    eps) of the scored item at batch B; ``wt`` the fixed wild-type item at batch B, or None; ``repeat``: the single form
+    of a pair-wide head, which reads its one item twice; ``params`` the head's weights; ``base`` the item's scores."""
+    item: tuple
+    wt: Optional[tuple]
+    repeat: bool
+    params: tuple
+    base: Predictive
+    _wt_r: dict = field(default_factory=dict, repr=False)
+
+    def score(self, item, *, r=None, sample=None, wt=None):
+        """(logits, prob_mean, prob_std) of a pass item.  The head reads it against ``wt`` when given, else against the
+        fixed wild type repeated for a pass of r copies of the batch (built once per r) or gathered by ``sample``."""
+        if self.repeat:
+            items = [item, item]
+        elif wt is not None:
+            items = [item, wt]
+        elif self.wt is None:
+            items = [item]
+        elif sample is not None:
+            items = [item, tuple(t[:, sample] if t.dim() == 3 else t[sample] for t in self.wt)]
+        else:
+            if r not in self._wt_r:
+                self._wt_r[r] = tuple(_repeat(t, r) for t in self.wt)
+            items = [item, self._wt_r[r]]
+        return IF._C.head_mc_infer(items, *self.params)
+
+
+def _scorer(model, graph_data, sequence_data, peptide_property, eps, samples) -> _Scorer:
+    """The scorer of ``model.forward``'s one item (``predictive``): drawn, then encoded and scored.  Under no_grad."""
+    params = _head_params(model)
+    e = _draws(model, eps, samples, graph_data.n_graphs, graph_data.ndata["x"])
+    item = _encode(model, graph_data, sequence_data, peptide_property) + (e,)
+    repeat = isinstance(model, _Comparative) and model.use_wt_for_downstream
+    base = Predictive(*IF._C.head_mc_infer([item, item] if repeat else [item], *params))
+    return _Scorer(item, None, repeat, params, base)
+
+
+def _scorer_pair(model, graph_pair, sequence_pair, property_pair, eps, samples) -> _Scorer:
+    """The scorer of ``model.forward_comparative``'s cancer item against its wild type (``predictive_pair``): both items
+    drawn, cancer first, then encoded and scored; the wild type is neither drawn nor run without
+    ``use_wt_for_downstream``.  Under no_grad."""
+    n = _pair_items(model, eps)
+    params = _head_params(model)
+    k = samples if eps is None else eps[0].shape[0]
+    draws = [_draws(model, None if eps is None else eps[i], k, graph_pair[i].n_graphs, graph_pair[i].ndata["x"])
+             for i in range(n)]
+    items = [_encode(model, graph_pair[i], sequence_pair[i], property_pair[i]) + (draws[i],) for i in range(n)]
+    base = Predictive(*IF._C.head_mc_infer(items, *params))
+    return _Scorer(items[0], items[1] if n == 2 else None, False, params, base)
 
 
 def predictive(model, graph_data, sequence_data, peptide_property, *, samples: int = 32,
@@ -110,12 +169,7 @@ def predictive(model, graph_data, sequence_data, peptide_property, *, samples: i
     trunk and the VAE encoder run once, the head runs once for all draws."""
     _check(model, samples, (_Hybrid, _Comparative), "predictive", _CLASSES)
     with torch.no_grad():
-        params = _head_params(model)
-        pooled, mu, logvar, z_vae = _encode(model, graph_data, sequence_data, peptide_property)
-        e = _draws(model, eps, samples, mu.shape[0], mu)
-        item = (pooled, mu, logvar, z_vae, e)
-        pair = isinstance(model, _Comparative) and model.use_wt_for_downstream
-        return Predictive(*IF._C.head_mc_infer([item, item] if pair else [item], *params))
+        return _scorer(model, graph_data, sequence_data, peptide_property, eps, samples).base
 
 
 def predictive_pair(model, graph_pair, sequence_pair, property_pair, *, samples: int = 32,
@@ -129,13 +183,5 @@ def predictive_pair(model, graph_pair, sequence_pair, property_pair, *, samples:
     numbers that K sequential forwards would consume, only numbers of the same distribution.  Eval mode, no_grad and
     ``.grad`` as in ``predictive``."""
     _check(model, samples, _Comparative, "predictive_pair", _PAIR_CLASSES)
-    n = _pair_items(model, eps)
     with torch.no_grad():
-        params = _head_params(model)
-        items = []
-        for i in range(n):
-            pooled, mu, logvar, z_vae = _encode(model, graph_pair[i], sequence_pair[i], property_pair[i])
-            k = samples if eps is None else eps[0].shape[0]
-            e = _draws(model, None if eps is None else eps[i], k, mu.shape[0], mu)
-            items.append((pooled, mu, logvar, z_vae, e))
-        return Predictive(*IF._C.head_mc_infer(items, *params))
+        return _scorer_pair(model, graph_pair, sequence_pair, property_pair, eps, samples).base

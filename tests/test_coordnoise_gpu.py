@@ -13,8 +13,8 @@ from scipy import stats
 import immunostruct_b200 as I
 from immunostruct_b200 import _C
 from immunostruct_b200.coordnoise import coordinate_ensemble, coordinate_ensemble_pair
-from immunostruct_b200.mutagenesis import scan_passes
 from immunostruct_b200.predictive import predictive, predictive_pair
+from immunostruct_b200.resident import scan_passes
 from immunostruct_b200.synthetic import synthetic_dense, synthetic_graph_arrays
 from oracle import reference_ops as R
 

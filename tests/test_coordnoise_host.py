@@ -12,7 +12,7 @@ from scipy import stats
 import immunostruct_b200 as I
 from immunostruct_b200 import _C, trunk
 from immunostruct_b200.coordnoise import coordinate_ensemble, coordinate_ensemble_pair
-from immunostruct_b200.mutagenesis import scan_passes
+from immunostruct_b200.resident import scan_passes
 from oracle import kernel_contracts as KC
 from oracle import reference_ops as R
 

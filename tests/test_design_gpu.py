@@ -15,8 +15,9 @@ import torch
 import immunostruct_b200 as I
 from immunostruct_b200 import _C
 from immunostruct_b200.design import beam_search, beam_search_pair, round_slots
-from immunostruct_b200.mutagenesis import mutational_scan, scan_passes, score_variants
+from immunostruct_b200.mutagenesis import mutational_scan, score_variants
 from immunostruct_b200.predictive import predictive, predictive_pair
+from immunostruct_b200.resident import scan_passes
 from immunostruct_b200.synthetic import synthetic_dense
 
 from helpers import graph_batch, inject_eps, log_error

@@ -12,7 +12,7 @@ import torch.nn.functional as F
 import immunostruct_b200 as I
 from immunostruct_b200 import _C, trunk
 from immunostruct_b200.design import beam_search, beam_search_pair, round_slots
-from immunostruct_b200.mutagenesis import scan_passes
+from immunostruct_b200.resident import scan_passes
 from oracle import kernel_contracts as KC
 from oracle import reference_ops as R
 

@@ -15,8 +15,9 @@ import torch.nn.functional as F
 
 import immunostruct_b200 as I
 from immunostruct_b200 import _C
-from immunostruct_b200.mutagenesis import mutational_scan, mutational_scan_pair, scan_passes, scan_sites
+from immunostruct_b200.mutagenesis import mutational_scan, mutational_scan_pair, scan_sites
 from immunostruct_b200.predictive import predictive, predictive_pair
+from immunostruct_b200.resident import scan_passes
 from immunostruct_b200.synthetic import split_graphs, synthetic_dense, synthetic_graph_arrays
 from oracle import reference_ops as R
 

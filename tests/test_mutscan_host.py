@@ -8,7 +8,8 @@ import torch.nn.functional as F
 
 import immunostruct_b200 as I
 from immunostruct_b200 import _C, trunk
-from immunostruct_b200.mutagenesis import mutational_scan, mutational_scan_pair, scan_passes, scan_sites
+from immunostruct_b200.mutagenesis import mutational_scan, mutational_scan_pair, scan_sites
+from immunostruct_b200.resident import scan_passes
 from oracle import kernel_contracts as KC
 from oracle import reference_ops as R
 

@@ -9,10 +9,10 @@ import torch
 
 import immunostruct_b200 as I
 from immunostruct_b200 import _C
-from immunostruct_b200.mutagenesis import variant_passes
 from immunostruct_b200.occlusion import (_contact_tables, _residue_tables, occlude_contacts, occlude_contacts_pair,
                                          occlude_residues, occlude_residues_pair)
 from immunostruct_b200.predictive import predictive, predictive_pair
+from immunostruct_b200.resident import variant_passes
 from immunostruct_b200.synthetic import synthetic_dense
 from oracle import reference_ops as R
 

@@ -8,9 +8,9 @@ import torch
 
 import immunostruct_b200 as I
 from immunostruct_b200 import _C, trunk
-from immunostruct_b200.mutagenesis import variant_passes
 from immunostruct_b200.occlusion import (_contact_tables, _residue_tables, occlude_contacts, occlude_contacts_pair,
                                          occlude_residues, occlude_residues_pair)
+from immunostruct_b200.resident import variant_passes
 from oracle import kernel_contracts as KC
 from oracle import reference_ops as R
 

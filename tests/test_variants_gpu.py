@@ -12,8 +12,9 @@ import torch
 
 import immunostruct_b200 as I
 from immunostruct_b200 import _C
-from immunostruct_b200.mutagenesis import mutational_scan, score_variants, score_variants_pair, variant_passes
+from immunostruct_b200.mutagenesis import mutational_scan, score_variants, score_variants_pair
 from immunostruct_b200.predictive import predictive, predictive_pair
+from immunostruct_b200.resident import variant_passes
 from immunostruct_b200.synthetic import split_graphs, synthetic_dense, synthetic_graph_arrays
 from oracle import reference_ops as R
 

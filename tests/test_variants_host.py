@@ -8,7 +8,8 @@ import torch.nn.functional as F
 
 import immunostruct_b200 as I
 from immunostruct_b200 import _C, trunk
-from immunostruct_b200.mutagenesis import score_variants, score_variants_pair, variant_passes
+from immunostruct_b200.mutagenesis import score_variants, score_variants_pair
+from immunostruct_b200.resident import variant_passes
 from oracle import kernel_contracts as KC
 from oracle import reference_ops as R
 
