@@ -50,7 +50,8 @@ def exported_symbols():
             "is_contrastive_bwd", "is_fused_adam", "is_rotate_coords", "is_mask_single_residue", "is_mask_rows", "is_gemm_tma_split_k",
             "is_split_planes", "is_gemm_planes_tma", "is_egnn_set_ws_buffers", "is_egnn_set_ws_variant", "is_reduce_partials3", "is_fused_adam_capturable",
             "is_egnn_edge_attr_grad", "is_head_mc_infer", "is_mutscan_expand", "is_variant_expand", "is_design_expand",
-            "is_design_select", "is_egnn_layer_fwd_fp16x2", "is_occlusion_expand", "is_coord_noise_expand"]
+            "is_design_select", "is_egnn_layer_fwd_fp16x2", "is_occlusion_expand", "is_coord_noise_expand",
+            "is_shapley_plan", "is_shapley_expand", "is_shapley_reduce"]
 
 
 def _check(rc: int, name: str):
@@ -700,6 +701,82 @@ def coord_noise_expand(x23, node_off, sigma, seed, item, draw0, x23_out):
     _call("is_coord_noise_expand", _t(x23, f32, "x23"), _t(node_off, i64, "node_off"), _t(sigma, f32, "sigma"), _i32(r),
           _i32(b), _i64(n), ctypes.c_uint64(seed), ctypes.c_uint32(item), ctypes.c_uint32(draw0),
           _t(x23_out, f32, "x23_out"), _stream())
+
+
+def shapley_plan(node_off, edge_off, src_local, dst_local, players, player_off, var_off, seed, ranks, kept, flag):
+    """Permutation plan of the Shapley chains (csrc/shapley.cu): ``ranks`` int32 [B, T, Pmax] gets the rank rows of the
+    antithetic pairs of every sample (row 2u: Philox4x32-10 keys of counter (p, b, u, 2), key ``seed``; row 2u+1 its
+    reverse; -1 past P_b), ``kept`` int64 [V] the kept-edge count of every chain variant.  ``players`` int32 [N] (graph-
+    local ids, -1: never removed), ``player_off`` / ``var_off`` int64 [B+1] the running player and variant counts.
+    ``flag`` (int32 [1], zeroed by the caller) is raised for counts that disagree."""
+    i64, i32 = torch.int64, torch.int32
+    if ranks.dim() != 3 or node_off.dim() != 1:
+        raise ValueError("shapley_plan: ranks [B, T, Pmax] and node_off [B+1] expected")
+    b, t, pmax = ranks.shape
+    e = src_local.shape[0]
+    if (node_off.shape != (b + 1,) or edge_off.shape != (b + 1,) or dst_local.shape != (e,) or players.dim() != 1
+            or player_off.shape != (b + 1,) or var_off.shape != (b + 1,) or kept.dim() != 1 or flag.shape != (1,)):
+        raise ValueError("shapley_plan: unexpected shapes")
+    if not (b >= 1 and 2 <= t <= 2 ** 16 and t % 2 == 0 and 1 <= pmax <= 256):
+        raise ValueError("shapley_plan: T even in [2, 2^16] and 1 <= Pmax <= 256 expected")
+    if not (isinstance(seed, int) and 0 <= seed < 2 ** 64):
+        raise ValueError("shapley_plan: seed in [0, 2^64) expected")
+    _call("is_shapley_plan", _t(node_off, i64, "node_off"), _t(edge_off, i64, "edge_off"),
+          _t(src_local, i64, "src_local"), _t(dst_local, i64, "dst_local"), _t(players, i32, "players"),
+          _t(player_off, i64, "player_off"), _t(var_off, i64, "var_off"), _i32(b), _i32(t), _i32(pmax),
+          ctypes.c_uint64(seed), _t(ranks, i32, "ranks"), _t(kept, i64, "kept"), _t(flag, i32, "flag"), _stream())
+
+
+def shapley_expand(x23, node_off, edge_off, src_local, dst_local, edge_attr, players, ranks, sample, rank_row, threshold,
+                   node_out, edge_out, x23_out, src_out, dst_out, edge_attr_out, flag):
+    """One pass of coalition variants (csrc/shapley.cu): variant v is base graph sample[v] with every row i removed for
+    which players[i] >= 0 and ranks[rank_row[v], players[i]] < threshold[v] (its 23 floats become 0.0, every edge touching
+    it is dropped); x23 rows from node_out[v], the kept edges in base order from edge_out[v].  ``ranks`` int32 [R, Pmax]
+    (or [B, T, Pmax], read as [B T, Pmax]).  ``flag`` (int32 [1], zeroed by the caller) is raised, and the variant not
+    written, for an index out of range or offsets that disagree with the node count or the kept edge count."""
+    f32, i64, i32 = torch.float32, torch.int64, torch.int32
+    if x23.dim() != 2 or sample.dim() != 1 or ranks.dim() < 2:
+        raise ValueError("shapley_expand: x23 [N,23], sample [r] and ranks [R, Pmax] expected")
+    b, r, e, n = node_off.shape[0] - 1, sample.shape[0], src_local.shape[0], x23.shape[0]
+    pmax = ranks.shape[-1]
+    if (x23.shape[1] != 23 or b < 1 or edge_off.shape != (b + 1,) or dst_local.shape != (e,) or edge_attr.numel() != e
+            or players.shape != (n,) or rank_row.shape != (r,) or threshold.shape != (r,) or r < 1 or pmax < 1):
+        raise ValueError("shapley_expand: unexpected input shapes")
+    n_out, e_out = x23_out.shape[0], src_out.shape[0]
+    if (x23_out.dim() != 2 or x23_out.shape[1] != 23 or node_out.shape != (r + 1,) or edge_out.shape != (r + 1,)
+            or dst_out.shape != (e_out,) or edge_attr_out.numel() != e_out or flag.shape != (1,)):
+        raise ValueError("shapley_expand: unexpected output shapes")
+    if 2 * r > 0x7ffffffe:
+        raise ValueError("shapley_expand: too many variants in one pass")
+    _call("is_shapley_expand", _t(x23, f32, "x23"), _t(node_off, i64, "node_off"), _t(edge_off, i64, "edge_off"),
+          _t(src_local, i64, "src_local"), _t(dst_local, i64, "dst_local"), _t(edge_attr, f32, "edge_attr"),
+          _t(players, i32, "players"), _t(ranks, i32, "ranks"), _t(sample, i64, "sample"), _t(rank_row, i64, "rank_row"),
+          _t(threshold, i64, "threshold"), _t(node_out, i64, "node_out"), _t(edge_out, i64, "edge_out"), _i32(r),
+          _i32(b), _i64(ranks.numel() // pmax), _i32(pmax), _i64(n_out), _i64(e_out), _t(x23_out, f32, "x23_out"),
+          _t(src_out, i64, "src_out"), _t(dst_out, i64, "dst_out"), _t(edge_attr_out, f32, "edge_attr_out"),
+          _t(flag, i32, "flag"), _stream())
+
+
+def shapley_reduce(logits, base_logits, ranks, player_off, var_off, phi, se, gap, flag):
+    """Shapley values of the chains (csrc/shapley.cu), one CTA per sample: from the variants' logits [V, K], the base
+    logits [B, K] and the plan's ranks [B, T, Pmax], phi / se fp32 [2, Q] (row 0: of v_logit, row 1: of v_prob) at
+    player_off[b] + p, and gap fp32 [2, B] = (v(base) - v(empty)) - Σ_p phi; fp64 throughout, fixed order.  ``flag``
+    (int32 [1]) is raised for variant tables or ranks that disagree."""
+    f32, i64, i32 = torch.float32, torch.int64, torch.int32
+    if ranks.dim() != 3 or base_logits.dim() != 2 or logits.dim() != 2:
+        raise ValueError("shapley_reduce: logits [V,K], base_logits [B,K] and ranks [B,T,Pmax] expected")
+    b, t, pmax = ranks.shape
+    k, v, q = base_logits.shape[1], logits.shape[0], phi.shape[-1]
+    if (base_logits.shape[0] != b or logits.shape[1] != k or player_off.shape != (b + 1,) or var_off.shape != (b + 1,)
+            or phi.shape != (2, q) or se.shape != (2, q) or gap.shape != (2, b) or flag.shape != (1,)):
+        raise ValueError("shapley_reduce: unexpected shapes")
+    if not (b >= 1 and 2 <= t <= 2 ** 16 and t % 2 == 0 and 1 <= pmax <= 256 and k >= 1):
+        raise ValueError("shapley_reduce: T even in [2, 2^16], 1 <= Pmax <= 256 and K >= 1 expected")
+    row1 = lambda x, n: _vp(x.data_ptr() + 4 * n)                      # row 1 of a contiguous fp32 [2, n]
+    _call("is_shapley_reduce", _t(logits, f32, "logits"), _t(base_logits, f32, "base_logits"), _t(ranks, i32, "ranks"),
+          _t(player_off, i64, "player_off"), _t(var_off, i64, "var_off"), _i32(b), _i32(t), _i32(pmax), _i32(k), _i64(v),
+          _t(phi, f32, "phi"), row1(phi, q), _t(se, f32, "se"), row1(se, q), _t(gap, f32, "gap"), row1(gap, b),
+          _t(flag, i32, "flag"), _stream())
 
 
 def unpack_nodes(aa, xyz, x):

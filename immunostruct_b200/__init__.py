@@ -13,6 +13,7 @@ from .optim import FusedAdam, FusedAdamW  # noqa: F401
 from .augment import TrainAugment  # noqa: F401
 from .graphed import CapturedStep  # noqa: F401
 from . import attribution, augment, coordnoise, dataloading, design, mutagenesis, nn, occlusion, optim, ops, predictive  # noqa: F401
+from . import shapley  # noqa: F401
 from .ops import use_custom_ops  # noqa: F401
 from .functional import invalidate_caches  # noqa: F401
 

@@ -19,30 +19,13 @@
 // coordinate's sigma and z from the owning lane by shuffles.  No atomics, no barriers, no device flag: the host checks
 // every argument before the launch.
 #include "common.cuh"
+#include "philox.cuh"
 
 namespace is {
 
 constexpr int CN_THREADS = 256;
 constexpr int CN_WARPS = CN_THREADS / 32;
 constexpr int CN_CTAS_PER_SM = 4;
-
-struct Philox4 {
-    uint32_t v[4];
-};
-
-// Philox4x32-10: ten rounds of the 4x32 S-box, the key bumped by the Weyl constants between rounds
-__device__ __forceinline__ Philox4 philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0,
-                                                 uint32_t k1) {
-    constexpr uint32_t M0 = 0xD2511F53u, M1 = 0xCD9E8D57u, W0 = 0x9E3779B9u, W1 = 0xBB67AE85u;
-#pragma unroll
-    for (int round = 0; round < 10; ++round) {
-        if (round > 0) { k0 += W0; k1 += W1; }
-        const uint64_t p0 = (uint64_t)M0 * c0, p1 = (uint64_t)M1 * c2;
-        const uint32_t n0 = (uint32_t)(p1 >> 32) ^ c1 ^ k0, n2 = (uint32_t)(p0 >> 32) ^ c3 ^ k1;
-        c0 = n0; c1 = (uint32_t)p1; c2 = n2; c3 = (uint32_t)p0;
-    }
-    return Philox4{{c0, c1, c2, c3}};
-}
 
 __device__ __forceinline__ float cn_uniform(uint32_t v) {
     return (float)(((v >> 8) << 1) | 1u) * 0x1p-25f;

@@ -307,6 +307,45 @@ int is_occlusion_expand(const float* x23, const int64_t* node_off, const int64_t
  * sigma == 0 are copied bit-exact.  No device flag: the caller checks every argument (draw0 + r <= 2^32).  No atomics. */
 int is_coord_noise_expand(const float* x23, const int64_t* node_off, const float* sigma, int r, int n_graphs,
                           int64_t n_nodes, uint64_t seed, uint32_t item, uint32_t draw0, float* x23_out, void* stream);
+/* Shapley values over structural removals (csrc/shapley.cu).  players int32 [N]: the graph-local player id of each node
+ * row, -1 for a row never removed; sample b has P_b = player_off[b+1] - player_off[b] <= 256 players (ids 0 .. P_b - 1)
+ * and var_off[b+1] - var_off[b] = 1 + T (P_b - 1) variants (0 without players): the empty coalition (every player
+ * removed) first, then coalitions j = 1 .. P_b - 1 of permutation t = 0 .. T-1, t ascending then j ascending.  Removing
+ * a player zeroes the 23 floats of its rows and drops every edge touching one of them; kept edges keep their base order.
+ * The flag (int32 [1], zeroed by the caller, never cleared) is set to 1 for tables that disagree with the batch.
+ *
+ * is_shapley_plan: T even in [2, 2^16].  ranks int32 [B, T, max_players]: row 2u of sample b ranks its players by the
+ * key v0 of Philox4x32-10 with counter (p, b, u, 2) and key (low, high 32 bits of seed), ties to the smaller id; row
+ * 2u+1 is P_b - 1 minus row 2u; entries past P_b are -1.  kept int64 [V]: the kept-edge count of every variant.  Flag:
+ * P_b > min(256, max_players) or a variant count that is not 1 + T (P_b - 1).  Integer counts, no float atomics. */
+int is_shapley_plan(const int64_t* node_off, const int64_t* edge_off, const int64_t* src_local, const int64_t* dst_local,
+                    const int* players, const int64_t* player_off, const int64_t* var_off, int n_graphs,
+                    int permutations, int max_players, uint64_t seed, int* ranks, int64_t* kept, int* flag,
+                    void* stream);
+/* is_shapley_expand: one pass of r coalition variants of a resident batch (inputs as is_occlusion_expand).  Variant v is
+ * base graph b = sample[v] with every row i removed for which players[i] >= 0 and ranks[rank_row[v]][players[i]] <
+ * threshold[v] (ranks int32 [n_rank_rows, max_players]); its rows go to x23_out from row node_out[v], its kept edges to
+ * src_out / dst_out / edge_attr_out from edge_out[v].  Bit-exact (copies and 0.0 only).  Flag, and that variant not
+ * written: sample outside [0, B), rank_row outside [0, n_rank_rows), threshold outside [0, max_players], n_b > 256, a
+ * player id >= max_players, node_out[v+1] - node_out[v] != n_b, a kept count that is not edge_out[v+1] - edge_out[v], or
+ * offsets past n_nodes_out / n_edges_out.  No atomics. */
+int is_shapley_expand(const float* x23, const int64_t* node_off, const int64_t* edge_off, const int64_t* src_local,
+                      const int64_t* dst_local, const float* edge_attr, const int* players, const int* ranks,
+                      const int64_t* sample, const int64_t* rank_row, const int64_t* threshold, const int64_t* node_out,
+                      const int64_t* edge_out, int r, int n_graphs, int64_t n_rank_rows, int max_players,
+                      int64_t n_nodes_out, int64_t n_edges_out, float* x23_out, int64_t* src_out, int64_t* dst_out,
+                      float* edge_attr_out, int* flag, void* stream);
+/* is_shapley_reduce: logits [V, K] of the variants, base_logits [B, K] of the unmodified batch, ranks [B, T,
+ * max_players] as is_shapley_plan writes them.  v_logit = mean over k of the logit, v_prob = mean of sigmoid(logit), in
+ * fp64; the player at position j-1 of permutation t gets Δ = v(t, j-1) - v(t, j) (j = 0: base, j = P_b: the empty
+ * variant); d_u = (Δ_2u + Δ_2u+1) / 2; phi = mean over u of d_u and se = sqrt(Σ_u (d_u - phi)^2 / (U (U - 1))), U = T/2
+ * (NaN for U = 1), accumulated over u ascending, rounded to fp32 into phi_* / se_* [Q] at player_off[b] + p.
+ * gap_* [B] = (v(base) - v(empty)) - Σ_p phi(p) (0 without players).  Flag: the variant tables or a rank outside
+ * [0, P_b).  Deterministic, no atomics. */
+int is_shapley_reduce(const float* logits, const float* base_logits, const int* ranks, const int64_t* player_off,
+                      const int64_t* var_off, int n_graphs, int permutations, int max_players, int n_draws,
+                      int64_t n_variants, float* phi_logit, float* phi_prob, float* se_logit, float* se_prob,
+                      float* gap_logit, float* gap_prob, int* flag, void* stream);
 /* Dense Linear layer on the tensor cores: C[M,N] = act(A[M,K] W[N,K]^T + bias), fp32 in / out, operands split
  * on the fly into three bf16 terms (precision 3, fp32-accurate) or rounded to bf16 (precision 0).  Replaces the
  * nn.Linear layers of the sequence VAE (reference models/hybrid_models.py:63-74: vae_fc1 with ReLU, vae_fc4) in the
