@@ -51,7 +51,7 @@ def exported_symbols():
             "is_split_planes", "is_gemm_planes_tma", "is_egnn_set_ws_buffers", "is_egnn_set_ws_variant", "is_reduce_partials3", "is_fused_adam_capturable",
             "is_egnn_edge_attr_grad", "is_head_mc_infer", "is_mutscan_expand", "is_variant_expand", "is_design_expand",
             "is_design_select", "is_egnn_layer_fwd_fp16x2", "is_occlusion_expand", "is_coord_noise_expand",
-            "is_shapley_plan", "is_shapley_expand", "is_shapley_reduce"]
+            "is_shapley_plan", "is_shapley_expand", "is_shapley_reduce", "is_head_features_infer", "is_knn"]
 
 
 def _check(rc: int, name: str):
@@ -521,6 +521,93 @@ def head_mc_infer(items, Wc, bc, coef, n_head, W1, b1, W2, b2):
           _t(coef, f32, "coef"), _i32(n_head), _t(W1, f32, "W1"), _t(b1, f32, "b1"), _t(W2, f32, "W2"), _t(b2, f32, "b2"),
           _t(logits, f32, "logits"), _t(mean, f32, "prob_mean"), _t(std, f32, "prob_std"), _i32(b), _i32(k), _stream())
     return logits, mean, std
+
+
+def head_features_infer(items, Wc, bc, coef, n_head, W1, b1):
+    """The classifier's hidden layer of the eval-mode head at z = mu (csrc/head.cu).  ``items``: one (pooled [B,64],
+    mu [B,LD], z_vae [B,LD+PD]) tuple, or two for a cancer / wild-type pair (tokens item-major); the weights as in
+    ``head_mc_infer``.  -> hid [B,32]."""
+    f32 = torch.float32
+    if len(items) not in (1, 2) or any(len(it) != 3 for it in items):
+        raise ValueError("head_features_infer: one or two (pooled, mu, z_vae) items")
+    b, ld = items[0][1].shape
+    lz = items[0][2].shape[1]
+    for pooled, mu, zv in items:
+        if pooled.shape != (b, 64) or mu.shape != (b, ld) or zv.shape != (b, lz):
+            raise ValueError("head_features_infer: unexpected item shapes")
+    L = len(items) * (64 + lz)
+    if b < 1 or W1.shape != (32, L) or b1.shape != (32,) or lz < ld or L > 256:
+        raise ValueError("head_features_infer: unexpected classifier shapes")
+    if (Wc is None) != (bc is None) or (Wc is not None and (Wc.shape != (64, 64) or bc.shape != (64,))):
+        raise ValueError("head_features_infer: Wc / bc must both be None or [64,64] / [64]")
+    if coef is not None and (not 1 <= n_head <= 8 or coef.shape != (4 * n_head + 1,)):
+        raise ValueError("head_features_infer: coef must hold 4 n_head + 1 values, 1 <= n_head <= 8")
+    hid = torch.empty(b, 32, dtype=f32, device=items[0][0].device)
+    names = ("pooled", "mu", "z_vae")
+    ptrs = [_t(t, f32, f"{n}{i}") for i, it in enumerate((items[0], items[1] if len(items) == 2 else (None,) * 3))
+            for t, n in zip(it, names)]
+    _call("is_head_features_infer", *ptrs, _i32(len(items)), _i32(ld), _i32(lz - ld), _t(Wc, f32, "Wc"),
+          _t(bc, f32, "bc"), _t(coef, f32, "coef"), _i32(n_head), _t(W1, f32, "W1"), _t(b1, f32, "b1"),
+          _t(hid, f32, "hid"), _i32(b), _stream())
+    return hid
+
+
+KNN_MAX_K, KNN_MAX_DIM, KNN_QUERY_TILE = 64, 256, 64
+
+
+def knn_max_slices(n_bank: int) -> int:
+    """Largest bank slice count of ``knn`` for a bank of ``n_bank`` rows (every slice holds a 128-row tile)."""
+    return min(65535, (n_bank + 127) // 128)
+
+
+def knn(query, bank, k, exclude=None, *, slices=1):
+    """Exact k nearest bank rows of every query row in squared Euclidean distance (csrc/knn.cu; the contract is in its
+    header).  query [Q, D], bank [R, D] fp32 CUDA contiguous, 1 <= k <= 64, 1 <= D <= 256, 1 <= R < 2^31; exclude int64
+    [Q] in [-1, R) or None.  ``slices`` = S bank slices searched by separate CTAs, 1 .. ``knn_max_slices(R)``; S > 1
+    adds a [Q, S, k] workspace and the merge kernel.  The range of ``exclude`` is checked with one host read.
+    -> (index [Q, k] int64, distance [Q, k] fp32), ascending by (distance, index); unfilled slots -1 / +inf."""
+    global LAUNCHES
+    for t, name in ((query, "query"), (bank, "bank")):
+        if not isinstance(t, torch.Tensor) or t.dim() != 2:
+            raise ValueError(f"knn: {name} must be a 2-D tensor [n, D]")
+        if t.dtype is not torch.float32:
+            raise ValueError(f"knn: {name} must be float32, got {t.dtype}")
+        if not t.is_contiguous():
+            raise ValueError(f"knn: {name} must be contiguous")
+    (q, d), (r, d2) = query.shape, bank.shape
+    if d != d2:
+        raise ValueError(f"knn: query and bank must have the same feature count, got {d} and {d2}")
+    if not 1 <= d <= KNN_MAX_DIM:
+        raise ValueError(f"knn: 1 <= D <= {KNN_MAX_DIM} features expected, got {d}")
+    if q < 1 or not 1 <= r < 2 ** 31:
+        raise ValueError(f"knn: at least one query and 1 <= R < 2^31 bank rows expected, got Q = {q}, R = {r}")
+    if isinstance(k, bool) or not isinstance(k, int) or not 1 <= k <= KNN_MAX_K:
+        raise ValueError(f"knn: k must be an int in [1, {KNN_MAX_K}], got {k!r}")
+    if isinstance(slices, bool) or not isinstance(slices, int) or not 1 <= slices <= knn_max_slices(r):
+        raise ValueError(f"knn: slices must be an int in [1, {knn_max_slices(r)}] for {r} bank rows, got {slices!r}")
+    if exclude is not None:
+        if not isinstance(exclude, torch.Tensor) or exclude.dtype is not torch.int64 or exclude.shape != (q,):
+            raise ValueError(f"knn: exclude must be an int64 tensor of shape [{q}]")
+        lo, hi = torch.stack([exclude.min(), exclude.max()]).tolist()
+        if lo < -1 or hi >= r:
+            raise ValueError(f"knn: exclude entries must lie in [-1, {r}), got [{lo}, {hi}]")
+        exclude = exclude.contiguous()
+    for t, name in ((query, "query"), (bank, "bank"), (exclude, "exclude")):
+        if t is not None and not t.is_cuda:
+            raise RuntimeError(f"knn: {name} must be a CUDA tensor (immunostruct_b200 has no CPU path), got {t.device}")
+        if t is not None and t.device != query.device:
+            raise RuntimeError(f"knn: {name} must live on {query.device}, got {t.device}")
+    dev = query.device
+    index = torch.empty(q, k, dtype=torch.int64, device=dev)
+    distance = torch.empty(q, k, dtype=torch.float32, device=dev)
+    ws = torch.empty(q * slices * k, dtype=torch.int64, device=dev) if slices > 1 else None
+    _call("is_knn", _t(query, torch.float32, "query"), _t(bank, torch.float32, "bank"),
+          _t(exclude, torch.int64, "exclude"), _i64(q), _i64(r), _i32(d), _i32(k), _i32(slices),
+          _t(ws, torch.int64, "workspace"), _t(index, torch.int64, "index"), _t(distance, torch.float32, "distance"),
+          _stream())
+    if slices > 1:
+        LAUNCHES += 1
+    return index, distance
 
 
 def mutscan_expand(x23, node_off, node_index, seq, seq_index, seq_columns, sites, x23_out, seq_out, flag):

@@ -348,6 +348,72 @@ head_mc_infer_kernel(McItem it0, McItem it1, int n_items, int LD, int PD, const 
     }
 }
 
+// ---- classifier hidden layer at z = mu: one CTA per sample ---------------------------------------------------------
+// The tokens of one item are [x_gat | mu | prop]; the head of head_infer_kernel up to hid, with the same device functions
+// (the extremes of c are order-independent), so a sample's features are bit-identical to head_infer's hid on z_vae =
+// [mu | prop].
+struct FeatItem {
+    const float* pooled;         // [B, 64]
+    const float* mu;             // [B, LD]
+    const float* zv;             // [B, LD + PD] (the PD property columns are read)
+};
+
+__global__ void __launch_bounds__(IS_THREADS)
+head_features_infer_kernel(FeatItem it0, FeatItem it1, int n_items, int LD, int PD, const float* __restrict__ Wc,
+                           const float* __restrict__ bc, const float* __restrict__ coef, int H,
+                           const float* __restrict__ W1, const float* __restrict__ b1, float* __restrict__ hid) {
+    __shared__ float c[IS_HEAD_LMAX];
+    __shared__ float f[IS_HEAD_LMAX];
+    __shared__ float Eh[IS_HEAD_LMAX * IS_HEAD_HMAX];
+    __shared__ float s_mm[2];
+    __shared__ float red[2 * 8];
+    const int b = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int LZ = LD + PD, LI = 64 + LZ, L = n_items * LI;
+    for (int r = warp; r < n_items * 64; r += IS_THREADS / 32) {
+        const int it = r >> 6, o = r & 63;
+        const float* pooled = (it ? it1 : it0).pooled + (int64_t)b * 64;
+        if (Wc != nullptr) {
+            const float a = head_xgat_row(Wc, bc, o, __ldg(pooled + lane), __ldg(pooled + 32 + lane), lane);
+            if (lane == 0) c[it * LI + o] = a;
+        } else if (lane == 0) {
+            c[it * LI + o] = __ldg(pooled + o);
+        }
+    }
+    for (int idx = tid; idx < n_items * LZ; idx += IS_THREADS) {
+        const int it = idx >= LZ, t = idx - it * LZ;
+        const FeatItem& m = it ? it1 : it0;
+        c[it * LI + 64 + t] = t < LD ? __ldg(m.mu + (int64_t)b * LD + t) : __ldg(m.zv + (int64_t)b * LZ + t);
+    }
+    __syncthreads();
+    const float* feat = c;
+    if (coef != nullptr) {
+        float lmax = -INFINITY, lmin = INFINITY;
+        for (int i = tid; i < L; i += IS_THREADS) { lmax = fmaxf(lmax, c[i]); lmin = fminf(lmin, c[i]); }
+        lmax = warp_max(lmax); lmin = -warp_max(-lmin);
+        if (lane == 0) { red[warp] = lmax; red[8 + warp] = lmin; }
+        __syncthreads();
+        if (tid == 0) {
+            float a = red[0], m = red[8];
+            for (int w = 1; w < 8; ++w) { a = fmaxf(a, red[w]); m = fminf(m, red[8 + w]); }
+            s_mm[0] = a; s_mm[1] = m;
+        }
+        __syncthreads();
+        const float cmax = s_mm[0], cmin = s_mm[1];
+        for (int idx = tid; idx < L * H; idx += IS_THREADS) {
+            const int i = idx / H, h = idx - i * H;
+            Eh[idx] = head_fusion_expect(c, L, i, coef, H, h, cmax, cmin);
+        }
+        __syncthreads();
+        for (int i = tid; i < L; i += IS_THREADS) f[i] = head_fusion_out(Eh + i * H, coef, H);
+        __syncthreads();
+        feat = f;
+    }
+    for (int o = warp; o < 32; o += IS_THREADS / 32) {
+        const float a = head_hidden_row(W1, b1, feat, L, o, lane);
+        if (lane == 0) hid[(int64_t)b * 32 + o] = a;
+    }
+}
+
 // mean and population standard deviation of sigmoid(logit) over the K draws of each sample: one warp per sample, lanes
 // strided over the draws, fp64, two passes, fixed butterfly order (no atomics: the result depends on the logits only)
 __device__ __forceinline__ double warp_sum_f64(double v) {
@@ -448,6 +514,26 @@ int is_head_mc_infer(const float* pooled0, const float* mu0, const float* logvar
     IS_LAUNCH_CHECK();
     head_mc_stats_kernel<<<(n_samples + IS_THREADS / 32 - 1) / (IS_THREADS / 32), IS_THREADS, 0, (cudaStream_t)stream>>>(
         logits, n_samples, n_draws, prob_mean, prob_std);
+    IS_LAUNCH_CHECK();
+    return IS_OK;
+}
+
+// The classifier's hidden layer of the eval-mode head at z = mu (see head_features_infer_kernel): item i = (pooled_i
+// [B,64], mu_i [B,LD], z_vae_i [B,LD+PD] (property columns)), tokens item-major as in is_head_mc_infer; Wc / bc, coef
+// and W1 / b1 as in is_head_infer.  -> hid [B,32].
+int is_head_features_infer(const float* pooled0, const float* mu0, const float* z_vae0, const float* pooled1,
+                           const float* mu1, const float* z_vae1, int n_items, int latent, int prop_dim, const float* Wc,
+                           const float* bc, const float* coef, int n_head, const float* W1, const float* b1, float* hid,
+                           int n_samples, void* stream) {
+    if (n_samples <= 0 || latent <= 0 || prop_dim < 0 || (n_items != 1 && n_items != 2)) return IS_ERR_ARG;
+    if (n_items * (64 + latent + prop_dim) > IS_HEAD_LMAX) return IS_ERR_ARG;
+    if (coef != nullptr && (n_head < 1 || n_head > IS_HEAD_HMAX)) return IS_ERR_ARG;
+    if ((Wc == nullptr) != (bc == nullptr) || !W1 || !b1 || !hid || !pooled0 || !mu0 || !z_vae0) return IS_ERR_ARG;
+    if (n_items == 2 && (!pooled1 || !mu1 || !z_vae1)) return IS_ERR_ARG;
+    const FeatItem it0{pooled0, mu0, z_vae0};
+    const FeatItem it1 = n_items == 2 ? FeatItem{pooled1, mu1, z_vae1} : it0;
+    head_features_infer_kernel<<<n_samples, IS_THREADS, 0, (cudaStream_t)stream>>>(
+        it0, it1, n_items, latent, prop_dim, Wc, bc, coef, coef != nullptr ? n_head : 0, W1, b1, hid);
     IS_LAUNCH_CHECK();
     return IS_OK;
 }

@@ -219,6 +219,15 @@ int is_head_mc_infer(const float* pooled0, const float* mu0, const float* logvar
                      int n_items, int latent, int prop_dim, const float* Wc, const float* bc, const float* coef, int n_head,
                      const float* W1, const float* b1, const float* W2, const float* b2, float* logits, float* prob_mean,
                      float* prob_std, int n_samples, int n_draws, void* stream);
+/* is_head_features_infer: the classifier's hidden layer ReLU(W1 f + b1) [B,32] of the head of is_head_mc_infer at
+ * z = mu (no noise), the features that the output layer reads (neighbors.embed).  Item i supplies pooled_i [B,64], mu_i
+ * [B,latent] and z_vae_i [B,latent+prop_dim] (only its property columns are read); tokens item-major as in
+ * is_head_mc_infer.  Bit-identical to the hid of is_head_infer on z_vae = [mu | prop].  Item 1's pointers are ignored
+ * when n_items = 1. */
+int is_head_features_infer(const float* pooled0, const float* mu0, const float* z_vae0, const float* pooled1,
+                           const float* mu1, const float* z_vae1, int n_items, int latent, int prop_dim, const float* Wc,
+                           const float* bc, const float* coef, int n_head, const float* W1, const float* b1, float* hid,
+                           int n_samples, void* stream);
 /* is_mutscan_expand (csrc/mutscan.cu): one pass of single-residue mutants for an in-silico saturation scan.  Copy k < r of
  * the base batch (x23 [N,23], node_off [B+1], seq [B,L,V]) carries sites[k] = (p, c) (int32 pairs): x23_out [r N, 23] and
  * seq_out [r B, L, V] are r copies of the base where, for every graph b with node_index[b,p] >= 0 (int64 [B,P], graph-local;
@@ -427,6 +436,20 @@ int is_mask_single_residue(float* x, int64_t ldx, int n_feat, const int64_t* nod
                            const int64_t* want_aa, int64_t* aa_out, int64_t* node_out, void* stream);
 int is_mask_rows(float* data, int64_t ld, int n_cols, const int64_t* seg_off, const int64_t* limit, int n_segments,
                  const float* keys, int count, int fill_col, int max_rows, void* stream);
+
+/* ---- exact k-nearest-neighbour search (csrc/knn.cu; neighbors.nearest) ---------------------------------------------
+ * query [Q, D], bank [R, D] fp32 row-major; 1 <= k <= 64, 1 <= D <= 256, 1 <= R < 2^31; exclude int64 [Q] (the bank row
+ * query q must not return, -1 = none; every entry in [-1, R)) or NULL.
+ *   distance: squared Euclidean in fp32, one rounding sequence per pair: acc = 0; for d = 0 .. D-1 ascending, t = q_d -
+ *     r_d, acc = fmaf(t, t, acc); independent of tiling, slicing and Q.  One metric: pass L2-normalised rows for cosine
+ *     order (|a - b|^2 = 2 - 2 cos).
+ *   order: ascending in (distance, bank index), ties to the smaller index; bit-identical for any slice count.
+ *   missing data: a pair whose distance is NaN is never returned (a bank row or a query with a NaN feature); unfilled
+ *     slots hold index -1 and distance +inf.
+ * slices S in [1, min(65535, ceil(R / 128))]: the bank is split among S CTAs per query tile; S > 1 needs workspace
+ * uint64 [Q, S, k] and adds one merge kernel.  -> index int64 [Q, k], distance fp32 [Q, k]. */
+int is_knn(const float* query, const float* bank, const int64_t* exclude, int64_t n_query, int64_t n_bank, int dim, int k,
+           int slices, unsigned long long* workspace, int64_t* index, float* distance, void* stream);
 
 #ifdef __cplusplus
 }
