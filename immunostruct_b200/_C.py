@@ -51,7 +51,8 @@ def exported_symbols():
             "is_split_planes", "is_gemm_planes_tma", "is_egnn_set_ws_buffers", "is_egnn_set_ws_variant", "is_reduce_partials3", "is_fused_adam_capturable",
             "is_egnn_edge_attr_grad", "is_head_mc_infer", "is_mutscan_expand", "is_variant_expand", "is_design_expand",
             "is_design_select", "is_egnn_layer_fwd_fp16x2", "is_occlusion_expand", "is_coord_noise_expand",
-            "is_shapley_plan", "is_shapley_expand", "is_shapley_reduce", "is_head_features_infer", "is_knn"]
+            "is_shapley_plan", "is_shapley_expand", "is_shapley_reduce", "is_head_features_infer", "is_knn",
+            "is_shapley_edge_plan", "is_shapley_edge_expand"]
 
 
 def _check(rc: int, name: str):
@@ -842,6 +843,57 @@ def shapley_expand(x23, node_off, edge_off, src_local, dst_local, edge_attr, pla
           _i32(b), _i64(ranks.numel() // pmax), _i32(pmax), _i64(n_out), _i64(e_out), _t(x23_out, f32, "x23_out"),
           _t(src_out, i64, "src_out"), _t(dst_out, i64, "dst_out"), _t(edge_attr_out, f32, "edge_attr_out"),
           _t(flag, i32, "flag"), _stream())
+
+
+def shapley_edge_plan(edge_off, edge_players, player_off, var_off, seed, ranks, kept, flag):
+    """Permutation plan of the contact Shapley chains (csrc/shapley.cu): as ``shapley_plan`` with the players held by
+    edges, ``edge_players`` int32 [E] (graph-local ids, -1: never removed), and the keys on counter (p, b, u, 3).  An edge
+    of player q is kept in coalition j of permutation t iff j <= rank_t(q)."""
+    i64, i32 = torch.int64, torch.int32
+    if ranks.dim() != 3 or edge_off.dim() != 1:
+        raise ValueError("shapley_edge_plan: ranks [B, T, Pmax] and edge_off [B+1] expected")
+    b, t, pmax = ranks.shape
+    if (edge_off.shape != (b + 1,) or edge_players.dim() != 1 or player_off.shape != (b + 1,)
+            or var_off.shape != (b + 1,) or kept.dim() != 1 or flag.shape != (1,)):
+        raise ValueError("shapley_edge_plan: unexpected shapes")
+    if not (b >= 1 and 2 <= t <= 2 ** 16 and t % 2 == 0 and 1 <= pmax <= 256):
+        raise ValueError("shapley_edge_plan: T even in [2, 2^16] and 1 <= Pmax <= 256 expected")
+    if not (isinstance(seed, int) and 0 <= seed < 2 ** 64):
+        raise ValueError("shapley_edge_plan: seed in [0, 2^64) expected")
+    _call("is_shapley_edge_plan", _t(edge_off, i64, "edge_off"), _t(edge_players, i32, "edge_players"),
+          _t(player_off, i64, "player_off"), _t(var_off, i64, "var_off"), _i32(b), _i32(t), _i32(pmax),
+          ctypes.c_uint64(seed), _t(ranks, i32, "ranks"), _t(kept, i64, "kept"), _t(flag, i32, "flag"), _stream())
+
+
+def shapley_edge_expand(x23, node_off, edge_off, src_local, dst_local, edge_attr, edge_players, ranks, sample, rank_row,
+                        threshold, node_out, edge_out, x23_out, src_out, dst_out, edge_attr_out, flag):
+    """One pass of contact coalition variants (csrc/shapley.cu): variant v is base graph sample[v] with its rows copied
+    and every edge e with edge_players[e] >= 0 and ranks[rank_row[v], edge_players[e]] < threshold[v] dropped, the kept
+    edges in base order from edge_out[v].  ``ranks`` int32 [R, Pmax] (or [B, T, Pmax]).  ``flag`` (int32 [1], zeroed by
+    the caller) is raised, and the variant not written, for an index out of range, an edge player id >= Pmax, or
+    offsets that disagree with the node count or the kept edge count."""
+    f32, i64, i32 = torch.float32, torch.int64, torch.int32
+    if x23.dim() != 2 or sample.dim() != 1 or ranks.dim() < 2:
+        raise ValueError("shapley_edge_expand: x23 [N,23], sample [r] and ranks [R, Pmax] expected")
+    b, r, e = node_off.shape[0] - 1, sample.shape[0], src_local.shape[0]
+    pmax = ranks.shape[-1]
+    if (x23.shape[1] != 23 or b < 1 or edge_off.shape != (b + 1,) or dst_local.shape != (e,) or edge_attr.numel() != e
+            or edge_players.shape != (e,) or rank_row.shape != (r,) or threshold.shape != (r,) or r < 1
+            or not 1 <= pmax <= 256):
+        raise ValueError("shapley_edge_expand: unexpected input shapes")
+    n_out, e_out = x23_out.shape[0], src_out.shape[0]
+    if (x23_out.dim() != 2 or x23_out.shape[1] != 23 or node_out.shape != (r + 1,) or edge_out.shape != (r + 1,)
+            or dst_out.shape != (e_out,) or edge_attr_out.numel() != e_out or flag.shape != (1,)):
+        raise ValueError("shapley_edge_expand: unexpected output shapes")
+    if 2 * r > 0x7ffffffe:
+        raise ValueError("shapley_edge_expand: too many variants in one pass")
+    _call("is_shapley_edge_expand", _t(x23, f32, "x23"), _t(node_off, i64, "node_off"), _t(edge_off, i64, "edge_off"),
+          _t(src_local, i64, "src_local"), _t(dst_local, i64, "dst_local"), _t(edge_attr, f32, "edge_attr"),
+          _t(edge_players, i32, "edge_players"), _t(ranks, i32, "ranks"), _t(sample, i64, "sample"),
+          _t(rank_row, i64, "rank_row"), _t(threshold, i64, "threshold"), _t(node_out, i64, "node_out"),
+          _t(edge_out, i64, "edge_out"), _i32(r), _i32(b), _i64(ranks.numel() // pmax), _i32(pmax), _i64(n_out),
+          _i64(e_out), _t(x23_out, f32, "x23_out"), _t(src_out, i64, "src_out"), _t(dst_out, i64, "dst_out"),
+          _t(edge_attr_out, f32, "edge_attr_out"), _t(flag, i32, "flag"), _stream())
 
 
 def shapley_reduce(logits, base_logits, ranks, player_off, var_off, phi, se, gap, flag):

@@ -32,6 +32,9 @@
 // The flag (int32, set to 1, never cleared here) reports tables that disagree with the batch: an index out of range, a
 // variant count that is not 1 + T (P_b - 1), P_b > min(256, Pmax), a player id of a row past the rank row, offsets that
 // disagree with the node or kept counts or run past the outputs, or a rank row that is not a permutation.
+//
+// Contact games (shapley.contact_shapley) use the same chains, variant order and reduction with edges as the players:
+// is_shapley_edge_plan and is_shapley_edge_expand below.
 #include "common.cuh"
 #include "philox.cuh"
 
@@ -44,6 +47,26 @@ constexpr int SH_CTAS_PER_SM = 4;
 constexpr uint32_t SH_STREAM = 2;               // counter word 3: apart from coordnoise's items 0 and 1
 
 __device__ __forceinline__ void sh_raise(int* flag) { *(volatile int*)flag = 1; }
+
+// The P keys of pair u of sample b (counter (p, b, u, stream)) and their ranks, ties to the smaller id; clears the two
+// histograms while the keys are drawn.  Ends with rank[0 .. P) written and not yet synchronised.  tid = threadIdx.x;
+// its range is restated so that the ranking loop compiles as it did written inline in shapley_plan_kernel.
+__device__ __forceinline__ void sh_rank(uint32_t* key, int* rank, int (*hist)[SH_MAX + 1], int tid, int P, int b,
+                                        int u, uint32_t stream, uint32_t k0, uint32_t k1) {
+    __builtin_assume(tid >= 0 && tid < SH_THREADS);
+    if (tid < P) key[tid] = philox4x32_10((uint32_t)tid, (uint32_t)b, (uint32_t)u, stream, k0, k1).v[0];
+    for (int i = tid; i < 2 * (SH_MAX + 1); i += SH_THREADS) (&hist[0][0])[i] = 0;
+    __syncthreads();
+    if (tid < P) {
+        const uint32_t kp = key[tid];
+        int r = 0;
+        for (int q = 0; q < P; ++q) {
+            const uint32_t kq = key[q];
+            r += kq < kp || (kq == kp && q < tid);
+        }
+        rank[tid] = r;
+    }
+}
 
 __global__ void __launch_bounds__(SH_THREADS) shapley_plan_kernel(
         const int64_t* __restrict__ node_off, const int64_t* __restrict__ edge_off, const int64_t* __restrict__ src_local,
@@ -67,18 +90,7 @@ __global__ void __launch_bounds__(SH_THREADS) shapley_plan_kernel(
         for (int p = tid; p < pmax; p += SH_THREADS) row0[p] = row1[p] = -1;
         return;
     }
-    if (tid < P) key[tid] = philox4x32_10((uint32_t)tid, (uint32_t)b, (uint32_t)u, SH_STREAM, k0, k1).v[0];
-    for (int i = tid; i < 2 * (SH_MAX + 1); i += SH_THREADS) (&hist[0][0])[i] = 0;
-    __syncthreads();
-    if (tid < P) {
-        const uint32_t kp = key[tid];
-        int r = 0;
-        for (int q = 0; q < P; ++q) {
-            const uint32_t kq = key[q];
-            r += kq < kp || (kq == kp && q < tid);
-        }
-        rank[tid] = r;
-    }
+    sh_rank(key, rank, hist, tid, P, b, u, SH_STREAM, k0, k1);
     __syncthreads();
     for (int p = tid; p < pmax; p += SH_THREADS) {
         row0[p] = p < P ? rank[p] : -1;
@@ -194,6 +206,146 @@ __global__ void __launch_bounds__(SH_THREADS, SH_CTAS_PER_SM) shapley_expand_ker
                 const int64_t o = out + __popc(m & ((1u << lane) - 1u));
                 src_out[o] = s;
                 dst_out[o] = d;
+                edge_attr_out[o] = __ldg(edge_attr + e0 + i);
+            }
+            out += __popc(m);
+        }
+    }
+}
+
+// ---- contact games: the players are sets of edges ------------------------------------------------------------------
+//
+// edge_players[e] is the graph-local player id of edge e (-1: never removed).  Removing a set of players drops their
+// edges; rows, the attributes of the kept edges and their base order are unchanged.  The keys use counter word 3 =
+// SH_EDGE_STREAM, so the permutations of a contact game are independent of a residue game's on the same seed.
+
+constexpr uint32_t SH_EDGE_STREAM = 3;          // apart from coordnoise's 0 and 1 and the residue games' 2
+
+// One CTA per (sample b, pair u), as shapley_plan_kernel: an edge of player q is kept in coalition j iff j <= rank_t(q),
+// an edge without a player (or with an id outside [0, P_b)) always, so a histogram of its rank per permutation, read as
+// a suffix sum, gives every kept count.
+__global__ void __launch_bounds__(SH_THREADS) shapley_edge_plan_kernel(
+        const int64_t* __restrict__ edge_off, const int* __restrict__ edge_players,
+        const int64_t* __restrict__ player_off, const int64_t* __restrict__ var_off, int T, int pmax, uint32_t k0,
+        uint32_t k1, int* __restrict__ ranks, int64_t* __restrict__ kept, int* __restrict__ flag) {
+    __shared__ uint32_t key[SH_MAX];
+    __shared__ int rank[SH_MAX];
+    __shared__ int hist[2][SH_MAX + 1];
+    const int b = blockIdx.x, u = blockIdx.y, tid = threadIdx.x;
+    const int64_t P64 = __ldg(player_off + b + 1) - __ldg(player_off + b);
+    const int64_t v0 = __ldg(var_off + b), nvar = __ldg(var_off + b + 1) - v0;
+    if (P64 < 0 || P64 > SH_MAX || P64 > pmax || v0 < 0 || nvar != (P64 ? 1 + (int64_t)T * (P64 - 1) : 0)) {
+        if (tid == 0) sh_raise(flag);
+        return;
+    }
+    const int P = (int)P64;
+    int* row0 = ranks + ((int64_t)b * T + 2 * u) * pmax;
+    int* row1 = row0 + pmax;
+    if (P == 0) {
+        for (int p = tid; p < pmax; p += SH_THREADS) row0[p] = row1[p] = -1;
+        return;
+    }
+    sh_rank(key, rank, hist, tid, P, b, u, SH_EDGE_STREAM, k0, k1);
+    __syncthreads();
+    for (int p = tid; p < pmax; p += SH_THREADS) {
+        row0[p] = p < P ? rank[p] : -1;
+        row1[p] = p < P ? P - 1 - rank[p] : -1;
+    }
+    const int64_t e0 = __ldg(edge_off + b), eb = __ldg(edge_off + b + 1) - e0;
+    for (int64_t i = tid; i < eb; i += SH_THREADS) {
+        const int q = __ldg(edge_players + e0 + i);
+        const bool h = (unsigned)q < (unsigned)P;
+        const int r = h ? rank[q] : P;                                              // P: never removed
+        atomicAdd(&hist[0][r], 1);
+        atomicAdd(&hist[1][h ? P - 1 - r : P], 1);                                  // the reversed permutation
+    }
+    __syncthreads();
+    // coalition j keeps the edges whose rank is >= j: kept(j) = hist[j] + ... + hist[P]
+    for (int j = 1 + tid; j < P; j += SH_THREADS) {
+        int64_t s0 = 0, s1 = 0;
+        for (int m = j; m <= P; ++m) { s0 += hist[0][m]; s1 += hist[1][m]; }
+        kept[v0 + 1 + (int64_t)(2 * u) * (P - 1) + (j - 1)] = s0;
+        kept[v0 + 1 + (int64_t)(2 * u + 1) * (P - 1) + (j - 1)] = s1;
+    }
+    if (u == 0 && tid == 0) kept[v0] = hist[0][P];                                 // every player removed
+}
+
+// One pass of contact coalitions, units (variant, part) grid-strided as shapley_expand_kernel.  The unit's rank row is
+// staged in shared memory; an edge with id q >= 0 is dropped iff rank[q] < j.  Part 0 copies the rows verbatim, part 1
+// compacts the kept edges in base order (warp slices, ballots, one scan of the warp counts); both check the kept count
+// against edge_out first, so a variant is written whole or not at all.
+__global__ void __launch_bounds__(SH_THREADS, SH_CTAS_PER_SM) shapley_edge_expand_kernel(
+        const float* __restrict__ x23, const int64_t* __restrict__ node_off, const int64_t* __restrict__ edge_off,
+        const int64_t* __restrict__ src_local, const int64_t* __restrict__ dst_local, const float* __restrict__ edge_attr,
+        const int* __restrict__ edge_players, const int* __restrict__ ranks, const int64_t* __restrict__ sample,
+        const int64_t* __restrict__ rank_row, const int64_t* __restrict__ threshold, const int64_t* __restrict__ node_out,
+        const int64_t* __restrict__ edge_out, int r, int B, int64_t n_rows, int pmax, int64_t n_out, int64_t e_out,
+        float* __restrict__ x23_out, int64_t* __restrict__ src_out, int64_t* __restrict__ dst_out,
+        float* __restrict__ edge_attr_out, int* __restrict__ flag) {
+    __shared__ int64_t warp_base[SH_WARPS + 1];
+    __shared__ int rk[SH_MAX];
+    const int64_t units = 2 * (int64_t)r;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    for (int64_t unit = blockIdx.x; unit < units; unit += gridDim.x) {
+        const int v = (int)(unit >> 1), part = (int)(unit & 1);
+        const int64_t b = __ldg(sample + v), row = __ldg(rank_row + v), j = __ldg(threshold + v);
+        if (b < 0 || b >= B || row < 0 || row >= n_rows || j < 0 || j > pmax) {
+            if (part == 0 && threadIdx.x == 0) sh_raise(flag);
+            continue;
+        }
+        const int64_t n0 = __ldg(node_off + b), nb = __ldg(node_off + b + 1) - n0;
+        const int64_t e0 = __ldg(edge_off + b), eb = __ldg(edge_off + b + 1) - e0;
+        const int64_t no = __ldg(node_out + v), eo = __ldg(edge_out + v), ek = __ldg(edge_out + v + 1) - eo;
+        if (nb < 0 || no < 0 || __ldg(node_out + v + 1) - no != nb || no + nb > n_out || eo < 0 || ek < 0 ||
+            eo + ek > e_out) {
+            if (part == 0 && threadIdx.x == 0) sh_raise(flag);
+            continue;
+        }
+        __syncthreads();                                                 // the previous unit's rank row is consumed
+        for (int p = threadIdx.x; p < pmax; p += SH_THREADS) rk[p] = __ldg(ranks + row * pmax + p);
+        __syncthreads();
+        const int* ids = edge_players + e0;
+        const int64_t per = (eb + SH_WARPS - 1) / SH_WARPS;              // warp slice: [warp * per, (warp + 1) * per)
+        const int64_t lo = min((int64_t)warp * per, eb), hi = min(lo + per, eb);
+        int64_t kept = 0;
+        bool bad = false;
+        for (int64_t i0 = lo; i0 < hi; i0 += 32) {
+            const int64_t i = i0 + lane;
+            const int q = i < hi ? __ldg(ids + i) : -1;
+            bad |= q >= pmax;
+            kept += __popc(__ballot_sync(0xffffffffu, i < hi && (q < 0 || (q < pmax && rk[q] >= j))));
+        }
+        if (lane == 0) warp_base[warp + 1] = kept;
+        if (__syncthreads_or(bad)) {                                     // CTA-uniform
+            if (part == 0 && threadIdx.x == 0) sh_raise(flag);
+            continue;
+        }
+        if (threadIdx.x == 0) {
+            warp_base[0] = 0;
+            for (int w = 1; w <= SH_WARPS; ++w) warp_base[w] += warp_base[w - 1];
+        }
+        __syncthreads();
+        if (warp_base[SH_WARPS] != ek) {                                 // CTA-uniform
+            if (part == 1 && threadIdx.x == 0) sh_raise(flag);
+            continue;
+        }
+        if (part == 0) {
+            const int64_t n = nb * 23;
+            const float* xs = x23 + n0 * 23;
+            float* xd = x23_out + no * 23;
+            for (int64_t i = threadIdx.x; i < n; i += SH_THREADS) xd[i] = __ldg(xs + i);
+            continue;
+        }
+        int64_t out = eo + warp_base[warp];
+        for (int64_t i0 = lo; i0 < hi; i0 += 32) {
+            const int64_t i = i0 + lane;
+            const int q = i < hi ? __ldg(ids + i) : -1;
+            const bool keep = i < hi && (q < 0 || rk[q] >= j);           // q < pmax: checked above
+            const unsigned m = __ballot_sync(0xffffffffu, keep);
+            if (keep) {
+                const int64_t o = out + __popc(m & ((1u << lane) - 1u));
+                src_out[o] = __ldg(src_local + e0 + i);
+                dst_out[o] = __ldg(dst_local + e0 + i);
                 edge_attr_out[o] = __ldg(edge_attr + e0 + i);
             }
             out += __popc(m);
@@ -343,6 +495,46 @@ int is_shapley_expand(const float* x23, const int64_t* node_off, const int64_t* 
     shapley_expand_kernel<<<(unsigned)(units < cap ? units : cap), SH_THREADS, 0, (cudaStream_t)stream>>>(
         x23, node_off, edge_off, src_local, dst_local, edge_attr, players, ranks, sample, rank_row, threshold, node_out,
         edge_out, r, n_graphs, n_rank_rows, max_players, n_nodes_out, n_edges_out, x23_out, src_out, dst_out,
+        edge_attr_out, flag);
+    IS_LAUNCH_CHECK();
+    return IS_OK;
+}
+
+// grid: (B, T/2) CTAs of 256 threads
+int is_shapley_edge_plan(const int64_t* edge_off, const int* edge_players, const int64_t* player_off,
+                         const int64_t* var_off, int n_graphs, int permutations, int max_players, uint64_t seed,
+                         int* ranks, int64_t* kept, int* flag, void* stream) {
+    if (n_graphs < 1 || permutations < 2 || permutations % 2 || max_players < 1 || !edge_off || !player_off ||
+        !var_off || !ranks || !kept || !flag)
+        return IS_ERR_ARG;
+    if (permutations > 65536 || max_players > SH_MAX) return IS_ERR_UNSUPPORTED;
+    shapley_edge_plan_kernel<<<dim3((unsigned)n_graphs, (unsigned)(permutations / 2)), SH_THREADS, 0,
+                               (cudaStream_t)stream>>>(edge_off, edge_players, player_off, var_off, permutations,
+                                                       max_players, (uint32_t)seed, (uint32_t)(seed >> 32), ranks,
+                                                       kept, flag);
+    IS_LAUNCH_CHECK();
+    return IS_OK;
+}
+
+// grid: min(2 r, 4 x SMs) CTAs of 256 threads, each looping over (variant, part) units
+int is_shapley_edge_expand(const float* x23, const int64_t* node_off, const int64_t* edge_off,
+                           const int64_t* src_local, const int64_t* dst_local, const float* edge_attr,
+                           const int* edge_players, const int* ranks, const int64_t* sample, const int64_t* rank_row,
+                           const int64_t* threshold, const int64_t* node_out, const int64_t* edge_out, int r,
+                           int n_graphs, int64_t n_rank_rows, int max_players, int64_t n_nodes_out,
+                           int64_t n_edges_out, float* x23_out, int64_t* src_out, int64_t* dst_out,
+                           float* edge_attr_out, int* flag, void* stream) {
+    if (r < 1 || n_graphs < 1 || n_rank_rows < 1 || max_players < 1 || n_nodes_out < 0 || n_edges_out < 0) return IS_ERR_ARG;
+    if (!x23 || !node_off || !edge_off || !ranks || !sample || !rank_row || !threshold || !node_out || !edge_out ||
+        !flag || (n_nodes_out > 0 && !x23_out) ||
+        (n_edges_out > 0 && (!src_local || !dst_local || !edge_attr || !edge_players || !src_out || !dst_out ||
+                             !edge_attr_out)))
+        return IS_ERR_ARG;
+    if ((int64_t)r > 0x3fffffff || max_players > SH_MAX) return IS_ERR_UNSUPPORTED;
+    const int64_t units = 2 * (int64_t)r, cap = (int64_t)SH_CTAS_PER_SM * current_num_sms();
+    shapley_edge_expand_kernel<<<(unsigned)(units < cap ? units : cap), SH_THREADS, 0, (cudaStream_t)stream>>>(
+        x23, node_off, edge_off, src_local, dst_local, edge_attr, edge_players, ranks, sample, rank_row, threshold,
+        node_out, edge_out, r, n_graphs, n_rank_rows, max_players, n_nodes_out, n_edges_out, x23_out, src_out, dst_out,
         edge_attr_out, flag);
     IS_LAUNCH_CHECK();
     return IS_OK;

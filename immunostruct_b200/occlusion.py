@@ -119,14 +119,12 @@ def _residue_tables(graph, nodes, max_graphs):
     return tables, rows[:tables[-1]]
 
 
-def _contact_tables(graph, nodes, max_graphs):
-    """Contact variants in (sample, u, v) order: (tables, edge_contact [ΣE])."""
-    variant_passes(1, max_graphs)
-    gs, gd, touch = _degrees(graph)
-    sel = _selection(graph, nodes, touch)
-    n, e = graph.n_nodes, graph.n_edges
-    if e == 0:
-        raise ValueError("the selection holds no contact: nothing to occlude")
+def _contacts(gs, gd, sel, n):
+    """The contacts of the global edges (gs, gd) [E > 0] with at least one endpoint selected by ``sel`` [N], numbered in
+    (sample, u, v) order, without a host read -> (edge_contact [E]: the contact id of each edge, -1 for self-loops and
+    unselected contacts; global endpoints ug, vg [E] of contact c at entry c, for c < C; edges of contact c [E]; C, a
+    device count)."""
+    e = gs.shape[0]
     # global node ids run in (sample, local row) order, so the key lo * N + hi orders contacts by (sample, u, v)
     lo, hi = torch.minimum(gs, gd), torch.maximum(gs, gd)
     sentinel = n * n
@@ -139,11 +137,22 @@ def _contact_tables(graph, nodes, max_graphs):
     mult = torch.zeros(e + 1, dtype=torch.int64, device=ks.device).scatter_add_(0, torch.where(live, cid, e),
                                                                                 torch.ones_like(cid))[:e]
     key = ks[_first_selected(first)]                              # the contacts' keys first, in order
-    ug, vg = (key // n).clamp_max(n - 1), key % n
+    return edge_contact, (key // n).clamp_max(n - 1), key % n, mult, first.sum()
+
+
+def _contact_tables(graph, nodes, max_graphs):
+    """Contact variants in (sample, u, v) order: (tables, edge_contact [ΣE])."""
+    variant_passes(1, max_graphs)
+    gs, gd, touch = _degrees(graph)
+    sel = _selection(graph, nodes, touch)
+    n, e = graph.n_nodes, graph.n_edges
+    if e == 0:
+        raise ValueError("the selection holds no contact: nothing to occlude")
+    edge_contact, ug, vg, mult, c = _contacts(gs, gd, sel, n)
     smp = graph.batch[ug]
     off = graph.node_off[smp]
-    kept = graph.batch_num_edges().to(ks.device)[smp] - mult
-    tables = _finish_tables(graph, smp, ug - off, vg - off, kept, first.sum(), -(-e // max_graphs), max_graphs, "contact")
+    kept = graph.batch_num_edges().to(ug.device)[smp] - mult
+    tables = _finish_tables(graph, smp, ug - off, vg - off, kept, c, -(-e // max_graphs), max_graphs, "contact")
     return tables, edge_contact
 
 

@@ -30,6 +30,14 @@ rows and compacted edges from the resident batch, the pass's topology is collate
 logits of all variants stay on the device (V K 4 bytes) for ``is_shapley_reduce``, which writes φ, se and gap in fp64
 in a fixed order; its flag and the expansion's are read once, after it.  An entry agrees with the fused eval forward of the host-built coalition batch to rounding, not bit for bit
 (mutagenesis module docstring, DESIGN 4.4c).
+
+Contacts.  ``contact_shapley`` plays the same game with sets of edges as the players, answering which contacts carry
+the call where residue removal cannot separate a residue's contacts.  Removing players drops their edges and nothing
+else: every row stays, and the kept edges keep their attributes and base order, so a coalition is exactly the graph a
+boolean edge mask builds.  Players are explicit edge groups (int64 [ΣE]) or every contact with a selected endpoint (bool
+[ΣN], numbered as ``occlusion.occlude_contacts`` numbers contacts).  The keys use counter word 3 = 3 instead of 2, so a
+contact game's permutations are independent of a residue game's on the same seed.  ``is_shapley_edge_plan`` and
+``is_shapley_edge_expand`` replace the plan and the expansion; variants, passes and the reduction are shared.
 """
 from __future__ import annotations
 
@@ -43,7 +51,7 @@ from .comparative_models import _Comparative
 from .coordnoise import _seed
 from .graph import MAX_GRAPH_NODES
 from .hybrid_models import _Hybrid
-from .occlusion import _degrees, _selection
+from .occlusion import _contacts, _degrees, _selection
 from .predictive import _CLASSES, _PAIR_CLASSES, Predictive, _check, _pair_items, _scorer, _scorer_pair
 from .resident import pass_totals, score_gathered, variant_passes
 
@@ -56,6 +64,26 @@ class ResidueShapley:
     order."""
     players: Tensor       # [ΣN]  int64, graph-local player id of each node row, -1 for rows never removed
     offsets: Tensor       # [B+1] int64
+    logit: Tensor         # [Q]   φ of v_logit (mean logit over the draws)
+    prob: Tensor          # [Q]   φ of v_prob (mean sigmoid(logit) over the draws)
+    logit_se: Tensor      # [Q]   standard error of the mean over the antithetic pairs; NaN for T = 2
+    prob_se: Tensor       # [Q]
+    empty: Predictive     # every player removed (base for a sample without players)
+    gap_logit: Tensor     # [B]   (v(base) - v(empty)) - Σ φ, of v_logit
+    gap_prob: Tensor      # [B]
+    base: Predictive      # the unmodified batch on the same draws
+    seed: int             # the seed of the permutation keys
+    permutations: int     # T
+
+
+@dataclass
+class ContactShapley:
+    """Shapley values of the contact players of every sample; sample b's players are entries offsets[b] ..
+    offsets[b+1]-1, in id order."""
+    edge_player: Tensor   # [ΣE]  int64, graph-local player id of each edge, -1 for edges never removed
+    offsets: Tensor       # [B+1] int64
+    u: Tensor             # [Q]   int64, graph-local endpoints of a bool-selected contact, u < v; -1 for explicit groups
+    v: Tensor             # [Q]
     logit: Tensor         # [Q]   φ of v_logit (mean logit over the draws)
     prob: Tensor          # [Q]   φ of v_prob (mean sigmoid(logit) over the draws)
     logit_se: Tensor      # [Q]   standard error of the mean over the antithetic pairs; NaN for T = 2
@@ -87,6 +115,20 @@ def _checked(model, permutations, seed, max_graphs, eps, graphs):
     return _seed(seed)
 
 
+def _counted(ids, owner, b):
+    """P_b of explicit graph-local ids [M] whose entries belong to graphs ``owner`` [M] -> (P_b int64 [B], device bools
+    (ids not exactly 0 .. P_b - 1, P_b > 256))."""
+    dev = ids.device
+    live = ids >= 0
+    count = torch.zeros(b, dtype=torch.int64, device=dev).scatter_reduce_(0, owner, ids + 1, "amax")
+    held = torch.zeros(b * MAX_GRAPH_NODES + 1, dtype=torch.int64, device=dev)
+    slot = torch.where(live & (ids < MAX_GRAPH_NODES), owner * MAX_GRAPH_NODES + ids, b * MAX_GRAPH_NODES)
+    held.index_fill_(0, slot, 1)
+    distinct = held[:-1].view(b, MAX_GRAPH_NODES).sum(1)
+    too_many = (count > MAX_GRAPH_NODES).any()
+    return count, (ids < -1).any() | (~too_many & (distinct != count).any()), too_many
+
+
 def _players(graph, players):
     """(graph-local ids int64 [ΣN], P_b int64 [B], device bools (ids not exactly 0 .. P_b - 1, P_b > 256)) on the
     batch's device."""
@@ -102,35 +144,83 @@ def _players(graph, players):
         ids = torch.where(players, c[1:] - 1 - c[first][batch], -1)
         count = c[graph.node_off[1:].to(dev)] - c[first]
         return ids, count, torch.zeros((), dtype=torch.bool, device=dev), (count > MAX_GRAPH_NODES).any()
-    ids = players
-    live = ids >= 0
-    count = torch.zeros(b, dtype=torch.int64, device=dev).scatter_reduce_(0, batch, ids + 1, "amax")
-    held = torch.zeros(b * MAX_GRAPH_NODES + 1, dtype=torch.int64, device=dev)
-    slot = torch.where(live & (ids < MAX_GRAPH_NODES), batch * MAX_GRAPH_NODES + ids, b * MAX_GRAPH_NODES)
-    held.index_fill_(0, slot, 1)
-    distinct = held[:-1].view(b, MAX_GRAPH_NODES).sum(1)
-    too_many = (count > MAX_GRAPH_NODES).any()
-    return ids, count, (ids < -1).any() | (~too_many & (distinct != count).any()), too_many
+    return (players, *_counted(players, batch, b))
 
 
-def _sizes(graph, players, permutations):
+def _edge_players(graph, players):
+    """(graph-local ids int64 [ΣE], P_b int64 [B], device bools (ids not exactly 0 .. P_b - 1, P_b > 256), graph-local
+    endpoints (u, v) [ΣE] of player q of sample b at entry offsets[b] + q, or None for explicit ids) on the batch's
+    device."""
+    n, e, b, dev = graph.n_nodes, graph.n_edges, graph.n_graphs, graph.ndata["x"].device
+    if not isinstance(players, Tensor) or not ((players.dtype == torch.bool and tuple(players.shape) == (n,)) or
+                                               (players.dtype == torch.int64 and tuple(players.shape) == (e,))):
+        raise ValueError(f"players must be an int64 tensor [ΣE={e}] of graph-local player ids over the batch's edges, "
+                         f"or a bool tensor [ΣN={n}] selecting node rows")
+    players = players.to(dev)
+    owner = torch.repeat_interleave(torch.arange(b, device=dev), graph.batch_num_edges().to(dev), output_size=e)
+    if players.dtype == torch.int64:
+        return (players, *_counted(players, owner, b), None)
+    no = torch.zeros((), dtype=torch.bool, device=dev)
+    if e == 0:
+        return torch.zeros(0, dtype=torch.int64, device=dev), torch.zeros(b, dtype=torch.int64, device=dev), no, no, None
+    # every contact with a selected endpoint is its own player, numbered as occlusion numbers contacts
+    gs, gd = graph.edge_index
+    edge_contact, ug, vg, _, c = _contacts(gs, gd, players, n)
+    smp = graph.batch[ug]
+    count = torch.zeros(b, dtype=torch.int64, device=dev).scatter_add_(0, smp, (torch.arange(e, device=dev) < c).long())
+    first = torch.cat([torch.zeros(1, dtype=torch.int64, device=dev), count.cumsum(0)[:-1]])
+    ids = torch.where(edge_contact >= 0, edge_contact - first[owner], -1)
+    off = graph.node_off[smp]
+    return ids, count, no, (count > MAX_GRAPH_NODES).any(), (ug - off, vg - off)
+
+
+def _sized(checked, permutations, holder, too_many_message):
     """The checked players and the call's sizes, with its first host read -> (ids, P_b [B], variants per sample [B],
-    Pmax, V, Q)."""
-    ids, count, bad, too_many = _players(graph, players)
+    Pmax, V, Q).  ``holder`` names what holds a player; ``too_many_message(Pmax)`` is the error for more than 256."""
+    ids, count, bad, too_many = checked
     nvar = torch.where(count > 0, 1 + permutations * (count - 1), 0)
     bad_ids, many, pmax, v, q = torch.stack([bad.long(), too_many.long(), count.max(), nvar.sum(), count.sum()]).tolist()
     if many:
-        raise ValueError(f"a sample has more than {MAX_GRAPH_NODES} players")
+        raise ValueError(too_many_message(pmax))
     if bad_ids:
-        raise ValueError("the player ids of each graph must be exactly 0 .. P_b - 1, each held by at least one row, "
-                         "and -1 for rows that are never removed")
+        raise ValueError(f"the player ids of each graph must be exactly 0 .. P_b - 1, each held by at least one "
+                         f"{holder}, and -1 for {holder}s that are never removed")
     if q == 0:
-        raise ValueError("the players hold no residue: nothing to attribute")
+        raise ValueError(f"the players hold no {'residue' if holder == 'row' else holder}: nothing to attribute")
     return ids, count, nvar, pmax, v, q
 
 
-def _plan(graph, sizes, permutations, seed, max_graphs):
-    """The plan launch and the pass tables, with the call's second host read -> dict of device tables and pass sizes."""
+def _sizes(graph, players, permutations):
+    """Residue players: ``_sized`` of the node-row ids."""
+    return _sized(_players(graph, players), permutations, "row",
+                  lambda pmax: f"a sample has more than {MAX_GRAPH_NODES} players")
+
+
+def _edge_sizes(graph, players, permutations):
+    """Contact players: (``_sized`` of the edge ids, graph-local endpoints (u, v) [Q] of the players, -1 for explicit
+    groups)."""
+    *checked, uv = _edge_players(graph, players)
+    sizes = _sized(checked, permutations, "edge",
+                   lambda pmax: f"a sample has {pmax} players, more than {MAX_GRAPH_NODES}: group its edges into "
+                                f"at most {MAX_GRAPH_NODES} players")
+    q = sizes[-1]
+    if uv is None:
+        uv = (torch.full((q,), -1, dtype=torch.int64, device=sizes[0].device),) * 2
+    return sizes, tuple(x[:q].contiguous() for x in uv)
+
+
+def _row_plan(graph, ids32, poff, voff, seed, ranks, kept, flag):
+    IF._C.shapley_plan(graph.node_off, graph.edge_off, graph._src_local.contiguous(), graph._dst_local.contiguous(),
+                       ids32, poff, voff, seed, ranks, kept, flag)
+
+
+def _edge_plan(graph, ids32, poff, voff, seed, ranks, kept, flag):
+    IF._C.shapley_edge_plan(graph.edge_off, ids32, poff, voff, seed, ranks, kept, flag)
+
+
+def _plan(graph, sizes, permutations, seed, max_graphs, launch=_row_plan):
+    """The plan launch (``launch``: ``_row_plan`` or ``_edge_plan``) and the pass tables, with the call's second host
+    read -> dict of device tables and pass sizes."""
     ids, count, nvar, pmax, v, q = sizes
     t = permutations
     dev = ids.device
@@ -148,8 +238,7 @@ def _plan(graph, sizes, permutations, seed, max_graphs):
     kept = torch.zeros(v, dtype=torch.int64, device=dev)                      # sizes the passes even if the plan fails
     flag = torch.zeros(1, dtype=torch.int32, device=dev)
     ids32 = ids.to(torch.int32)
-    IF._C.shapley_plan(graph.node_off, graph.edge_off, graph._src_local.contiguous(), graph._dst_local.contiguous(),
-                       ids32, poff, voff, seed, ranks, kept, flag)
+    launch(graph, ids32, poff, voff, seed, ranks, kept, flag)
     nv = graph.batch_num_nodes().to(dev)[smp]
     passes = variant_passes(v, max_graphs)
     ncs, ecs, node_tot, edge_tot = pass_totals(nv, kept, v, len(passes), max_graphs)
@@ -159,19 +248,20 @@ def _plan(graph, sizes, permutations, seed, max_graphs):
                 edge_tot=totals[len(passes):], flag=flag, q=q)
 
 
-def _shapley(model, scorer, graph, plan, seed, permutations):
-    """Every chain variant in gathered passes, then the reduction -> ResidueShapley."""
+def _shapley(model, scorer, graph, plan, expand):
+    """Every chain variant in gathered passes, each expanded by ``expand`` (``_C.shapley_expand`` or
+    ``_C.shapley_edge_expand``), then the reduction -> (φ [2, Q], se [2, Q], gap [2, B], empty)."""
     mu, logvar, z_vae, e = scorer.item[1:]
     smp, row, thr, ranks, flag = plan["smp"], plan["row"], plan["thr"], plan["ranks"], plan["flag"]
 
-    def expand(j, r, inputs, outputs):
-        IF._C.shapley_expand(*inputs, plan["ids32"], ranks, smp[j:j + r], row[j:j + r], thr[j:j + r], *outputs, flag)
+    def expand_pass(j, r, inputs, outputs):
+        expand(*inputs, plan["ids32"], ranks, smp[j:j + r], row[j:j + r], thr[j:j + r], *outputs, flag)
 
     def pass_item(g, sp, _):
         return model.structure_embedding(g, project=False)[0].contiguous(), mu[sp], logvar[sp], z_vae[sp], e[:, sp]
 
     logits, mean, std = score_gathered(scorer, graph, smp, plan["nv"], plan["kept"], plan["ncs"], plan["ecs"],
-                                       plan["passes"], plan["node_tot"], plan["edge_tot"], expand, pass_item)
+                                       plan["passes"], plan["node_tot"], plan["edge_tot"], expand_pass, pass_item)
     base, q, b = scorer.base, plan["q"], plan["count"].shape[0]
     f32 = dict(dtype=torch.float32, device=logits.device)
     phi, se, gap = torch.empty(2, q, **f32), torch.empty(2, q, **f32), torch.empty(2, b, **f32)
@@ -182,8 +272,19 @@ def _shapley(model, scorer, graph, plan, seed, permutations):
     first = plan["voff"][:-1].clamp_max(logits.shape[0] - 1)
     empty = Predictive(torch.where(has[:, None], logits[first], base.logits), torch.where(has, mean[first], base.prob_mean),
                        torch.where(has, std[first], base.prob_std))
-    return ResidueShapley(plan["ids"], plan["poff"], phi[0], phi[1], se[0], se[1], empty, gap[0], gap[1], base, seed,
-                          permutations)
+    return phi, se, gap, empty
+
+
+def _residue_result(scorer, plan, out, seed, permutations):
+    phi, se, gap, empty = out
+    return ResidueShapley(plan["ids"], plan["poff"], phi[0], phi[1], se[0], se[1], empty, gap[0], gap[1], scorer.base,
+                          seed, permutations)
+
+
+def _contact_result(scorer, plan, uv, out, seed, permutations):
+    phi, se, gap, empty = out
+    return ContactShapley(plan["ids"], plan["poff"], *uv, phi[0], phi[1], se[0], se[1], empty, gap[0], gap[1],
+                          scorer.base, seed, permutations)
 
 
 def residue_shapley(model, graph, seq, prop, *, players: Optional[Tensor] = None, permutations: int = 32,
@@ -207,7 +308,8 @@ def residue_shapley(model, graph, seq, prop, *, players: Optional[Tensor] = None
         sizes = _sizes(graph, players, permutations)
         scorer = _scorer(model, graph, seq, prop, eps, samples)
         plan = _plan(graph, sizes, permutations, seed, max_graphs)
-        return _shapley(model, scorer, graph, plan, seed, permutations)
+        return _residue_result(scorer, plan, _shapley(model, scorer, graph, plan, IF._C.shapley_expand), seed,
+                               permutations)
 
 
 def residue_shapley_pair(model, graph_pair, seq_pair, prop_pair, *, players: Optional[Tensor] = None,
@@ -226,4 +328,46 @@ def residue_shapley_pair(model, graph_pair, seq_pair, prop_pair, *, players: Opt
         sizes = _sizes(graph_pair[0], players, permutations)
         scorer = _scorer_pair(model, graph_pair, seq_pair, prop_pair, eps, samples)
         plan = _plan(graph_pair[0], sizes, permutations, seed, max_graphs)
-        return _shapley(model, scorer, graph_pair[0], plan, seed, permutations)
+        return _residue_result(scorer, plan, _shapley(model, scorer, graph_pair[0], plan, IF._C.shapley_expand), seed,
+                               permutations)
+
+
+def contact_shapley(model, graph, seq, prop, players: Tensor, *, permutations: int = 32, seed: Optional[int] = None,
+                    eps: Optional[Tensor] = None, samples: int = 1, max_graphs: int = 4096) -> ContactShapley:
+    """Shapley values of contacts, or of contact groups, of every sample for ``model(graph, seq, prop)[3]`` (the
+    logit).  A player is a set of edges of one graph; removing players drops their edges and nothing else (rows, the
+    attributes and base order of the kept edges, sequence, properties and draws are unchanged).
+
+    ``players``: int64 [ΣE] aligned with ``graph.edata['edge_attr']``, the graph-local player id of each edge (-1: never
+    removed; the ids of graph b exactly 0 .. P_b - 1, each held by at least one edge; any edge may be grouped, a
+    self-loop included), or bool [ΣN] selecting node rows: every contact (an unordered pair u != v joined by at least one
+    edge, both directions and multi-edges included) with a selected endpoint is its own player, numbered in (u, v) order
+    within its graph as ``occlusion.occlude_contacts`` numbers them; a self-loop is never a player.  P_b <= 256 (group
+    edges to cover more); a sample may have none.  Permutations, seed, draws, passes, classes, eval mode, no_grad and
+    ``.grad`` as in ``residue_shapley``; the keys are drawn on their own Philox stream, so a contact game's permutations
+    are independent of a residue game's on the same seed."""
+    _check(model, samples, (_Hybrid, _Comparative), "contact_shapley", _CLASSES)
+    seed = _checked(model, permutations, seed, max_graphs, eps, [graph])
+    with torch.no_grad():
+        sizes, uv = _edge_sizes(graph, players, permutations)
+        scorer = _scorer(model, graph, seq, prop, eps, samples)
+        plan = _plan(graph, sizes, permutations, seed, max_graphs, _edge_plan)
+        return _contact_result(scorer, plan, uv, _shapley(model, scorer, graph, plan, IF._C.shapley_edge_expand), seed,
+                               permutations)
+
+
+def contact_shapley_pair(model, graph_pair, seq_pair, prop_pair, players: Tensor, *, permutations: int = 32,
+                         seed: Optional[int] = None, eps=None, samples: int = 1,
+                         max_graphs: int = 4096) -> ContactShapley:
+    """``contact_shapley`` of the cancer item of ``model.forward_comparative(graph_pair, seq_pair, prop_pair)`` against
+    its fixed wild type, for the four comparative classes; ``players`` indexes the cancer graph's edges (or rows).  The
+    wild type and the draws as in ``residue_shapley_pair``."""
+    _check(model, samples, _Comparative, "contact_shapley_pair", _PAIR_CLASSES)
+    seed = _checked(model, permutations, seed, max_graphs, eps, graph_pair)
+    with torch.no_grad():
+        sizes, uv = _edge_sizes(graph_pair[0], players, permutations)
+        scorer = _scorer_pair(model, graph_pair, seq_pair, prop_pair, eps, samples)
+        plan = _plan(graph_pair[0], sizes, permutations, seed, max_graphs, _edge_plan)
+        return _contact_result(scorer, plan, uv,
+                               _shapley(model, scorer, graph_pair[0], plan, IF._C.shapley_edge_expand), seed,
+                               permutations)

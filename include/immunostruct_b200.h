@@ -344,6 +344,28 @@ int is_shapley_expand(const float* x23, const int64_t* node_off, const int64_t* 
                       const int64_t* edge_out, int r, int n_graphs, int64_t n_rank_rows, int max_players,
                       int64_t n_nodes_out, int64_t n_edges_out, float* x23_out, int64_t* src_out, int64_t* dst_out,
                       float* edge_attr_out, int* flag, void* stream);
+/* Shapley values of contacts and contact groups (csrc/shapley.cu): the players are sets of edges.  edge_players int32
+ * [E]: the graph-local player id of each edge, -1 for an edge never removed.  Removing a player drops its edges; rows,
+ * the attributes of the kept edges and their base order are unchanged.  Tables, variant order and flag as above.
+ *
+ * is_shapley_edge_plan: as is_shapley_plan, the keys with counter (p, b, u, 3).  An edge of player q is kept in
+ * coalition j of permutation t iff j <= rank_t(q); an edge with id -1 (or outside [0, P_b)) always.  max_players <= 256.
+ * edge_players may be NULL when the batch has no edge. */
+int is_shapley_edge_plan(const int64_t* edge_off, const int* edge_players, const int64_t* player_off,
+                         const int64_t* var_off, int n_graphs, int permutations, int max_players, uint64_t seed,
+                         int* ranks, int64_t* kept, int* flag, void* stream);
+/* is_shapley_edge_expand: as is_shapley_expand, with every row copied verbatim and every edge e with edge_players[e] >= 0
+ * and ranks[rank_row[v]][edge_players[e]] < threshold[v] dropped.  Flag, and that variant not written: sample outside
+ * [0, B), rank_row outside [0, n_rank_rows), threshold outside [0, max_players], an edge player id >= max_players,
+ * node_out[v+1] - node_out[v] != n_b, a kept count that is not edge_out[v+1] - edge_out[v], or offsets past n_nodes_out /
+ * n_edges_out.  Bit-exact (copies only), no atomics. */
+int is_shapley_edge_expand(const float* x23, const int64_t* node_off, const int64_t* edge_off,
+                           const int64_t* src_local, const int64_t* dst_local, const float* edge_attr,
+                           const int* edge_players, const int* ranks, const int64_t* sample, const int64_t* rank_row,
+                           const int64_t* threshold, const int64_t* node_out, const int64_t* edge_out, int r,
+                           int n_graphs, int64_t n_rank_rows, int max_players, int64_t n_nodes_out,
+                           int64_t n_edges_out, float* x23_out, int64_t* src_out, int64_t* dst_out,
+                           float* edge_attr_out, int* flag, void* stream);
 /* is_shapley_reduce: logits [V, K] of the variants, base_logits [B, K] of the unmodified batch, ranks [B, T,
  * max_players] as is_shapley_plan writes them.  v_logit = mean over k of the logit, v_prob = mean of sigmoid(logit), in
  * fp64; the player at position j-1 of permutation t gets Δ = v(t, j-1) - v(t, j) (j = 0: base, j = P_b: the empty
